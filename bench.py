@@ -27,6 +27,8 @@ resident in HBM, each far larger than L2), the state carries over.
             (1,048,576-filter parameter sweep, when 4 or 8 GPUs are used), strong scaling (65,536 filters split over the
             ranks), the dense kernel variant, the parameter sweep over shared inputs, the "next" rows.
 --impl reference times the CPU path alone on the same workload shape (1,024 filters per step, all host threads).
+--dump-outputs DIR writes what the timed steps computed (ensemble state after the last step, reduced statistics) as .npy
+files; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import gc
@@ -54,6 +56,7 @@ BYTES_PER_STEP = 48 + 24 / 2 + (48 + 32) / 100     # IMU + leg odometry + pose r
 NOMINAL_FP64_TFLOPS = 148 * 64 * 2 * 1.965e9 / 1e12
 TOTAL_FILTERS = 65_536
 REF_FILTERS = 1024                                  # filters per step of the CPU arms (fixed, stated)
+RESIDENT_INPUT_BYTES = 100e9                        # HBM for the input chunks of one run; beyond it they are cycled (180 GB B200)
 
 
 def kernel_source_sha():
@@ -119,7 +122,12 @@ def parse():
     ap.add_argument("--launch-groups", type=int, default=0, help="0 = library default (automatic)")
     ap.add_argument("--mapping", type=int, default=0, help="lanes per filter (rbis_batch_config_t::mapping); 0 = automatic")
     ap.add_argument("--dense-only", action="store_true", help="force the dense kernel variant (rbis_batch_config_t::dense_only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed (rank 0's ensemble state, the reduced statistics) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -298,7 +306,8 @@ class ClockSampler:
 # CPU oracle timing (cpu_baseline leg and --impl reference)
 # ------------------------------------------------------------------------------------------------
 def cpu_oracle_rate(Tc, n_filters, threads, repeats=1):
-    """filter-steps/s of the CPU oracle (all `threads` host threads) on the config-3 schedule."""
+    """filter-steps/s of the CPU oracle (all `threads` host threads) on the config-3 schedule.  -> (rate, times, the last
+    run's result: run_ensemble's dict)."""
     from oracle import oracle_api
     from pronto_b200 import synth
 
@@ -319,7 +328,7 @@ def cpu_oracle_rate(Tc, n_filters, threads, repeats=1):
         out = oracle_api.run_ensemble(vec, quat, cov, None, 0, q, st["imu"], streams, st["events"], n_threads=threads)
         times.append(time.perf_counter() - t0)
         assert np.isfinite(out["vec"]).all()
-    return n_filters * Tc / min(times), times
+    return n_filters * Tc / min(times), times, out
 
 
 def cpu_config1_rate():
@@ -356,9 +365,11 @@ def run_reference(args):
     K, W = args.steps, args.warmup
     rates = []
     for i in range(W + K):
-        r, _ = cpu_oracle_rate(Tc, n_filters, threads)
+        r, _, out = cpu_oracle_rate(Tc, n_filters, threads)
         if i >= W:
             rates.append(r)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out["vec"], out["quat"], out["cov"], out["loglik"])
     total_t = sum(n_filters * Tc / r for r in rates)
     value = K * n_filters * Tc / total_t
     sample = f"{n_filters} filters x {Tc} steps per bench step (config-3 schedule), {threads} threads"
@@ -433,6 +444,40 @@ class Workload:
 
     def prepare(self, b):
         return [b.prepare_fused(self.progs[c], imu=self.chunks[c]["imu"], streams=self.streams[c]) for c in range(self.n)]
+
+
+DUMP_STATE_FILTERS = 65_536    # filters whose vec / quat / loglik --dump-outputs writes (every filter at the default size)
+DUMP_COV_FILTERS = 4_096       # filters whose covariance it writes (441 doubles each)
+
+
+def dump_outputs(path, vec, quat, cov, loglik, stats=None):
+    """--dump-outputs: what a caller of the timed path holds after its last step -- the ensemble state vec [21][N], quat [4][N],
+    cov [441][N], loglik [N] (numpy or torch arrays) and, where the path computes them, the reduced statistics -- as float64 .npy
+    files.  Larger ensembles are represented by a fixed, seeded sample of filters (their indices are written beside them), so the
+    files stay below 32 MB for any --filters."""
+    N = vec.shape[-1]
+
+    def sample(k, seed):
+        if N <= k:
+            return np.arange(N)
+        return np.sort(np.random.default_rng(seed).choice(N, size=k, replace=False))
+
+    def pick(t, idx):
+        if isinstance(t, np.ndarray):
+            return t[..., idx]
+        import torch
+
+        return t[..., torch.from_numpy(idx).to(t.device)].cpu().numpy()
+
+    s, sc = sample(DUMP_STATE_FILTERS, 1), sample(DUMP_COV_FILTERS, 2)
+    out = {"vec": pick(vec, s), "quat": pick(quat, s), "loglik": pick(loglik, s), "state_filters": s,
+           "cov": pick(cov, sc), "cov_filters": sc}
+    if stats is not None:
+        out["stats"] = stats
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+    log(f"[rank 0] wrote {', '.join(sorted(out))} (.npy) to {path}")
 
 
 def timed_launches(b, preps, stream, first, count, sampler=None):
@@ -517,11 +562,15 @@ def run_b200(args):
     dfma_tf, dmma_tf = measure_fp64_peak(local, 4000)
     log(f"[rank {rank}] FP64 peak measured: DFMA {dfma_tf:.2f} TFLOP/s, DMMA(mma.sync m8n8k4) {dmma_tf:.2f} TFLOP/s")
 
-    # ---- synthetic inputs: all launches of the run resident in HBM (bounded by the free memory) ----
+    # ---- synthetic inputs: all launches of the run resident in HBM, up to the fixed RESIDENT_INPUT_BYTES (not the free memory,
+    # so that the same arguments give the same inputs, and hence the same outputs, on every run and machine) ----
     n_launches = (W + K) * L
-    free_b, _ = torch.cuda.mem_get_info()
     chunk_bytes = N * Tc * (48 + 12 + 0.8) * 1.02
-    resident = max(2, min(n_launches, int(0.6 * free_b / chunk_bytes)))
+    resident = max(2, min(n_launches, int(RESIDENT_INPUT_BYTES / chunk_bytes)))
+    free_b, _ = torch.cuda.mem_get_info()
+    if resident * chunk_bytes > 0.6 * free_b:
+        raise SystemExit(f"bench.py: the run's resident inputs ({resident} chunks, {resident * chunk_bytes / 1e9:.1f} GB) need more than 60% "
+                         f"of the {free_b / 1e9:.1f} GB free on cuda:{local}; other processes hold the device's memory")
     wl = Workload(N, Tc, resident, dev, 0x5EED + rank, R_lego, R_pose)
     b = new_batch(N, dense_only=args.dense_only)
     b.set_state(wl.vec0, wl.quat0, wl.cov0)
@@ -570,6 +619,12 @@ def run_b200(args):
     stats_sha = hashlib.sha256(np.ascontiguousarray(totals).tobytes()).hexdigest()[:16]
     log(f"[rank {rank}] ensemble after {n_launches * Tc} steps: filters={summ['filters']} non_finite={summ['non_finite']} "
         f"mean NEES(9)={summ['mean_nees']:.3f} in-95%={summ['nees_in_95pct']:.3f} rms pos err={np.sqrt(np.mean(summ['rms_err'][9:12] ** 2)):.4f} m")
+    if args.dump_outputs and rank == 0:
+        st = [torch.empty(shape, dtype=torch.float64, device=dev) for shape in ((21, N), (4, N), (441, N), (N,))]
+        b.get_state_into(*st)
+        b.synchronize()
+        dump_outputs(args.dump_outputs, *st, stats=totals)
+        del st
 
     legs = {}
 
@@ -1126,7 +1181,7 @@ def run_b200(args):
     cpu = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         threads = os.cpu_count() or 1
-        rate, times = cpu_oracle_rate(args.cpu_sample_steps, REF_FILTERS, threads)
+        rate, times, _ = cpu_oracle_rate(args.cpu_sample_steps, REF_FILTERS, threads)
         rate1, t1 = cpu_config1_rate()
         cpu = {"value": rate, "unit": UNIT, "cores": threads, "kind": "port", "per_thread_value": rate / threads,
                "sample": f"{REF_FILTERS} filters x {args.cpu_sample_steps} steps of the same schedule, {threads} threads, {times[0]:.2f} s wall",
