@@ -76,7 +76,15 @@ typedef enum {
 
 typedef enum {
   RBIS_R_SHARED_FULL = 0,      /* one m x m column-major matrix for all filters (HOST pointer always) */
-  RBIS_R_PER_FILTER_DIAG = 1   /* diagonal, [m][N], located as `mem` says */
+  RBIS_R_PER_FILTER_DIAG = 1,  /* diagonal, [m][N], located as `mem` says */
+  RBIS_R_PER_ROW_FULL = 2      /* HOST [rows][m][m]: row r (column-major like the shared matrix) is the covariance of the update that
+                                  reads row r of the stream -- the measurement_cov each RBISIndexed[PlusOrientation]Measurement carries
+                                  (MSE/rbis_update_interface.hpp:90-96,111-117), e.g. leg odometry switching between its certain and
+                                  uncertain R, or indexed_measurement_t's R_effective per message.  Shared by all filters as the log is;
+                                  column maps do not apply to it.  The m rows are cut into chunks along the union of the off-diagonal
+                                  non-zeros of all rows of the call, so rows that all equal one R run exactly as RBIS_R_SHARED_FULL
+                                  with that R (same chunks, same kernel variant, same bits).  rbis_batch_run_fused and
+                                  rbis_batch_run_fused_synth only: the single-update entry points reject it (one update has one R). */
 } rbis_r_mode_t;
 
 typedef struct {
@@ -122,7 +130,7 @@ typedef struct {
 
 /* One measurement stream = the constant part of an RBISIndexedMeasurement /
  * RBISIndexedPlusOrientationMeasurement constructor (MSE/rbis_update_interface.hpp:90-96,111-117)
- * plus where its per-row data live. */
+ * plus where its per-row data live (with RBIS_R_PER_ROW_FULL the measurement covariance is per-row data too). */
 typedef struct {
   int32_t m;                      /* 1..RBIS_MAX_MEAS */
   int32_t has_orientation;        /* 0 indexedMeasurement, 1 indexedPlusOrientationMeasurement */
@@ -426,6 +434,11 @@ typedef struct {
  * R = Map<MatrixXd>(R_effective, m, m), column-major, copied to R_out[m*m]; sensor_id = indexed_sensor).  z rows are the
  * messages' z_effective; out->z / rows stay for the caller to fill. */
 int rbis_stream_from_indexed_measurement(const rbis_indexed_measurement_t* msg, rbis_stream_t* out, double* R_out);
+/* The same for a sequence of `count` messages that become rows 0..count-1 of ONE stream: all must have message 0's measured_dim,
+ * measured_cov_dim and index set (else RBIS_ERR_INVALID).  R_out [count][m][m] receives every message's R_effective; r_mode is
+ * RBIS_R_SHARED_FULL when all of them are bit-identical (R_out's first matrix is then the stream's R), else RBIS_R_PER_ROW_FULL.
+ * out->rows = count; out->z stays for the caller to fill. */
+int rbis_stream_from_indexed_measurements(const rbis_indexed_measurement_t* msgs, int64_t count, rbis_stream_t* out, double* R_out);
 
 /* KVH raw IMU batches of the Atlas INS path.  rbis_kvh_packet_t = bot_core::kvh_raw_imu_t; a batch message carries
  * num_packets of them, NEWEST FIRST, most of which were already seen in earlier batches.

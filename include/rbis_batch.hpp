@@ -267,10 +267,20 @@ class MavStateEstimator {
   struct StreamBuild {
     const RBISIndexedMeasurement* proto;
     std::vector<double> z, quat;
+    std::vector<double> R;  // [rows][m][m]: every row's measurement_cov
+    bool same_R = true;     // all rows carry proto's measurement_cov
     int64_t rows = 0;
   };
+  // Updates share a stream when they share the index set, the orientation flag and the off-diagonal zero pattern of R: each row then
+  // runs the chunk plan and decorrelation of its own R (rbis_r_mode_t), whatever the values -- a new R does not cost a flush.
   static bool same_stream(const RBISIndexedMeasurement* a, const RBISIndexedMeasurement* b) {
-    return a->index == b->index && a->measurement_cov == b->measurement_cov && (a->orientationRows() != nullptr) == (b->orientationRows() != nullptr);
+    if (a->index != b->index || (a->orientationRows() != nullptr) != (b->orientationRows() != nullptr)) return false;
+    if (a->measurement_cov.size() != b->measurement_cov.size()) return false;
+    const size_t m = a->index.size();
+    for (size_t i = 0; i < m; i++)
+      for (size_t j = 0; j < m; j++)
+        if (i != j && (a->measurement_cov[i + m * j] != 0.0) != (b->measurement_cov[i + m * j] != 0.0)) return false;
+    return true;
   }
   void flush(std::vector<rbis_op_t>& ops, std::vector<double>& imu, int64_t& imu_rows, std::vector<StreamBuild>& sb) {
     if (ops.empty()) return;
@@ -280,12 +290,12 @@ class MavStateEstimator {
       const RBISIndexedMeasurement* m = sb[s].proto;
       st[s].m = (int32_t)m->index.size();
       st[s].has_orientation = m->orientationRows() ? 1 : 0;
-      st[s].r_mode = RBIS_R_SHARED_FULL;
+      st[s].r_mode = sb[s].same_R ? RBIS_R_SHARED_FULL : RBIS_R_PER_ROW_FULL;
       st[s].sensor_id = (int32_t)m->sensor_id;
       for (size_t a = 0; a < m->index.size(); a++) st[s].idx[a] = m->index[a];
       st[s].z = sb[s].z.data();
       st[s].quat = st[s].has_orientation ? sb[s].quat.data() : nullptr;
-      st[s].R = m->measurement_cov.data();
+      st[s].R = sb[s].same_R ? m->measurement_cov.data() : sb[s].R.data();
       st[s].rows = sb[s].rows;
     }
     check(rbis_batch_run_fused(filters_->handle(), (int64_t)ops.size(), ops.data(), imu_rows ? imu.data() : nullptr, imu_rows,
@@ -324,8 +334,10 @@ class MavStateEstimator {
           if (same_stream(sb[s].proto, u)) break;
         if (s == sb.size()) {
           if (sb.size() == RBIS_MAX_STREAMS) { flush(ops, imu, imu_rows, sb); s = 0; }
-          sb.push_back(StreamBuild{u, {}, {}, 0});
+          sb.push_back(StreamBuild{u, {}, {}, {}, true, 0});
         }
+        sb[s].same_R = sb[s].same_R && u->measurement_cov == sb[s].proto->measurement_cov;
+        sb[s].R.insert(sb[s].R.end(), u->measurement_cov.begin(), u->measurement_cov.end());
         sb[s].z.insert(sb[s].z.end(), u->measurement.begin(), u->measurement.begin() + (long)(u->index.size() * (size_t)N));
         if (const std::vector<double>* q = u->orientationRows()) sb[s].quat.insert(sb[s].quat.end(), q->begin(), q->end());
         op.stream = (int32_t)s;

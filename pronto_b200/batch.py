@@ -61,7 +61,10 @@ def _common_mem(mems, what):
 
 class MeasStream:
     """Constant part + data of an RBISIndexed[PlusOrientation]Measurement stream
-    (MSE/rbis_update_interface.hpp:84-120): index set, z rows, R, optional orientation rows."""
+    (MSE/rbis_update_interface.hpp:84-120): index set, z rows, R, optional orientation rows.
+
+    R: one m x m matrix for every row; or [rows][m][m], row r's matrix for the update that reads row r
+    (RBIS_R_PER_ROW_FULL); or [m][N] per-filter diagonals with per_filter_diag=True."""
 
     def __init__(self, idx, z, R, quat=None, per_filter_diag=False, sensor_id=0):
         self.idx = [int(i) for i in idx]
@@ -115,6 +118,16 @@ class SynthSpec:
             self.shapes.append((rows, m, mq is not None))
         self.c.n_streams = len(streams)
         self.c.streams = self.sarr
+
+
+def _shared_or_row_R(R, m, rows, s):
+    """(r_mode, column-major host copy) of a stream's R given as m x m (shared) or [rows][m][m] (per row)."""
+    R = np.asarray(R, dtype=np.float64)
+    if R.ndim == 3:
+        if R.shape != (rows, m, m):
+            raise ValueError(f"stream {s}: a per-row R must be [rows][{m}][{m}] = {(rows, m, m)}, got {R.shape}")
+        return capi.R_PER_ROW_FULL, np.ascontiguousarray(R.transpose(0, 2, 1))
+    return capi.R_SHARED_FULL, np.ascontiguousarray(R.reshape(m, m).T)
 
 
 def make_ops(entries):
@@ -332,7 +345,7 @@ class RBISBatch:
             if st.per_filter_diag:
                 d.R, mm = _ptr(st.R, (m, self.N), "R"); mems.append(mm)
             else:
-                R = np.ascontiguousarray(np.asarray(st.R, dtype=np.float64).reshape(m, m).T)
+                d.r_mode, R = _shared_or_row_R(st.R, m, d.rows, s)
                 keep.append(R)
                 d.R = R.ctypes.data
             keep.append(st)
@@ -377,7 +390,7 @@ class RBISBatch:
                 if mm != capi.MEM_DEVICE:
                     raise ValueError("run_fused_synth: a per-filter R must be a device tensor")
             else:
-                R = np.ascontiguousarray(np.asarray(st.R, dtype=np.float64).reshape(m, m).T)
+                d.r_mode, R = _shared_or_row_R(st.R, m, int(spec.sarr[s].rows) if s < spec.c.n_streams else 0, s)
                 keep.append(R)
                 d.R = R.ctypes.data
             keep.append(st)

@@ -18,7 +18,7 @@ NUM_STATS = 96
 MEM_HOST, MEM_DEVICE = 0, 1
 MEM_F32_ROWS = 4  # rbis_batch_run_fused: imu / z / quat are float32 arrays (widened exactly on the device)
 OP_IMU, OP_MEAS, OP_SNAPSHOT, OP_RESTORE = 0, 1, 2, 3
-R_SHARED_FULL, R_PER_FILTER_DIAG = 0, 1
+R_SHARED_FULL, R_PER_FILTER_DIAG, R_PER_ROW_FULL = 0, 1, 2
 
 c_double_p = C.POINTER(C.c_double)
 c_int32_p = C.POINTER(C.c_int32)
@@ -151,6 +151,7 @@ PROTOTYPES = {
     "rbis_batch_get_filter_states": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(FilterState)]),
     "rbis_batch_set_filter_states": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(FilterState)]),
     "rbis_stream_from_indexed_measurement": (C.c_int, [C.POINTER(IndexedMeasurement), C.POINTER(Stream), C.c_void_p]),
+    "rbis_stream_from_indexed_measurements": (C.c_int, [C.POINTER(IndexedMeasurement), C.c_int64, C.POINTER(Stream), C.c_void_p]),
     "rbis_kvh_stream_create": (C.c_int, [C.POINTER(C.c_void_p)]),
     "rbis_kvh_stream_destroy": (C.c_int, [C.c_void_p]),
     "rbis_kvh_decode_batch": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.POINTER(KvhPacket), C.POINTER(ImuPacket), c_int32_p, C.POINTER(ImuPacket), c_int32_p]),

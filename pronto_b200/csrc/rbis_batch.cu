@@ -69,6 +69,7 @@ struct StagingSlot {  // device copies of caller-host input arrays for one fused
   DevBuf imu;
   DevBuf z[RBIS_MAX_STREAMS], quat[RBIS_MAX_STREAMS], rdiag[RBIS_MAX_STREAMS];
   DevBuf f32;  // RBIS_MEM_F32_ROWS: device copy of the host float rows of one call (all arrays back to back), widened into the above
+  DevBuf rtab; // RBIS_R_PER_ROW_FULL: the per-row R tables of the call's streams, back to back
   cudaEvent_t copied = nullptr, consumed = nullptr;
   int ring = -1;  // grouped launches: ring slot whose group events mark the consumption of this staging slot
 };
@@ -138,7 +139,7 @@ struct rbis_batch {
   cudaEvent_t uploaded[kRing] = {};
   cudaEvent_t pre_evt = nullptr;
   cudaEvent_t syn_evt = nullptr;
-  // ---- pinned host ring for the small per-call uploads (op table, shared R matrices, noise-free synth rows): a
+  // ---- pinned host ring for the small per-call uploads (op table, shared R matrices, per-row R tables, noise-free synth rows): a
   // cudaMemcpyAsync from PAGEABLE memory makes the host wait until the stream has drained to the copy, which would stop
   // the host from running ahead of the device; from pinned memory it is truly asynchronous.
   static constexpr int kPinSlots = 16;
@@ -341,12 +342,14 @@ int decorrelate_block(const double* R, int m, int a0, int len, double* W, double
   return 0;
 }
 
+// R_host: the m x m matrix whose off-diagonal zero pattern decides the cuts (for RBIS_R_PER_ROW_FULL, the union over the
+// rows of the call: every row of the stream then runs the same chunk plan)
 void plan_chunks(int m, int r_mode, const double* R_host, rbisk::StreamDesc& d) {
   std::vector<int> cut;  // start indices of the finest blocks
   cut.push_back(0);
   for (int k = 1; k < m; k++) {
     bool sep = true;
-    if (r_mode == RBIS_R_SHARED_FULL) {
+    if (r_mode != RBIS_R_PER_FILTER_DIAG) {
       for (int a = 0; a < k && sep; a++)
         for (int b = k; b < m; b++)
           if (R_host[a + m * b] != 0.0 || R_host[b + m * a] != 0.0) { sep = false; break; }
@@ -439,7 +442,18 @@ int validate_stream(int s, const rbis_stream_t& in) {
   if (in.rows < 0) return fail(RBIS_ERR_INVALID, "stream %d: negative rows", s);
   if (in.rows > 0 && (!in.z || !in.R)) return fail(RBIS_ERR_INVALID, "stream %d: z and R are required", s);
   if (in.has_orientation && in.rows > 0 && !in.quat) return fail(RBIS_ERR_INVALID, "stream %d: has_orientation but quat is NULL", s);
-  if (in.r_mode != RBIS_R_SHARED_FULL && in.r_mode != RBIS_R_PER_FILTER_DIAG) return fail(RBIS_ERR_INVALID, "stream %d: bad r_mode", s);
+  if (in.r_mode != RBIS_R_SHARED_FULL && in.r_mode != RBIS_R_PER_FILTER_DIAG && in.r_mode != RBIS_R_PER_ROW_FULL)
+    return fail(RBIS_ERR_INVALID, "stream %d: bad r_mode", s);
+  return 0;
+}
+
+// The device table of one R (layout of rbisk::RS_STRIDE): the m x m matrix, then for the correlated chunks the rows of
+// L^-1 and D (decorrelate_block).  Without correlated chunks only the matrix is read, so a per-row stream stores m * m.
+int r_table(const double* R, const rbisk::StreamDesc& d, double* out) {
+  std::memcpy(out, R, sizeof(double) * d.m * d.m);
+  for (int c = 0; c < d.n_chunks; c++)
+    if (d.chunk_fast[c] == -1)
+      if (int rc = decorrelate_block(R, d.m, d.chunk_start[c], d.chunk_len[c], out + rbisk::RS_W, out + rbisk::RS_D)) return rc;
   return 0;
 }
 
@@ -548,6 +562,8 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
   std::vector<double> rshared((size_t)RBIS_MAX_STREAMS * kRShared, 0.0);
   bool any_shared = false;
   bool shared_r[RBIS_MAX_STREAMS] = {};
+  std::vector<double> rtab_host;                  // RBIS_R_PER_ROW_FULL tables of all streams, staged like z
+  size_t rtab_off[RBIS_MAX_STREAMS] = {};
   bool needs_general = false;  // some chunk is not an aligned triple -> the kernel instantiations that contain meas1 / meas_block
   bool passive_index = false;  // some stream measures omega or a directly -> couplings become non-zero
   for (int s = 0; s < n_streams; s++) {
@@ -559,19 +575,36 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     d.map = use_maps ? h->d_map[1 + s] : nullptr;
     d.cols = d.map ? h->map_cols[1 + s] : N;
     if (in.rows == 0) { d.n_chunks = 0; continue; }
-    plan_chunks(in.m, in.r_mode, in.r_mode == RBIS_R_SHARED_FULL ? in.R : nullptr, d);
+    const size_t mm = (size_t)in.m * in.m;
+    if (in.r_mode == RBIS_R_PER_ROW_FULL) {
+      // off-diagonal non-zeros of any row cut the chunks of every row; rows that all share one R plan as that R does
+      std::vector<double> pattern(mm, 0.0);
+      for (int64_t r = 0; r < in.rows; r++)
+        for (size_t k = 0; k < mm; k++)
+          if (in.R[(size_t)r * mm + k] != 0.0) pattern[k] = 1.0;
+      plan_chunks(in.m, in.r_mode, pattern.data(), d);
+    } else {
+      plan_chunks(in.m, in.r_mode, in.r_mode == RBIS_R_SHARED_FULL ? in.R : nullptr, d);
+    }
     mark_fast_chunks(d, &needs_general);
     for (int a = 0; a < in.m; a++)
       if (!rbisk::is_act(in.idx[a])) passive_index = true;
     if (in.r_mode == RBIS_R_SHARED_FULL) {
-      double* rs = &rshared[(size_t)s * kRShared];
-      std::memcpy(rs, in.R, sizeof(double) * in.m * in.m);
-      for (int c = 0; c < d.n_chunks; c++)
-        if (d.chunk_fast[c] == -1)
-          if (int rc = decorrelate_block(in.R, in.m, d.chunk_start[c], d.chunk_len[c], rs + rbisk::RS_W, rs + rbisk::RS_D)) return rc;
+      if (int rc = r_table(in.R, d, &rshared[(size_t)s * kRShared])) return rc;
       d.R = h->d_rshared + (size_t)s * kRShared;  // grouped launches: re-pointed into the piece's ring slot below
       shared_r[s] = true;
       any_shared = true;
+    } else if (in.r_mode == RBIS_R_PER_ROW_FULL) {
+      bool blocks = false;
+      for (int c = 0; c < d.n_chunks; c++) blocks = blocks || d.chunk_fast[c] == -1;
+      d.r_stride = blocks ? kRShared : (long long)mm;
+      rtab_off[s] = rtab_host.size();
+      rtab_host.resize(rtab_host.size() + (size_t)in.rows * (size_t)d.r_stride, 0.0);
+      for (int64_t r = 0; r < in.rows; r++)
+        if (r_table(in.R + (size_t)r * mm, d, &rtab_host[rtab_off[s] + (size_t)r * (size_t)d.r_stride])) {
+          const std::string why = g_last_error;
+          return fail(RBIS_ERR_INVALID, "stream %d, stream row %lld: %s", s, (long long)r, why.c_str());
+        }
     }
   }
   // ---- kernel variant ----
@@ -648,7 +681,8 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
   // ---- inputs: stage host arrays on the copy stream (double buffered), or use device arrays in place ----
   StagingSlot& slot = h->slots[h->slot_toggle];
   cudaStream_t cst = h->copy_stream;
-  const bool staging = ((mem == RBIS_MEM_HOST) || syn != nullptr || f32_rows) && !fuse_syn;
+  // per-row R tables are per-call input like z: always staged, so that no launch reads a table a later call overwrote
+  const bool staging = (((mem == RBIS_MEM_HOST) || syn != nullptr || f32_rows) && !fuse_syn) || !rtab_host.empty();
   const bool grouped = h->n_groups > 1;
   if (staging) {
     h->slot_toggle ^= 1;
@@ -712,9 +746,15 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
       if (in.has_orientation)
         if (int rc = copy_in(h, slot.quat[s], in.quat, (size_t)in.rows * 4 * (size_t)d.cols, mem, cst, &d.quat)) return rc;
     }
-    if (in.r_mode != RBIS_R_SHARED_FULL) {
+    if (in.r_mode == RBIS_R_PER_FILTER_DIAG) {
       if (int rc = copy_in(h, slot.rdiag[s], in.R, (size_t)in.m * N, mem, cst, &d.R)) return rc;
     }
+  }
+  if (!rtab_host.empty()) {
+    if (slot.rtab.ensure(rtab_host.size())) return fail(RBIS_ERR_ALLOC, "device staging allocation of %zu doubles failed", rtab_host.size());
+    if (int rc = upload_small(h, slot.rtab.p, rtab_host.data(), rtab_host.size() * sizeof(double), cst)) return rc;
+    for (int s = 0; s < n_streams; s++)
+      if (streams[s].r_mode == RBIS_R_PER_ROW_FULL && streams[s].rows > 0) kp.streams[s].R = slot.rtab.p + rtab_off[s];
   }
   if (staging) CUDA_TRY(cudaEventRecord(slot.copied, cst));
   const LaunchGeom geom = launch_geom(variant, h->mapping, h->lane_tpb, N, h->n_sms);
@@ -1020,7 +1060,7 @@ int rbis_batch_destroy(rbis_batch_t* h) {
   if (h->stats_stream) cudaStreamDestroy(h->stats_stream);
   for (auto& b : h->d_syn_ring) b.release();
   for (auto& s : h->slots) {
-    s.imu.release(); s.f32.release();
+    s.imu.release(); s.f32.release(); s.rtab.release();
     for (int i = 0; i < RBIS_MAX_STREAMS; i++) { s.z[i].release(); s.quat[i].release(); s.rdiag[i].release(); }
     if (s.copied) cudaEventDestroy(s.copied);
     if (s.consumed) cudaEventDestroy(s.consumed);
@@ -1315,6 +1355,8 @@ static int single_meas(rbis_batch_t* h, int m, const int32_t* idx, const double*
                        const double* R, int r_mode, int64_t utime, int mem, int has_orient) {
   if (!h) return fail(RBIS_ERR_INVALID, "null handle");
   if (m < 1 || m > RBIS_MAX_MEAS || !idx) return fail(RBIS_ERR_INVALID, "bad m / idx");
+  if (r_mode == RBIS_R_PER_ROW_FULL)
+    return fail(RBIS_ERR_INVALID, "RBIS_R_PER_ROW_FULL applies to fused programs only: one update has one R (RBIS_R_SHARED_FULL)");
   rbis_stream_t st;
   std::memset(&st, 0, sizeof(st));
   st.m = m; st.has_orientation = has_orient; st.r_mode = r_mode;

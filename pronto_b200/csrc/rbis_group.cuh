@@ -356,7 +356,7 @@ __device__ __forceinline__ void g_meas3(double* Pf, const int l, FilterState& s,
   if (st.r_mode == 1) {
     S00 += Rdg[0]; S11 += Rdg[1]; S22 += Rdg[2];
   } else {
-    const double* Rm = st.R + a0 + (long long)st.m * a0;
+    const double* Rm = st.R + row * st.r_stride + a0 + (long long)st.m * a0;
     S00 += __ldg(Rm); S11 += __ldg(Rm + st.m + 1); S22 += __ldg(Rm + 2 * st.m + 2);
     S10 += __ldg(Rm + 1); S20 += __ldg(Rm + 2); S21 += __ldg(Rm + st.m + 2);
   }
@@ -409,7 +409,7 @@ __device__ __forceinline__ void g_meas1(double* Pf, const int l, FilterState& s,
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   const double z = src.z(st, row, a0, sn);
-  const double Rv = (st.r_mode == 1) ? ldg_early(st.R + (long long)a0 * N + n) : __ldg(st.R + a0 + (long long)st.m * a0);
+  const double Rv = (st.r_mode == 1) ? ldg_early(st.R + (long long)a0 * N + n) : __ldg(st.R + row * st.r_stride + a0 + (long long)st.m * a0);
   const Own<G, NA> w(l);
   const int pi = pos_of<DC>(idx);
   const double* rp = Pf + pi * LD;
@@ -451,8 +451,8 @@ __device__ __forceinline__ void g_meas_block(double* Pf, const int l, FilterStat
                                              long long row, long long sn, const V3& dquat, const V3& chi0) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
-  const double* W = st.R + RS_W;
-  const double* Dg = st.R + RS_D;
+  const double* W = st.R + row * st.r_stride + RS_W;
+  const double* Dg = st.R + row * st.r_stride + RS_D;
   const Own<G, NA> w(l);
   for (int a = 0; a < M; a++) {
     double g[1][NA];

@@ -237,9 +237,10 @@ struct StreamDesc {
   int chunk_fast[MAX_CHUNKS];  // >= 0: the chunk is the aligned index triple I0..I0+2 (I0 = chunk_fast) -> meas3<I0>
   const double* z;     // [rows][m][cols]
   const double* quat;  // [rows][4][cols]
-  const double* R;     // r_mode 0: device copy of m*m column-major; 1: [m][N]
+  const double* R;     // r_mode 0: device copy of m*m column-major (+ RS_W / RS_D); 1: [m][N]; 2: one such table per row
   const int* map;      // column of z / quat read by filter n (nullptr: column n)
   long long cols;      // columns of z / quat (N without a map)
+  long long r_stride;  // r_mode 2: doubles from the table of row r to that of row r + 1; 0 otherwise (every row reads R)
 };
 
 struct Op {
@@ -1106,7 +1107,7 @@ __device__ __forceinline__ void meas3(Cov& P, FilterState& s, const StreamDesc& 
     S00 = Rdg[0] + Y[0][J0]; S11 = Rdg[1] + Y[1][J0 + 1]; S22 = Rdg[2] + Y[2][J0 + 2];
     S10 = Y[1][J0]; S20 = Y[2][J0]; S21 = Y[2][J0 + 1];
   } else {
-    const double* Rm = st.R + a0 + (long long)st.m * a0;
+    const double* Rm = st.R + row * st.r_stride + a0 + (long long)st.m * a0;
     S00 = __ldg(Rm) + Y[0][J0]; S11 = __ldg(Rm + st.m + 1) + Y[1][J0 + 1]; S22 = __ldg(Rm + 2 * st.m + 2) + Y[2][J0 + 2];
     S10 = __ldg(Rm + 1) + Y[1][J0]; S20 = __ldg(Rm + 2) + Y[2][J0]; S21 = __ldg(Rm + st.m + 2) + Y[2][J0 + 1];
   }
@@ -1289,7 +1290,7 @@ __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& 
   constexpr int NC = DC ? N_ACT : NS;
   constexpr auto pos = &carried_pos<DC>;
   const double z = src.z(st, row, a0, sn);
-  const double Rv = (st.r_mode == 1) ? ldg_early(st.R + (long long)a0 * N + n) : __ldg(st.R + a0 + (long long)st.m * a0);
+  const double Rv = (st.r_mode == 1) ? ldg_early(st.R + (long long)a0 * N + n) : __ldg(st.R + row * st.r_stride + a0 + (long long)st.m * a0);
   double h[NC];
 #if RBIS_MEAS1_GETR
   // element by element, blocking: keeps this rarely executed path small inside the common kernels
@@ -1333,8 +1334,8 @@ template <bool DC, bool SYN>
 __device__ __forceinline__ void meas_block(Cov& P, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int M, long long row, long long N,
                                            long long n, long long sn, const V3& dquat, const V3& chi0) {
   constexpr int NC = DC ? N_ACT : NS;
-  const double* W = st.R + RS_W;
-  const double* Dg = st.R + RS_D;
+  const double* W = st.R + row * st.r_stride + RS_W;
+  const double* Dg = st.R + row * st.r_stride + RS_D;
   (void)N; (void)n;
   for (int a = 0; a < M; a++) {
     double g[NC];

@@ -84,6 +84,27 @@ int rbis_stream_from_indexed_measurement(const rbis_indexed_measurement_t* msg, 
   return 0;
 }
 
+int rbis_stream_from_indexed_measurements(const rbis_indexed_measurement_t* msgs, int64_t count, rbis_stream_t* out, double* R_out) {
+  if (!msgs || !out || !R_out || count < 1) return rbis_set_error(RBIS_ERR_INVALID, "null argument or count < 1");
+  if (int rc = rbis_stream_from_indexed_measurement(&msgs[0], out, R_out)) return rc;
+  const int m = out->m;
+  const size_t mm = (size_t)m * m;
+  bool same_R = true;
+  for (int64_t k = 1; k < count; k++) {
+    const rbis_indexed_measurement_t& g = msgs[k];
+    if (g.measured_dim != m || g.measured_cov_dim != m * m)
+      return rbis_set_error(RBIS_ERR_INVALID, "message %lld: measured_dim %d / measured_cov_dim %d differ from message 0", (long long)k,
+                            g.measured_dim, g.measured_cov_dim);
+    for (int a = 0; a < m; a++)
+      if (g.z_indices[a] != out->idx[a]) return rbis_set_error(RBIS_ERR_INVALID, "message %lld: index set differs from message 0", (long long)k);
+    std::memcpy(R_out + (size_t)k * mm, g.R_effective, sizeof(double) * mm);
+    same_R = same_R && std::memcmp(g.R_effective, msgs[0].R_effective, sizeof(double) * mm) == 0;
+  }
+  out->r_mode = same_R ? RBIS_R_SHARED_FULL : RBIS_R_PER_ROW_FULL;
+  out->rows = count;
+  return 0;
+}
+
 // ---- KVH raw IMU batches ----
 int rbis_kvh_stream_create(rbis_kvh_stream_t** out) {
   if (!out) return rbis_set_error(RBIS_ERR_INVALID, "out is NULL");
