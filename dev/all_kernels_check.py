@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """dev/all_kernels_check.py -- one small pass through every fused-kernel family with a bit-identity check (compute-sanitizer is closed on the GPU pool):
-lane-per-filter decoupled + dense, warp-group 4 / 8 lanes, SYN instantiations, snapshot / restore, snapshot statistics."""
+lane-per-filter decoupled + dense, warp-group 4 / 8 lanes, SYN instantiations, snapshot / restore, snapshot statistics, and the
+REC instantiations (RBIS_OP_RECORD) over the same mappings and variants."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -45,4 +46,45 @@ for cfg in (dict(mapping=1), dict(mapping=4), dict(mapping=8), dict(mapping=1, s
     same = all(np.array_equal(x, y) for x, y in zip(got[:4], ref[:4]))
     print("synth", cfg, "same bits" if same else "DIFFERENT", flush=True)
     assert same
+# records: a RECORD of every field after every op of the same programs, through the REC instantiations
+rec_prog, rows = [], 0
+for o in prog:
+    rec_prog += [o, (capi.OP_RECORD, 0, rows, 0, 0.0)]
+    rows += 1
+ALL = (1 << capi.REC_FIELDS) - 1
+ref_rec = ref_state = None
+for cfg in (dict(mapping=1, lane_filters_per_cta=384), dict(mapping=1, lane_filters_per_cta=128), dict(mapping=1, dense_only=True),
+            dict(mapping=4), dict(mapping=8), dict(mapping=4, dense_only=True)):
+    out = torch.full((rows, capi.REC_FIELDS, N), float("nan"), dtype=torch.float64, device="cuda")
+    with RBISBatch(N, snapshot_slots=2, **cfg) as b:
+        b.set_process_noise(*nominal_q())
+        b.set_state(sc["vec"], sc["quat"], sc["cov"])
+        b.set_record(out, ALL)
+        b.run_fused(rec_prog, imu=st["imu"], streams=gpu_streams(st))
+        variant = b.last_kernel_variant
+        got = b.get_state()
+    rec = out.cpu().numpy()
+    if ref_rec is None:
+        ref_rec, ref_state = rec, got
+    same = np.array_equal(rec, ref_rec) and all(np.array_equal(x, y) for x, y in zip(got[:4], ref_state[:4])) and not np.isnan(rec).any()
+    print("record", cfg, "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
+    assert same and variant & 8
+syn_rec = [x for i, o in enumerate(ev) for x in (o, (capi.OP_RECORD, 0, i, 0, 0.0))]
+ref_rec = None
+for cfg in (dict(mapping=1), dict(mapping=4), dict(mapping=8), dict(mapping=1, synth_materialize=True)):
+    out = torch.full((rows, capi.REC_FIELDS, N), float("nan"), dtype=torch.float64, device="cuda")
+    with RBISBatch(N, **cfg) as b:
+        b.set_process_noise(*nominal_q())
+        b.set_state(sc["vec"], sc["quat"], sc["cov"])
+        b.set_record(out, ALL)
+        b.run_fused_synth(syn_rec, [MeasStream(synth.LEGODO_IDX, None, st["R_legodo"]), MeasStream(synth.POSE_IDX, None, st["R_pose"], quat=True)],
+                          SynthSpec(synth.SEED, d["imu_mean"], d["imu_step"], d["streams"], mode=1))
+        variant = b.last_kernel_variant
+        b.synchronize()
+    rec = out.cpu().numpy()[:len(ev)]
+    if ref_rec is None:
+        ref_rec = rec
+    same = np.array_equal(rec, ref_rec) and not np.isnan(rec).any()
+    print("record synth", cfg, "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
+    assert same and variant & 8
 print("ok")

@@ -130,6 +130,39 @@ def _shared_or_row_R(R, m, rows, s):
     return capi.R_SHARED_FULL, np.ascontiguousarray(R.reshape(m, m).T)
 
 
+_QUAT_NAMES = ("quat_w", "quat_x", "quat_y", "quat_z")
+
+
+def record_fields(vec=(), quat=False, loglik=False, cov_diag=()):
+    """rbis_record_t::fields of a record set: state vector entries `vec` (indices 0..20), the quaternion (w, x, y, z), the
+    log-likelihood and the covariance diagonal entries P(i, i) for i in `cov_diag`."""
+    mask = 0
+    for i in list(vec) + list(cov_diag):
+        if not 0 <= int(i) < capi.NUM_STATES:
+            raise ValueError(f"state index {i} outside [0, {capi.NUM_STATES})")
+    for i in vec:
+        mask |= 1 << int(i)
+    if quat:
+        mask |= 0xF << 21
+    if loglik:
+        mask |= 1 << 25
+    for i in cov_diag:
+        mask |= 1 << (26 + int(i))
+    return mask
+
+
+def record_layout(mask):
+    """Names of the fields of a record row in output order: 'vec<i>', 'quat_w' .. 'quat_z', 'loglik', 'cov_diag<i>'."""
+    mask = int(mask)
+    if mask <= 0 or mask >> capi.REC_FIELDS:
+        raise ValueError(f"record fields {mask:#x}: need a non-empty set of bits 0..{capi.REC_FIELDS - 1}")
+    names = []
+    for f in range(capi.REC_FIELDS):
+        if mask >> f & 1:
+            names.append(f"vec{f}" if f < 21 else _QUAT_NAMES[f - 21] if f < 25 else "loglik" if f == 25 else f"cov_diag{f - 26}")
+    return names
+
+
 def make_ops(entries):
     """entries: iterable of (kind, stream, row, utime, dt) -> structured numpy op array."""
     entries = list(entries)
@@ -356,6 +389,28 @@ class RBISBatch:
             mem |= capi.MEM_F32_ROWS   # float rows: widened exactly on the device (rbis_mem_t)
         return (len(ops), ops.ctypes.data_as(C.POINTER(capi.Op)), p_imu, imu_rows, len(streams), sarr, mem, keep)
 
+    # ---- records ----
+    def set_record(self, out, fields):
+        """Record set of the RBIS_OP_RECORD ops of later fused calls (rbis_batch_set_record).  out: float64 [rows][k][N], k the number
+        of fields (record_fields / record_layout), a CUDA tensor (written in place) or a PINNED CPU tensor or array (filled by an
+        asynchronous copy); its rows are valid after wait(record()) or synchronize().  Does not synchronise."""
+        fields = int(fields)
+        if 0 < fields < 1 << capi.REC_FIELDS:
+            k = bin(fields).count("1")
+            if out.ndim != 3 or tuple(out.shape[1:]) != (k, self.N):
+                raise ValueError(f"record output must be [rows][{k}][{self.N}], got {tuple(out.shape)}")
+        p, mem = _ptr(out, None, "out")
+        rec = capi.Record()
+        rec.fields, rec.out, rec.rows, rec.mem = fields, p, int(out.shape[0]), mem
+        capi.check(self.lib.rbis_batch_set_record(self.h, C.byref(rec)))
+        # the previous buffer may still be written by enqueued calls: held until the next synchronize()
+        self._pending_keep = getattr(self, "_pending_keep", [])
+        self._pending_keep.append(getattr(self, "_record_out", None))
+        self._record_out = out
+
+    def clear_record(self):
+        capi.check(self.lib.rbis_batch_set_record(self.h, None))
+
     def run_prepared(self, prep):
         capi.check(self.lib.rbis_batch_run_fused(self.h, *prep[:7]))
 
@@ -427,8 +482,8 @@ class RBISBatch:
 
     @property
     def last_kernel_variant(self):
-        """0 dense, 2 decoupled (rbis_batch_config_t::dense_only), +1 with correlated-row chunks, +16 * lanes per filter for
-        the warp-group kernels; -1 before any launch."""
+        """0 dense, 2 decoupled (rbis_batch_config_t::dense_only), +1 with correlated-row chunks, +4 input rows drawn in the
+        kernel, +8 a program with RBIS_OP_RECORD ops, +16 * lanes per filter for the warp-group kernels; -1 before any launch."""
         return int(self.lib.rbis_batch_last_kernel_variant(self.h))
 
     @property

@@ -17,7 +17,8 @@ NUM_STATS = 96
 
 MEM_HOST, MEM_DEVICE = 0, 1
 MEM_F32_ROWS = 4  # rbis_batch_run_fused: imu / z / quat are float32 arrays (widened exactly on the device)
-OP_IMU, OP_MEAS, OP_SNAPSHOT, OP_RESTORE = 0, 1, 2, 3
+OP_IMU, OP_MEAS, OP_SNAPSHOT, OP_RESTORE, OP_RECORD = 0, 1, 2, 3, 4
+REC_FIELDS = 47  # record fields: 0..20 vec, 21..24 quat w,x,y,z, 25 loglik, 26..46 covariance diagonal
 R_SHARED_FULL, R_PER_FILTER_DIAG, R_PER_ROW_FULL = 0, 1, 2
 
 c_double_p = C.POINTER(C.c_double)
@@ -109,6 +110,16 @@ class ImuPacket(C.Structure):
                 ("packet_count", C.c_int64), ("delta_rotation", C.c_double * 3), ("linear_acceleration", C.c_double * 3)]
 
 
+class Record(C.Structure):
+    _fields_ = [
+        ("fields", C.c_uint64),
+        ("out", C.c_void_p),
+        ("rows", C.c_int64),
+        ("mem", C.c_int32),
+        ("reserved", C.c_int32),
+    ]
+
+
 class Op(C.Structure):
     _fields_ = [
         ("kind", C.c_int32),
@@ -145,6 +156,7 @@ PROTOTYPES = {
     "rbis_batch_indexed_update": (C.c_int, [C.c_void_p, C.c_int, c_int32_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int]),
     "rbis_batch_indexed_orient_update": (C.c_int, [C.c_void_p, C.c_int, c_int32_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int]),
     "rbis_batch_set_column_map": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
+    "rbis_batch_set_record": (C.c_int, [C.c_void_p, C.POINTER(Record)]),
     "rbis_batch_run_fused": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Op), C.c_void_p, C.c_int64, C.c_int, C.POINTER(Stream), C.c_int]),
     "rbis_batch_synthesize": (C.c_int, [C.c_void_p, C.POINTER(Synth), C.c_void_p, C.c_void_p, C.c_void_p]),
     "rbis_batch_run_fused_synth": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Op), C.c_int, C.POINTER(Stream), C.POINTER(Synth)]),

@@ -109,7 +109,7 @@ struct rbis_batch {
   double* d_notch_state = nullptr;  // [3][MAX_NOTCH][4][notch_cols]
   int64_t notch_cols = 0;
   DevBuf notch_stage;               // device copy of a host chunk
-  int last_variant = -1;  // kernel variant of the last fused launch: bit 1 decoupled, bit 0 with meas_block, bit 2 SYN (rows drawn in the kernel), bits 4.. lanes per filter (0 = one)
+  int last_variant = -1;  // kernel variant of the last fused launch: bit 1 decoupled, bit 0 with meas_block, bit 2 SYN (rows drawn in the kernel), bit 3 REC (the program records), bits 4.. lanes per filter (0 = one)
   int mapping = 1;        // lanes per filter of the fused kernels: 1 = lane-per-filter kernels, 2/4/8/16 = warp-group kernels
   int lane_tpb = 384;     // filters per CTA of the decoupled lane-per-filter kernels (384, 256, 128)
   int n_sms = 148;
@@ -158,6 +158,21 @@ struct rbis_batch {
   bool stream_dirty = true;   // the main stream got work since the last grouped launch
   cudaEvent_t tickets[8] = {};
   int next_ticket = 0;
+  // ---- records (rbis_batch_set_record): RBIS_OP_RECORD ops write into the caller's device buffer in place; for a pinned host
+  // buffer the kernels write the call's record rows into a staging buffer (double buffered across calls) that one copy on
+  // rec_stream moves out after the call's last launches.  Nothing but the reuse of a staging buffer waits for that copy.
+  bool rec_set = false;
+  rbis_record_t rec{};
+  int rec_k = 0;                          // popcount(rec.fields)
+  cudaStream_t rec_stream = nullptr;
+  cudaEvent_t rec_launched = nullptr;     // ungrouped launch done (rec_stream waits for it)
+  DevBuf rec_stage[2];
+  cudaEvent_t rec_copied[2] = {};         // the copy out of rec_stage[b] has run
+  bool rec_pending[2] = {};
+  int rec_toggle = 0;
+  bool rec_copies = false;                // rec_stream has been given work
+  cudaEvent_t ticket_rec[8] = {};         // rec_stream's position when ticket t was recorded
+  bool ticket_rec_valid[8] = {};
   // ---- statistics over a snapshot slot on a side stream (rbis_batch_stats_snapshot_enqueue): the fused launches that follow do
   // not wait for it; a launch that REWRITES the slot waits for the slot's last reader
   cudaStream_t stats_stream = nullptr;
@@ -224,11 +239,19 @@ LaunchGeom launch_geom(int variant, int mapping, int lane_tpb, long long N, int 
   return g;
 }
 
+// variant bit 3: the program records (REC instantiations)
 cudaError_t launch_variant(int variant, int syn, const LaunchGeom& g, unsigned blocks, cudaStream_t st, const rbisk::KParams& kp) {
-  if (g.tu) return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, blocks, g.threads, g.smem, st, &kp);
+  const int rec = (variant & 8) ? 1 : 0;
+  if (g.tu) return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, rec, blocks, g.threads, g.smem, st, &kp);
   if (syn) return cudaErrorInvalidValue;  // the dense lane-per-filter kernels have no SYN instantiation
-  if (variant & 1) rbisk::rbis_fused_kernel<true><<<blocks, g.threads, g.smem, st>>>(kp);
-  else rbisk::rbis_fused_kernel<false><<<blocks, g.threads, g.smem, st>>>(kp);
+  if (rec) {
+    if (variant & 1) rbisk::rbis_fused_kernel<true, false, false, true><<<blocks, g.threads, g.smem, st>>>(kp);
+    else rbisk::rbis_fused_kernel<false, false, false, true><<<blocks, g.threads, g.smem, st>>>(kp);
+  } else if (variant & 1) {
+    rbisk::rbis_fused_kernel<true><<<blocks, g.threads, g.smem, st>>>(kp);
+  } else {
+    rbisk::rbis_fused_kernel<false><<<blocks, g.threads, g.smem, st>>>(kp);
+  }
   return cudaGetLastError();
 }
 
@@ -504,6 +527,8 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
   // by a decoupled launch, or by an earlier SNAPSHOT of this program)
   std::vector<char> snap_dc = h->snap_dc;
   bool restores_ok = true, any_snapshot = false;
+  bool any_record = false;
+  std::vector<int64_t> rec_rows;  // record rows of the call, in op order
   int64_t last_utime = h->utime;
   for (int64_t i = 0; i < n_ops; i++) {
     const rbis_op_t& o = ops[i];
@@ -532,6 +557,12 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
         if (!snap_valid[(size_t)o.row]) return fail(RBIS_ERR_STATE, "op %lld: restore of empty snapshot slot %lld", (long long)i, (long long)o.row);
         if (!snap_dc[(size_t)o.row]) restores_ok = false;
         last_utime = o.utime;
+        break;
+      case RBIS_OP_RECORD:  // changes neither the filters nor the ensemble's utime
+        if (!h->rec_set) return fail(RBIS_ERR_STATE, "op %lld: RBIS_OP_RECORD but no record set (rbis_batch_set_record)", (long long)i);
+        if (o.row < 0 || o.row >= h->rec.rows) return fail(RBIS_ERR_INVALID, "op %lld: record row %lld out of range (%lld rows)", (long long)i, (long long)o.row, (long long)h->rec.rows);
+        rec_rows.push_back(o.row);
+        any_record = true;
         break;
       default:
         return fail(RBIS_ERR_INVALID, "op %lld: unknown kind %d", (long long)i, o.kind);
@@ -678,6 +709,33 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     }
   };
 
+  // records: the REC instantiations.  A host output goes through staging buffer rec_b, which holds only the DISTINCT rows the
+  // call records, in ascending order: the RECORD ops are renumbered into it, and each run of consecutive rows is copied out on
+  // its own, so rows the call does not record stay untouched in the caller's buffer.
+  const bool rec_host = any_record && h->rec.mem == RBIS_MEM_HOST;
+  const int rec_b = h->rec_toggle;
+  std::vector<int64_t> rec_distinct;
+  if (any_record) {
+    variant |= 8;
+    kp.rec.fields = h->rec.fields;
+    kp.rec.k = h->rec_k;
+    kp.rec.out = h->rec.out;
+    if (rec_host) {
+      rec_distinct = rec_rows;
+      std::sort(rec_distinct.begin(), rec_distinct.end());
+      rec_distinct.erase(std::unique(rec_distinct.begin(), rec_distinct.end()), rec_distinct.end());
+      for (rbisk::Op& k : kops)
+        if (k.kind == RBIS_OP_RECORD) k.row = std::lower_bound(rec_distinct.begin(), rec_distinct.end(), k.row) - rec_distinct.begin();
+      const size_t rec_count = rec_distinct.size() * (size_t)h->rec_k * (size_t)N;
+      DevBuf& sb = h->rec_stage[rec_b];
+      if (sb.cap < rec_count) {
+        if (h->rec_pending[rec_b]) CUDA_TRY(cudaEventSynchronize(h->rec_copied[rec_b]));  // its last copy (and launches) are done
+        if (sb.ensure(rec_count)) return fail(RBIS_ERR_ALLOC, "record staging allocation of %zu doubles failed", rec_count);
+      }
+      h->rec_toggle ^= 1;
+      kp.rec.out = sb.p;
+    }
+  }
   // ---- inputs: stage host arrays on the copy stream (double buffered), or use device arrays in place ----
   StagingSlot& slot = h->slots[h->slot_toggle];
   cudaStream_t cst = h->copy_stream;
@@ -772,6 +830,7 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     if (int rc = main_stream_work(h)) return rc;
     for (cudaEvent_t e : slot_readers) CUDA_TRY(cudaStreamWaitEvent(h->stream, e, 0));
     if (staging) CUDA_TRY(cudaStreamWaitEvent(h->stream, slot.copied, 0));
+    if (rec_host && h->rec_pending[rec_b]) CUDA_TRY(cudaStreamWaitEvent(h->stream, h->rec_copied[rec_b], 0));
     // ---- op table and shared R matrices (small, pageable source: staged synchronously by the runtime) ----
     if ((size_t)n_ops > h->d_ops_cap) {
       if (h->d_ops) {
@@ -801,6 +860,10 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     CUDA_TRY(launch_variant(variant, fuse_syn ? 1 : 0, geom, grid, h->stream, kp));
     h->launches++;
     if (staging) CUDA_TRY(cudaEventRecord(slot.consumed, h->stream));
+    if (rec_host) {
+      CUDA_TRY(cudaEventRecord(h->rec_launched, h->stream));
+      CUDA_TRY(cudaStreamWaitEvent(h->rec_stream, h->rec_launched, 0));
+    }
   } else {
     // ---- grouped launch: the program is cut into consecutive PIECES of ~piece_ops ops over the same (already staged)
     // inputs; every piece is one kernel per launch group, uploads on their own stream into the piece's ring slot.  Group g
@@ -856,6 +919,7 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
         if (pc == 0)
           for (cudaEvent_t e : slot_readers) CUDA_TRY(cudaStreamWaitEvent(gs, e, 0));
         if (staging && pc == 0) CUDA_TRY(cudaStreamWaitEvent(gs, slot.copied, 0));
+        if (rec_host && pc == 0 && h->rec_pending[rec_b]) CUDA_TRY(cudaStreamWaitEvent(gs, h->rec_copied[rec_b], 0));
         CUDA_TRY(cudaStreamWaitEvent(gs, h->uploaded[ring], 0));
         if (b1 > b0) {
           kp.block_offset = (int)b0;
@@ -872,6 +936,21 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
       if (staging) slot.ring = ring;   // the LAST piece that reads the staging slot marks its consumption
       if (pc + 1 < pieces) h->launch_seq++;
     }
+    if (rec_host)  // every group of the last piece: the groups of earlier pieces ran before them on the same streams
+      for (int g = 0; g < h->n_groups; g++) CUDA_TRY(cudaStreamWaitEvent(h->rec_stream, h->gdone[h->last_ring][g], 0));
+  }
+  if (rec_host) {
+    const size_t row_doubles = (size_t)h->rec_k * (size_t)N;
+    for (size_t a = 0; a < rec_distinct.size();) {  // one copy per run of consecutive record rows
+      size_t e = a + 1;
+      while (e < rec_distinct.size() && rec_distinct[e] == rec_distinct[e - 1] + 1) e++;
+      CUDA_TRY(cudaMemcpyAsync(h->rec.out + (size_t)rec_distinct[a] * row_doubles, h->rec_stage[rec_b].p + a * row_doubles,
+                               (e - a) * row_doubles * sizeof(double), cudaMemcpyDeviceToHost, h->rec_stream));
+      a = e;
+    }
+    CUDA_TRY(cudaEventRecord(h->rec_copied[rec_b], h->rec_stream));
+    h->rec_pending[rec_b] = true;
+    h->rec_copies = true;
   }
   h->launch_seq++;
   h->snap_valid = snap_valid;
@@ -997,6 +1076,10 @@ int rbis_batch_create(rbis_batch_t** out, int64_t n_filters, const rbis_batch_co
     CREATE_TRY(cudaEventCreateWithFlags(&s.consumed, cudaEventDisableTiming));
   }
   for (auto& t : h->tickets) CREATE_TRY(cudaEventCreateWithFlags(&t, cudaEventDisableTiming));
+  for (auto& t : h->ticket_rec) CREATE_TRY(cudaEventCreateWithFlags(&t, cudaEventDisableTiming));
+  CREATE_TRY(cudaStreamCreateWithFlags(&h->rec_stream, cudaStreamNonBlocking));
+  CREATE_TRY(cudaEventCreateWithFlags(&h->rec_launched, cudaEventDisableTiming));
+  for (auto& e : h->rec_copied) CREATE_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   CREATE_TRY(cudaMallocHost(&h->pin_base, rbis_batch::kPinSlots * rbis_batch::kPinBytes));
   for (auto& e : h->pin_evt) CREATE_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
   CREATE_TRY(cudaMalloc(&h->vec, N * 21 * sizeof(double)));
@@ -1014,6 +1097,8 @@ int rbis_batch_create(rbis_batch_t** out, int64_t n_filters, const rbis_batch_co
   CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_smooth_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, rbisk::SMOOTH_SMEM_BYTES));
   CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+  CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
+  CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
   for (const rbis_fused_tu_t* t : kLaneTus) CREATE_TRY(t->prepare());
   for (const rbis_fused_tu_t* t : kGroupTus) CREATE_TRY(t->prepare());
   // default state: zeros, identity quaternion, zero covariance, zero process noise
@@ -1035,6 +1120,13 @@ int rbis_batch_destroy(rbis_batch_t* h) {
   cudaSetDevice(h->cfg.device);
   if (h->stream) cudaStreamSynchronize(h->stream);
   if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
+  if (h->rec_stream) { cudaStreamSynchronize(h->rec_stream); cudaStreamDestroy(h->rec_stream); }
+  if (h->rec_launched) cudaEventDestroy(h->rec_launched);
+  for (auto& e : h->rec_copied)
+    if (e) cudaEventDestroy(e);
+  for (auto& e : h->ticket_rec)
+    if (e) cudaEventDestroy(e);
+  for (auto& b : h->rec_stage) b.release();
   if (h->upload_stream) { cudaStreamSynchronize(h->upload_stream); cudaStreamDestroy(h->upload_stream); }
   for (int g = 0; g < rbis_batch::kMaxGroups; g++)
     if (h->gstream[g]) { cudaStreamSynchronize(h->gstream[g]); cudaStreamDestroy(h->gstream[g]); }
@@ -1081,6 +1173,7 @@ int rbis_batch_synchronize(rbis_batch_t* h) {
   CUDA_TRY(cudaStreamSynchronize(h->copy_stream));
   if (h->upload_stream) CUDA_TRY(cudaStreamSynchronize(h->upload_stream));
   CUDA_TRY(cudaStreamSynchronize(h->stream));
+  CUDA_TRY(cudaStreamSynchronize(h->rec_stream));  // record copies to host memory
   if (h->stats_stream) {  // side-stream statistics (rbis_batch_stats_snapshot_enqueue): done too, their slots are free again
     CUDA_TRY(cudaStreamSynchronize(h->stats_stream));
     std::fill(h->snap_read_pending.begin(), h->snap_read_pending.end(), 0);
@@ -1244,6 +1337,34 @@ int rbis_batch_set_column_map(rbis_batch_t* h, int which, const int32_t* map, in
   if (!h->d_map[k]) CUDA_TRY(cudaMalloc(&h->d_map[k], (size_t)h->N * sizeof(int)));
   CUDA_TRY(cudaMemcpy(h->d_map[k], map, (size_t)h->N * sizeof(int), cudaMemcpyHostToDevice));
   h->map_cols[k] = cols;
+  return 0;
+}
+
+int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec) {
+  if (!h) return fail(RBIS_ERR_INVALID, "null handle");
+  if (!rec) {
+    h->rec_set = false;
+    return 0;
+  }
+  if (rec->fields == 0 || (rec->fields >> rbisk::REC_FIELDS) != 0)
+    return fail(RBIS_ERR_INVALID, "record fields 0x%llx: need a non-empty set of bits 0..%d", (unsigned long long)rec->fields, rbisk::REC_FIELDS - 1);
+  if (!rec->out) return fail(RBIS_ERR_INVALID, "record output is NULL");
+  if (rec->rows <= 0) return fail(RBIS_ERR_INVALID, "record rows must be positive");
+  if (rec->mem != RBIS_MEM_HOST && rec->mem != RBIS_MEM_DEVICE) return fail(RBIS_ERR_INVALID, "record mem must be RBIS_MEM_HOST or RBIS_MEM_DEVICE");
+  if (int rc = use_device(h)) return rc;
+  cudaPointerAttributes a;
+  cudaError_t e = cudaPointerGetAttributes(&a, rec->out);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(RBIS_ERR_INVALID, "record output: cudaPointerGetAttributes failed: %s", cudaGetErrorString(e));
+  }
+  if (rec->mem == RBIS_MEM_HOST && a.type != cudaMemoryTypeHost)
+    return fail(RBIS_ERR_INVALID, "a host record output must be pinned (page-locked) memory: a copy into pageable memory would synchronise");
+  if (rec->mem == RBIS_MEM_DEVICE && ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != h->cfg.device))
+    return fail(RBIS_ERR_INVALID, "record output is not memory of device %d", h->cfg.device);
+  h->rec = *rec;
+  h->rec_k = __builtin_popcountll(rec->fields);
+  h->rec_set = true;
   return 0;
 }
 
@@ -1610,6 +1731,9 @@ int rbis_batch_record(rbis_batch_t* h, int32_t* ticket) {
   const int t = h->next_ticket;
   h->next_ticket = (t + 1) % 8;
   CUDA_TRY(cudaEventRecord(h->tickets[t], h->stream));
+  // the record copies enqueued so far run on their own stream, which the main stream does not join
+  h->ticket_rec_valid[t] = h->rec_copies;
+  if (h->rec_copies) CUDA_TRY(cudaEventRecord(h->ticket_rec[t], h->rec_stream));
   *ticket = t;
   return 0;
 }
@@ -1619,6 +1743,7 @@ int rbis_batch_wait(rbis_batch_t* h, int32_t ticket) {
   if (ticket < 0 || ticket >= 8) return fail(RBIS_ERR_INVALID, "bad ticket");
   if (int rc = use_device(h)) return rc;
   CUDA_TRY(cudaEventSynchronize(h->tickets[ticket]));
+  if (h->ticket_rec_valid[ticket]) CUDA_TRY(cudaEventSynchronize(h->ticket_rec[ticket]));
   return 0;
 }
 

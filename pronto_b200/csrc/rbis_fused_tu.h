@@ -14,7 +14,9 @@ struct rbis_fused_tu_t {
   cudaError_t (*prepare)();
   // blocks_variant: the program has one-row / correlated chunks (lane-per-filter kernels: instantiation with those paths)
   // syn: the SYN instantiation (input rows drawn inside the kernel, KParams::syn); decoupled kernels without blocks_variant only
-  cudaError_t (*launch)(int blocks_variant, int decoupled, int syn, unsigned grid, int threads, int smem, cudaStream_t st, const void* kparams);
+  // rec: the REC instantiation (the program has RBIS_OP_RECORD ops, KParams::rec)
+  cudaError_t (*launch)(int blocks_variant, int decoupled, int syn, int rec, unsigned grid, int threads, int smem, cudaStream_t st,
+                        const void* kparams);
 };
 extern "C" {
 extern const rbis_fused_tu_t rbis_fused_tu_dc384, rbis_fused_tu_dc256, rbis_fused_tu_dc128;

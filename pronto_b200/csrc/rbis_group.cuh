@@ -553,6 +553,37 @@ __device__ __forceinline__ void g_cov_store(const double* Pf, const int l, doubl
   }
 }
 
+// RBIS_OP_RECORD: the fields of rbisk::record_fields with the same values; the state is replicated in the group, so lane l
+// stores the fields whose output position is l modulo G.  Diagonal (i, i) belongs to the lane of column i: one __syncwarp.
+template <int G, bool DC>
+__device__ __forceinline__ void g_record_fields(const KParams& p, const double* Pf, const int l, const FilterState& s, const QNoise& qn,
+                                                long long row, long long n, bool active, bool imu_seen) {
+  constexpr int LD = Geo<G, DC>::LD;
+  const long long N = p.N;
+  const unsigned long long fields = p.rec.fields;
+  double* const d = p.rec.out + row * p.rec.k * N + n;
+  __syncwarp();
+  static_for<REC_FIELDS>([&](auto fc) {
+    constexpr int f = fc;
+    if (!((fields >> f) & 1ull)) return;
+    const int pos = __popcll(fields & ((1ull << f) - 1));
+    if ((pos & (G - 1)) != l) return;
+    double v;
+    if constexpr (f < 26) {
+      v = rec_state_field<f>(s);
+    } else {
+      constexpr int i = f - 26;
+      if constexpr (DC && !is_act(i)) {
+        v = imu_seen ? (i < 3 ? qn.q_gyro : qn.q_accel) : p.P[(long long)slot(i, i) * N + n];
+      } else {
+        constexpr int a = DC ? act_pos(i) : i;
+        v = Pf[a * LD + a];
+      }
+    }
+    if (active) d[(long long)pos * N] = v;
+  });
+}
+
 // ------------------------------------------------------------------------------------------------
 // The fused kernel, warp-group mapping.  Same parameter block, op program and semantics as rbisk::rbis_fused_kernel;
 // all chunk kinds (aligned triples, one-row chunks, correlated blocks) are compiled in (the indices are run-time
@@ -560,7 +591,8 @@ __device__ __forceinline__ void g_cov_store(const double* Pf, const int l, doubl
 // MAXW = warps per CTA the launch may use (register budget: 8 -> 255 registers, 16 -> 128).
 // ------------------------------------------------------------------------------------------------
 // SYN = true: input rows drawn inside the kernel (KParams::syn), as in rbisk::rbis_fused_kernel.
-template <int G, bool DC, int MAXW, bool SYN = false>
+// REC = true: programs with RBIS_OP_RECORD ops (KParams::rec), as in rbisk::rbis_fused_kernel.
+template <int G, bool DC, int MAXW, bool SYN = false, bool REC = false>
 __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_constant__ KParams p) {
   using GE = Geo<G, DC>;
   constexpr int FPW = GE::FPW, S = GE::S;
@@ -727,6 +759,13 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
         }
       }
     } else {
+      if constexpr (REC) {
+        if (op.kind == 4) {
+          // ---- record the chosen fields into record row op.row ----
+          g_record_fields<G, DC>(p, Pf, l, s, qn, op.row, n, active, imu_seen);
+          continue;
+        }
+      }
       // ---- restore from ring slot ----
       const double* d = p.snap + op.row * SNAP_ROWS * N + n;
       static_for<NS>([&](auto i) { s.x[i] = d[(long long)i * N]; });

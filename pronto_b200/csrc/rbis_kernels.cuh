@@ -332,6 +332,16 @@ struct SynK {
   double sigma_gyro, sigma_accel, dt;  // sigma < 0: per filter sqrt(q / dt)
   SynStreamK st[8];
 };
+// RBIS_OP_RECORD (REC kernel instantiations): bit f of `fields` records field f -- 0..20 state vector, 21..24 quaternion
+// w, x, y, z, 25 log-likelihood, 26..46 covariance diagonal P(f-26, f-26) -- at out[row * k + pos][n], pos =
+// popcount(fields & ((1 << f) - 1)).  For a host output `out` is the call's staging buffer and the host has renumbered the
+// RECORD rows into it (rbis_batch.cu).
+constexpr int REC_FIELDS = 47;
+struct RecK {
+  double* out;
+  unsigned long long fields;
+  long long k;  // popcount(fields)
+};
 
 struct KParams {
   long long N;
@@ -354,6 +364,7 @@ struct KParams {
   int block_offset;  // first CTA of this launch's range (launch groups)
   StreamDesc streams[MAX_STREAMS];
   SynK syn;          // SYN kernel instantiations only
+  RecK rec;          // REC kernel instantiations only (last: the parameter offsets of everything above stay as they were)
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -1448,6 +1459,48 @@ __device__ __forceinline__ void store_overwritten_blocks(double* __restrict__ ds
   });
 }
 
+// ---- RBIS_OP_RECORD (see RecK) ----
+// record field F < 26: the state in registers
+template <int F>
+__device__ __forceinline__ double rec_state_field(const FilterState& s) {
+  if constexpr (F < NS) return s.x[F];
+  else if constexpr (F == 21) return s.qw;
+  else if constexpr (F == 22) return s.qx;
+  else if constexpr (F == 23) return s.qy;
+  else if constexpr (F == 24) return s.qz;
+  else return s.ll;
+}
+// The chosen fields of this lane's filter, with the values an RBIS_OP_SNAPSHOT at the same position stores: the diagonal
+// from shared / tensor memory through the slot helpers; in the DC kernels the (omega,omega) / (a,a) diagonals as
+// store_overwritten_blocks writes them, or the parked p.P values before the first IMU step.  `fields` is uniform, so the
+// tensor-memory loads stay warp-aligned; each chosen field is one coalesced 8-byte store per lane.
+template <bool DC>
+__device__ __forceinline__ void record_fields(const KParams& p, const Cov& P, const FilterState& s, long long row, long long n, bool active,
+                                              bool imu_seen) {
+  const long long N = p.N;
+  const unsigned long long fields = p.rec.fields;
+  double* const d = p.rec.out + row * p.rec.k * N + n;
+  static_for<REC_FIELDS>([&](auto fc) {
+    constexpr int f = fc;
+    if (!((fields >> f) & 1ull)) return;
+    double v;
+    if constexpr (f < 26) {
+      v = rec_state_field<f>(s);
+    } else {
+      constexpr int i = f - 26, s_ = slot(i, i);
+      if constexpr (DC && !is_act(i)) {
+        v = imu_seen ? __ldg((i < 3 ? p.q_gyro : p.q_accel) + n) : p.P[(long long)s_ * N + n];
+      } else {
+        Buf<1> b;
+        issue<SlotRun<s_, 1>>(P, b);
+        commit<SlotRun<s_, 1>>(b);
+        v = b.d[0];
+      }
+    }
+    if (active) d[(long long)__popcll(fields & ((1ull << f) - 1)) * N] = v;
+  });
+}
+
 // ------------------------------------------------------------------------------------------------
 // The fused kernel: every lane loads its filter, runs the whole op program, stores it back.
 // BLOCKS = true variants also contain meas1 and meas_block (one-row chunks, chunks of correlated rows); they are launched
@@ -1457,7 +1510,8 @@ __device__ __forceinline__ void store_overwritten_blocks(double* __restrict__ ds
 // DC = true is launched when the host has verified that every filter's omega / a couplings are exactly zero and no
 // measurement of the program indexes omega or a (see "decoupled filters" above).
 // SYN = true: the input rows are drawn inside the kernel (KParams::syn, mode-1 generator) instead of being read from HBM.
-template <bool BLOCKS, bool DC = false, bool SYN = false>
+// REC = true: the program has RBIS_OP_RECORD ops (KParams::rec); launched only then, so that other programs keep their code.
+template <bool BLOCKS, bool DC = false, bool SYN = false, bool REC = false>
 #ifdef RBIS_MAXNREG  // dev probe: cap the registers directly instead of through the launch bounds
 __global__ void __maxnreg__(RBIS_MAXNREG) rbis_fused_kernel(const __grid_constant__ KParams p) {
 #else
@@ -1700,6 +1754,13 @@ __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constan
         cov_store_all(P, d + 26 * N, N, active);
       }
     } else {
+      if constexpr (REC) {
+        if (op.kind == 4) {
+          // ---- record the chosen fields into record row op.row ----
+          record_fields<DC>(p, P, s, op.row, n, active, imu_seen);
+          continue;
+        }
+      }
       // ---- restore from ring slot ----
       const double* d = p.snap + op.row * SNAP_ROWS * N + n;
       static_for<NS>([&](auto i) { s.x[i] = d[(long long)i * N]; });
