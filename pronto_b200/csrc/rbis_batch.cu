@@ -14,12 +14,12 @@
 #include <vector>
 
 #include "../../include/rbis_batch.h"
-#include "rbis_kernels.cuh"   // namespace rbisk: the DENSE lane-per-filter kernels (256 filters per CTA, whole covariance on chip)
+#include "rbis_kernels.cuh"   // namespace rbisk: the kernel parameter block and the layout-conversion kernels
 #include "rbis_stats.cuh"
 #include "rbis_smooth.cuh"
 #include "rbis_synth.cuh"
-// The other fused-kernel configurations live in translation units of their own (rbis_fused_*.cu over rbis_fused_tu.inc):
-// the decoupled lane-per-filter kernels at 384 / 256 / 128 filters per CTA and the warp-group kernels of rbis_group.cuh.
+// The fused kernels live in translation units of their own (rbis_fused_*.cu over rbis_fused_tu.inc): the dense
+// lane-per-filter kernels, the decoupled ones at 384 / 256 / 128 filters per CTA and the warp-group kernels of rbis_group.cuh.
 #include "rbis_fused_tu.h"
 
 namespace {
@@ -179,27 +179,29 @@ struct rbis_batch {
   std::vector<cudaEvent_t> snap_read_evt;   // per slot, created on first use
   std::vector<char> snap_read_pending;
   std::vector<DevBuf> snap_stats_scratch;   // per slot: truth [25] + chunk partials
-  int smem_bytes = 0;
 };
 
 namespace {
 
-constexpr int kSmemBytes = rbisk::SMEM_BYTES;
 // per stream in the shared-R device buffer: R (m x m column-major, 81), then for its correlated blocks the rows of
 // L_R^-1 ([9][9] row-major, absolute row numbers) and D_R ([9]) of R_block = L_R D_R L_R^T (rbisk::RS_W, RS_D)
 constexpr int kRShared = rbisk::RS_STRIDE;
 
+static_assert(rbisk::OP_IMU == RBIS_OP_IMU && rbisk::OP_MEAS == RBIS_OP_MEAS && rbisk::OP_SNAPSHOT == RBIS_OP_SNAPSHOT &&
+              rbisk::OP_RECORD == RBIS_OP_RECORD, "op kinds of the kernels and of the C ABI differ");
+
 constexpr int kMaxSmemOptin = 232448;
-const rbis_fused_tu_t* const kLaneTus[] = {&rbis_fused_tu_dc384, &rbis_fused_tu_dc256, &rbis_fused_tu_dc128};
-const rbis_fused_tu_t* const kGroupTus[] = {&rbis_fused_tu_g2, &rbis_fused_tu_g4, &rbis_fused_tu_g8, &rbis_fused_tu_g16};
+const rbis_fused_tu_t* const kTus[] = {&rbis_fused_tu_dense, &rbis_fused_tu_dc384, &rbis_fused_tu_dc256, &rbis_fused_tu_dc128,
+                                       &rbis_fused_tu_g2,    &rbis_fused_tu_g4,    &rbis_fused_tu_g8,    &rbis_fused_tu_g16};
 const rbis_fused_tu_t* group_tu(int G) {
-  for (const rbis_fused_tu_t* t : kGroupTus)
+  for (const rbis_fused_tu_t* t : kTus)
     if (t->lanes_per_filter == G) return t;
   return nullptr;
 }
+// the decoupled lane-per-filter kernels at tpb filters per CTA
 const rbis_fused_tu_t* lane_tu(int tpb) {
-  for (const rbis_fused_tu_t* t : kLaneTus)
-    if (t->threads == tpb) return t;
+  for (const rbis_fused_tu_t* t : kTus)
+    if (t != &rbis_fused_tu_dense && t->lanes_per_filter == 1 && t->threads == tpb) return t;
   return nullptr;
 }
 
@@ -210,14 +212,14 @@ struct LaunchGeom {
   unsigned grid;        // CTAs for the whole ensemble
   int threads, smem;
   long long fpc;        // filters per CTA
-  const rbis_fused_tu_t* tu;  // nullptr: the dense lane-per-filter kernels of this translation unit
+  const rbis_fused_tu_t* tu;
 };
 LaunchGeom launch_geom(int variant, int mapping, int lane_tpb, long long N, int n_sms) {
   LaunchGeom g{};
   if (mapping <= 1) {
-    g.tu = (variant & 2) ? lane_tu(lane_tpb) : nullptr;
-    g.threads = g.tu ? g.tu->threads : rbisk::TPB;
-    g.smem = g.tu ? g.tu->smem : rbisk::SMEM_BYTES;
+    g.tu = (variant & 2) ? lane_tu(lane_tpb) : &rbis_fused_tu_dense;
+    g.threads = g.tu->threads;
+    g.smem = g.tu->smem;
     g.fpc = g.threads;
   } else {
     // warps per CTA so that the ensemble spreads over all SMs in whole waves
@@ -241,18 +243,7 @@ LaunchGeom launch_geom(int variant, int mapping, int lane_tpb, long long N, int 
 
 // variant bit 3: the program records (REC instantiations)
 cudaError_t launch_variant(int variant, int syn, const LaunchGeom& g, unsigned blocks, cudaStream_t st, const rbisk::KParams& kp) {
-  const int rec = (variant & 8) ? 1 : 0;
-  if (g.tu) return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, rec, blocks, g.threads, g.smem, st, &kp);
-  if (syn) return cudaErrorInvalidValue;  // the dense lane-per-filter kernels have no SYN instantiation
-  if (rec) {
-    if (variant & 1) rbisk::rbis_fused_kernel<true, false, false, true><<<blocks, g.threads, g.smem, st>>>(kp);
-    else rbisk::rbis_fused_kernel<false, false, false, true><<<blocks, g.threads, g.smem, st>>>(kp);
-  } else if (variant & 1) {
-    rbisk::rbis_fused_kernel<true><<<blocks, g.threads, g.smem, st>>>(kp);
-  } else {
-    rbisk::rbis_fused_kernel<false><<<blocks, g.threads, g.smem, st>>>(kp);
-  }
-  return cudaGetLastError();
+  return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, (variant & 8) ? 1 : 0, blocks, g.threads, g.smem, st, &kp);
 }
 
 // Automatic choice of the mapping (rbis_batch_config_t::mapping == 0) from the ensemble size: cycles per filter step of one
@@ -261,34 +252,9 @@ cudaError_t launch_variant(int variant, int syn, const LaunchGeom& g, unsigned b
 struct MappingChoice {
   int mapping, lane_tpb;
 };
-int auto_mapping_lane_only(long long N, int n_sms);
-MappingChoice auto_mapping(long long N, int n_sms) {
-  struct Cand { int mapping, tpb; double cycles; };
-  double best = 1e300;
-  MappingChoice pick{1, 384};
-  auto consider = [&](int mapping, int tpb, double cost) {
-    if (cost < best) { best = cost; pick = {mapping, tpb}; }
-  };
-  auto waves = [&](long long ctas) { return (double)((ctas + n_sms - 1) / n_sms); };
-  // lane-per-filter: one CTA per SM; large ensembles overlap their waves through the launch groups, so beyond one wave
-  // the cost grows with the CTA count, not with whole waves
-  const struct { int tpb; double cyc; } lane[] = {{384, 16200.0}, {256, 12500.0}, {128, 9300.0}};
-  for (const auto& k : lane) {
-    const long long ctas = (N + k.tpb - 1) / k.tpb;
-    const double w = ctas <= n_sms ? 1.0 : (k.tpb == 384 ? (double)ctas / n_sms : waves(ctas));
-    consider(1, k.tpb, w * k.cyc);
-  }
-  // warp groups of 4 lanes: one wave holds n_sms * 8 warps * 8 filters; cost grows with the warps per CTA
-  {
-    const long long warps = (N + 7) / 8;
-    const long long wv = (warps + (long long)n_sms * 8 - 1) / ((long long)n_sms * 8);
-    const double wpc = (double)((warps + n_sms * wv - 1) / (n_sms * wv));
-    consider(4, 384, (double)wv * (4300.0 + 560.0 * wpc));
-  }
-  return pick;
-}
-
-int auto_mapping_lane_only(long long N, int n_sms) {
+// The decoupled lane-per-filter kernels of least cost (filters per CTA), and that cost.  One CTA per SM; large ensembles
+// overlap their waves through the launch groups, so beyond one wave the cost grows with the CTA count, not with whole waves.
+int auto_lane_tpb(long long N, int n_sms, double* cost = nullptr) {
   const struct { int tpb; double cyc; } lane[] = {{384, 16200.0}, {256, 12500.0}, {128, 9300.0}};
   double best = 1e300;
   int pick = 384;
@@ -297,6 +263,17 @@ int auto_mapping_lane_only(long long N, int n_sms) {
     const double w = ctas <= n_sms ? 1.0 : (k.tpb == 384 ? (double)ctas / n_sms : (double)((ctas + n_sms - 1) / n_sms));
     if (w * k.cyc < best) { best = w * k.cyc; pick = k.tpb; }
   }
+  if (cost) *cost = best;
+  return pick;
+}
+MappingChoice auto_mapping(long long N, int n_sms) {
+  double best;
+  MappingChoice pick{1, auto_lane_tpb(N, n_sms, &best)};
+  // warp groups of 4 lanes: one wave holds n_sms * 8 warps * 8 filters; cost grows with the warps per CTA
+  const long long warps = (N + 7) / 8;
+  const long long wv = (warps + (long long)n_sms * 8 - 1) / ((long long)n_sms * 8);
+  const double wpc = (double)((warps + n_sms * wv - 1) / (n_sms * wv));
+  if ((double)wv * (4300.0 + 560.0 * wpc) < best) pick = {4, 384};
   return pick;
 }
 
@@ -484,11 +461,10 @@ int r_table(const double* R, const rbisk::StreamDesc& d, double* out) {
 extern "C" int synthesize_into(rbis_batch_t* h, const rbis_synth_t* syn, double* imu_out, double* const* z_out, double* const* quat_out, cudaStream_t stream);
 namespace {
 
-// dry_run: validate the whole call (ops, streams) and return without enqueueing anything.
 // syn != nullptr: the input rows are synthesised on the device into the staging slot (rbis_batch_run_fused_synth) instead of
 // being copied from the host; everything else -- double buffering, overlap with the previous launch -- is the host path's.
 int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const double* imu, int64_t imu_rows,
-                 int n_streams, const rbis_stream_t* streams_in, int mem, bool use_maps = true, bool dry_run = false,
+                 int n_streams, const rbis_stream_t* streams_in, int mem, bool use_maps = true,
                  const rbis_synth_t* syn = nullptr) {
   if (!h) return fail(RBIS_ERR_INVALID, "null handle");
   if (n_ops < 0 || (n_ops > 0 && !ops)) return fail(RBIS_ERR_INVALID, "bad op list");
@@ -567,12 +543,6 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
       default:
         return fail(RBIS_ERR_INVALID, "op %lld: unknown kind %d", (long long)i, o.kind);
     }
-  }
-
-  if (dry_run) {
-    for (int s = 0; s < n_streams; s++)
-      if (int rc = validate_stream(s, streams[s])) return rc;
-    return 0;
   }
 
   rbisk::KParams kp;
@@ -1020,22 +990,19 @@ int rbis_batch_create(rbis_batch_t** out, int64_t n_filters, const rbis_batch_co
   CUDA_TRY(cudaGetDeviceProperties(&prop, c.device));
   if (prop.major != 10)
     return fail(RBIS_ERR_CUDA, "device %d is sm_%d%d; this library is built for sm_100a (B200) only", c.device, prop.major, prop.minor);
-  if ((int)prop.sharedMemPerBlockOptin < kSmemBytes)
-    return fail(RBIS_ERR_CUDA, "device offers %zu B shared memory per block, %d needed", prop.sharedMemPerBlockOptin, kSmemBytes);
+  if ((int)prop.sharedMemPerBlockOptin < rbis_fused_tu_dense.smem)
+    return fail(RBIS_ERR_CUDA, "device offers %zu B shared memory per block, %d needed", prop.sharedMemPerBlockOptin, rbis_fused_tu_dense.smem);
 
   rbis_batch* h = new (std::nothrow) rbis_batch();
   if (!h) return fail(RBIS_ERR_ALLOC, "host allocation failed");
   h->N = n_filters;
   h->cfg = c;
-  h->smem_bytes = kSmemBytes;
   h->n_sms = prop.multiProcessorCount;
   {
     const MappingChoice mc = auto_mapping(n_filters, h->n_sms);
     h->mapping = c.mapping ? c.mapping : mc.mapping;
-    h->lane_tpb = c.lane_filters_per_cta ? c.lane_filters_per_cta : (c.mapping == 1 ? auto_mapping_lane_only(n_filters, h->n_sms) : mc.lane_tpb);
-    for (const rbis_fused_tu_t* t : kLaneTus)
-      if (t->kparams_bytes != sizeof(rbisk::KParams)) { fail(RBIS_ERR_CUDA, "kernel parameter block mismatch between translation units"); rbis_batch_destroy(h); return RBIS_ERR_CUDA; }
-    for (const rbis_fused_tu_t* t : kGroupTus)
+    h->lane_tpb = c.lane_filters_per_cta ? c.lane_filters_per_cta : (c.mapping == 1 ? auto_lane_tpb(n_filters, h->n_sms) : mc.lane_tpb);
+    for (const rbis_fused_tu_t* t : kTus)
       if (t->kparams_bytes != sizeof(rbisk::KParams)) { fail(RBIS_ERR_CUDA, "kernel parameter block mismatch between translation units"); rbis_batch_destroy(h); return RBIS_ERR_CUDA; }
   }
   const size_t N = (size_t)n_filters;
@@ -1053,7 +1020,8 @@ int rbis_batch_create(rbis_batch_t** out, int64_t n_filters, const rbis_batch_co
   CREATE_TRY(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
   {
     // launch groups: explicit, or automatic = 6 when the CTAs do not fill a whole number of waves (measured: 2 groups 2.12, 3: 1.92, 4: 1.89, 6: 1.865, 8: 1.88 ms per launch)
-    const long long ctas = (long long)((n_filters + rbisk::TPB - 1) / rbisk::TPB), sms = prop.multiProcessorCount;
+    const int dense_tpb = rbis_fused_tu_dense.threads;
+    const long long ctas = (long long)((n_filters + dense_tpb - 1) / dense_tpb), sms = prop.multiProcessorCount;
     const long long ctas_dc = (long long)((n_filters + h->lane_tpb - 1) / h->lane_tpb);
     int g = c.launch_groups;
     if (g == 0) g = (h->mapping == 1 && ((ctas > sms && ctas % sms != 0) || (!c.dense_only && ctas_dc > sms && ctas_dc % sms != 0))) ? 6 : 1;
@@ -1095,12 +1063,7 @@ int rbis_batch_create(rbis_batch_t** out, int64_t n_filters, const rbis_batch_co
   }
   CREATE_TRY(cudaMalloc(&h->d_flag, sizeof(int)));
   CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_smooth_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, rbisk::SMOOTH_SMEM_BYTES));
-  CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  CREATE_TRY(cudaFuncSetAttribute(rbisk::rbis_fused_kernel<false, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemBytes));
-  for (const rbis_fused_tu_t* t : kLaneTus) CREATE_TRY(t->prepare());
-  for (const rbis_fused_tu_t* t : kGroupTus) CREATE_TRY(t->prepare());
+  for (const rbis_fused_tu_t* t : kTus) CREATE_TRY(t->prepare());
   // default state: zeros, identity quaternion, zero covariance, zero process noise
   CREATE_TRY(cudaMemsetAsync(h->vec, 0, N * 21 * sizeof(double), h->stream));
   CREATE_TRY(cudaMemsetAsync(h->quat, 0, N * 4 * sizeof(double), h->stream));
@@ -1453,7 +1416,7 @@ int rbis_batch_run_fused_synth(rbis_batch_t* h, int64_t n_ops, const rbis_op_t* 
   if (!h) return fail(RBIS_ERR_INVALID, "null handle");
   if (!syn) return fail(RBIS_ERR_INVALID, "syn is NULL");
   if (n_streams > 0 && !streams) return fail(RBIS_ERR_INVALID, "streams is NULL");
-  return launch_fused(h, n_ops, ops, nullptr, 0, n_streams, streams, RBIS_MEM_DEVICE, true, false, syn);
+  return launch_fused(h, n_ops, ops, nullptr, 0, n_streams, streams, RBIS_MEM_DEVICE, true, syn);
 }
 
 int rbis_batch_ins_step(rbis_batch_t* h, const double* gyro, const double* accel, double dt, int64_t utime, int mem) {

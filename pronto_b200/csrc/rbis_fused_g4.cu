@@ -2,5 +2,4 @@
 #define RBIS_TU_NAME g4
 #define RBIS_TU_NS rbisk_g4
 #define RBIS_TU_GROUP 4
-#define RBIS_GROUP_STATE_FIRST 0
 #include "rbis_fused_tu.inc"

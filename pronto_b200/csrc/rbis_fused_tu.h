@@ -5,7 +5,6 @@
 #include <cstddef>
 struct rbis_fused_tu_t {
   int lanes_per_filter;  // 1: lane-per-filter kernels; 2/4/8/16: warp-group kernels
-  int decoupled;         // 1: decoupled kernels only; 2: both decoupled and dense
   int threads, smem;     // lane-per-filter kernels: fixed launch shape
   int max_warps;         // warp-group kernels: warps per CTA at most
   int filters_per_warp;
@@ -13,13 +12,14 @@ struct rbis_fused_tu_t {
   size_t kparams_bytes;
   cudaError_t (*prepare)();
   // blocks_variant: the program has one-row / correlated chunks (lane-per-filter kernels: instantiation with those paths)
+  // decoupled: which kernels of a warp-group unit (it holds both); a lane-per-filter unit holds either kind and ignores it
   // syn: the SYN instantiation (input rows drawn inside the kernel, KParams::syn); decoupled kernels without blocks_variant only
   // rec: the REC instantiation (the program has RBIS_OP_RECORD ops, KParams::rec)
   cudaError_t (*launch)(int blocks_variant, int decoupled, int syn, int rec, unsigned grid, int threads, int smem, cudaStream_t st,
                         const void* kparams);
 };
 extern "C" {
-extern const rbis_fused_tu_t rbis_fused_tu_dc384, rbis_fused_tu_dc256, rbis_fused_tu_dc128;
+extern const rbis_fused_tu_t rbis_fused_tu_dense, rbis_fused_tu_dc384, rbis_fused_tu_dc256, rbis_fused_tu_dc128;
 extern const rbis_fused_tu_t rbis_fused_tu_g2, rbis_fused_tu_g4, rbis_fused_tu_g8, rbis_fused_tu_g16;
 }
 #endif

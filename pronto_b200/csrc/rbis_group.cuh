@@ -25,12 +25,9 @@
 // Lanes synchronise with __syncwarp() only; a CTA is any number of warps (chosen by the host so that the ensemble
 // spreads over all SMs), there is no CTA-wide barrier and no tensor memory.
 //
-// Included by rbis_batch.cu after the first (default-configuration) inclusion of rbis_kernels.cuh.
+// Included after rbis_kernels.cuh, into the same namespace, by the warp-group translation units (rbis_fused_g*.cu).
 #ifndef RBIS_GROUP_CUH_
 #define RBIS_GROUP_CUH_
-#ifndef RBIS_GROUP_STATE_FIRST
-#define RBIS_GROUP_STATE_FIRST 0  // insUpdateState before (1) or after (0) the covariance passes of an IMU step (dev knob; 0 measured 5-10 % faster)
-#endif
 
 namespace rbisk {
 namespace grp {
@@ -382,10 +379,6 @@ __device__ __forceinline__ void g_meas3(double* Pf, const int l, FilterState& s,
   }
   g_sweep<G, DC, 3>(Pf, w, Y, wj);
   __syncwarp();
-#ifdef RBIS_GROUP_COVONLY
-  s.ll += logdet + z[0] + z[1] + z[2] + Y[0][3] + Y[1][7] + Y[2][11];
-  return;
-#endif
   double r[3];
   if (I0 == 6 && st.has_orient) {
     r[0] = dquat.x - (s.x[6] - chi0.x); r[1] = dquat.y - (s.x[7] - chi0.y); r[2] = dquat.z - (s.x[8] - chi0.z);
@@ -640,11 +633,11 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
     syn_sa = p.syn.sigma_accel >= 0 ? p.syn.sigma_accel : sqrt(__ldg(p.q_accel + n) / p.syn.dt);
   }
   auto prefetch_inputs = [&](const Op& o) {
-    if (o.kind == 0) {
+    if (o.kind == OP_IMU) {
       const double* base = p.imu + o.row * 6 * p.imu_cols + imu_n;
 #pragma unroll
       for (int k = 0; k < 6; k++) prefetch(base + k * p.imu_cols);
-    } else if (o.kind == 1) {
+    } else if (o.kind == OP_MEAS) {
       const StreamDesc& st = p.streams[o.stream];
       const long long sn = st.map ? (long long)__ldg(st.map + n) : n;
       const double* zb = st.z + o.row * st.m * st.cols + sn;
@@ -665,7 +658,7 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
     if constexpr (!SYN) {
       if (oi + 1 < p.n_ops) prefetch_inputs(op1);
     }
-    if (op.kind == 0) {
+    if (op.kind == OP_IMU) {
       // ---- IMU process step: same linearisation / state code as the lane-per-filter kernel ----
       const double* base = p.imu + op.row * 6 * p.imu_cols + imu_n;
       const long long Ni = p.imu_cols;
@@ -707,16 +700,9 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
         s.x[11] += fma(R22, vz, fma(R21, vy, R20 * vx)) * dt;
       }
       imu_seen = true;
-      // the state step only needs the prior state (already captured in L): issued first, its long dependent chain
-      // (rsqrt, sin / cos, quaternion product) overlaps the covariance passes
-#if RBIS_GROUP_STATE_FIRST && !defined(RBIS_GROUP_COVONLY)
-      state_propagate<true>(s, gyro, acc, dt, gb, p.chi_tol, p.renorm);
-#endif
       g_cov_propagate<G, DC>(Pf, l, L, qn);
-#if !RBIS_GROUP_STATE_FIRST && !defined(RBIS_GROUP_COVONLY)
-      state_propagate<true>(s, gyro, acc, dt, gb, p.chi_tol, p.renorm);
-#endif
-    } else if (op.kind == 1) {
+      state_propagate(s, gyro, acc, dt, gb, p.chi_tol, p.renorm);
+    } else if (op.kind == OP_MEAS) {
       // ---- indexed / indexed-plus-orientation measurement ----
       const StreamDesc& st = p.streams[op.stream];
       const long long sn = st.map ? (long long)__ldg(st.map + n) : n;
@@ -735,10 +721,8 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
         else if (fast >= 100) g_meas1<G, DC>(Pf, l, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0);
         else g_meas_block<G, DC>(Pf, l, s, st, src, a0, st.chunk_len[ci], op.row, sn, dquat, chi0);
       }
-#ifndef RBIS_GROUP_COVONLY
       meas_finish(s, chi0, p.chi_tol, p.ctor_folds_chi, p.renorm);
-#endif
-    } else if (op.kind == 2) {
+    } else if (op.kind == OP_SNAPSHOT) {
       // ---- snapshot into ring slot ----
       double* d = p.snap + op.row * SNAP_ROWS * N + n;
       if (writer) {
@@ -760,7 +744,7 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
       }
     } else {
       if constexpr (REC) {
-        if (op.kind == 4) {
+        if (op.kind == OP_RECORD) {
           // ---- record the chosen fields into record row op.row ----
           g_record_fields<G, DC>(p, Pf, l, s, qn, op.row, n, active, imu_seen);
           continue;
