@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """dev/all_kernels_check.py -- one small pass through every fused-kernel family with a bit-identity check (compute-sanitizer is closed on the GPU pool):
-lane-per-filter decoupled + dense, warp-group 4 / 8 lanes, SYN instantiations, snapshot / restore, snapshot statistics, and the
-REC instantiations (RBIS_OP_RECORD) over the same mappings and variants."""
+lane-per-filter decoupled + dense, warp-group 4 / 8 lanes, SYN instantiations, snapshot / restore, snapshot statistics, the
+REC instantiations (RBIS_OP_RECORD) and the MASK instantiations (RBIS_STREAM_SKIP_NAN_ROWS, with and without records) over the
+same mappings and variants."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -87,4 +88,39 @@ for cfg in (dict(mapping=1), dict(mapping=4), dict(mapping=8), dict(mapping=1, s
     same = np.array_equal(rec, ref_rec) and not np.isnan(rec).any()
     print("record synth", cfg, "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
     assert same and variant & 8
+# missing rows: per-filter NaN dropouts on both streams through the MASK (and MASK + REC) instantiations; a flagged program
+# without NaN gives the unflagged bits
+rng = np.random.default_rng(3)
+lego, pose_z = st["legodo"].copy(), st["pose_z"].copy()
+lego[rng.random(lego.shape) < 0.1] = np.nan
+pose_z[:, 0][rng.random(pose_z[:, 0].shape) < 0.2] = np.nan
+
+
+def masked(z_lego, z_pose):
+    return [MeasStream(synth.LEGODO_IDX, z_lego, st["R_legodo"], skip_nan_rows=True),
+            MeasStream(synth.POSE_IDX, z_pose, st["R_pose"], quat=st["pose_q"], skip_nan_rows=True)]
+
+
+ref_mask = None
+for cfg in (dict(mapping=1, lane_filters_per_cta=384), dict(mapping=1, lane_filters_per_cta=128), dict(mapping=1, dense_only=True),
+            dict(mapping=4), dict(mapping=8), dict(mapping=4, dense_only=True)):
+    for with_rec in (False, True):
+        out = torch.full((rows, capi.REC_FIELDS, N), float("nan"), dtype=torch.float64, device="cuda")
+        with RBISBatch(N, snapshot_slots=2, **cfg) as b:
+            b.set_process_noise(*nominal_q())
+            b.set_state(sc["vec"], sc["quat"], sc["cov"])
+            b.run_fused(prog, imu=st["imu"], streams=masked(st["legodo"], st["pose_z"]))
+            clean = b.get_state()
+            b.set_state(sc["vec"], sc["quat"], sc["cov"])
+            if with_rec:
+                b.set_record(out, ALL)
+            b.run_fused(rec_prog if with_rec else prog, imu=st["imu"], streams=masked(lego, pose_z))
+            variant = b.last_kernel_variant
+            got = b.get_state()
+        if ref_mask is None:
+            ref_mask = got
+        same = all(np.array_equal(x, y) for x, y in zip(got[:4], ref_mask[:4])) and all(np.array_equal(x, y) for x, y in zip(clean[:4], ref_state[:4]))
+        same = same and not np.isnan(got[0]).any()
+        print("masked", cfg, "records" if with_rec else "", "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
+        assert same and variant & 512
 print("ok")

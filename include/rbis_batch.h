@@ -140,12 +140,24 @@ typedef struct {
   int32_t r_mode;                 /* rbis_r_mode_t */
   int32_t sensor_id;              /* RBISUpdateInterface::sensor_enum value, carried only */
   int32_t idx[RBIS_MAX_MEAS];     /* state indices, 0..20 */
-  int32_t reserved;
+  int32_t flags;                  /* RBIS_STREAM_* bits; 0 = none (every other bit is rejected) */
   const double* z;                /* [rows][m][N]; entries at chi indices are ignored when has_orientation */
   const double* quat;             /* [rows][4][N] or NULL */
   const double* R;                /* see rbis_r_mode_t */
   int64_t rows;
 } rbis_stream_t;
+
+/* rbis_stream_t::flags.
+ * RBIS_STREAM_SKIP_NAN_ROWS: rows that some filters did not receive (sensor dropouts that differ from one realisation to the next,
+ *   logs whose gaps fall in different places).  Row r is MISSING for filter n when any z value the update reads in filter n's
+ *   column -- the column-map column where a map is set -- is NaN; the chi entries of an orientation stream are not read and do not
+ *   count, quat is not inspected.  For that filter the RBIS_OP_MEAS op of row r does nothing: state, quaternion, covariance and
+ *   log-likelihood keep their bits, and no addState runs (so renormalize_quat does not renormalise either).  Every other filter,
+ *   the ensemble's utime, SNAPSHOT, RESTORE and RECORD proceed as usual.  Hence for an in-order or planner-built program, filter n
+ *   ends exactly where the same program ends with the MEAS ops of its missing rows deleted.  Without the flag a NaN is used
+ *   as a value (and poisons the filter).  rbis_batch_run_fused only (any mem, r_mode, chunk kind, column map, mapping);
+ *   rbis_batch_run_fused_synth rejects it, its rows are drawn, not read. */
+#define RBIS_STREAM_SKIP_NAN_ROWS 1
 
 typedef struct {
   int32_t kind;    /* rbis_op_kind_t */
@@ -175,7 +187,8 @@ int64_t rbis_batch_launch_count(const rbis_batch_t* h);
  * triples (the instantiations that also contain the one-row and the correlated-block updates), +4 when the kernel drew its
  * input rows itself (rbis_batch_run_fused_synth, SYN instantiations), + 16 * lanes per filter for the warp-group kernels
  * (rbis_batch_config_t::mapping > 1), +8 when the program records (RBIS_OP_RECORD: the REC instantiations, which programs without
- * records never run); -1 before the first launch. */
+ * records never run), +512 when a stream has RBIS_STREAM_SKIP_NAN_ROWS (the MASK instantiations, which contain the one-row and
+ * correlated-block updates whatever +1 says); -1 before the first launch. */
 int rbis_batch_last_kernel_variant(const rbis_batch_t* h);
 
 /* ---- RBISResetUpdate::updateFilter (MSE/rbis_update_interface.cpp:23-28): posterior := given,
@@ -319,7 +332,10 @@ int rbis_batch_run_fused_synth(rbis_batch_t* h, int64_t n_ops, const rbis_op_t* 
  *
  * ONE SCHEDULE PER HANDLE.  A planner serves one rbis_batch_t: all of its filters see the same arrivals in the same order --
  * the shape of every workload in BASELINE.json (a noise sweep or a parameter sweep replays ONE log; delayed pose fixes are
- * late for every realisation alike).  Filters whose measurements arrive on DIFFERENT schedules belong in different handles,
+ * late for every realisation alike).  One schedule, but rows may be MISSING per filter: with RBIS_STREAM_SKIP_NAN_ROWS a
+ * filter whose row is NaN skips that update, so dropouts that differ between realisations stay in one handle and one
+ * planner (the program is planned as if every filter received every row).  Filters whose measurements arrive in a
+ * different ORDER or with different latency belong in different handles,
  * one planner each: handles are independent (own streams, own snapshot ring), their launches run concurrently on the device,
  * and the warp-group kernels keep small sub-ensembles efficient; tests/test_gpu_parity.py
  * (test_two_arrival_schedules_as_two_handles) runs two schedules side by side against the oracle's per-filter histories. */

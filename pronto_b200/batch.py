@@ -64,13 +64,18 @@ class MeasStream:
     (MSE/rbis_update_interface.hpp:84-120): index set, z rows, R, optional orientation rows.
 
     R: one m x m matrix for every row; or [rows][m][m], row r's matrix for the update that reads row r
-    (RBIS_R_PER_ROW_FULL); or [m][N] per-filter diagonals with per_filter_diag=True."""
+    (RBIS_R_PER_ROW_FULL); or [m][N] per-filter diagonals with per_filter_diag=True.
 
-    def __init__(self, idx, z, R, quat=None, per_filter_diag=False, sensor_id=0):
+    skip_nan_rows=True (RBIS_STREAM_SKIP_NAN_ROWS): a filter whose row holds a NaN in a value the update reads (z[row, :, n],
+    without the chi entries of an orientation stream) did not receive that row and skips the update, bit for bit as if its
+    MEAS op were deleted from the program.  run_fused only."""
+
+    def __init__(self, idx, z, R, quat=None, per_filter_diag=False, sensor_id=0, skip_nan_rows=False):
         self.idx = [int(i) for i in idx]
         self.z, self.R, self.quat = z, R, quat
         self.per_filter_diag = bool(per_filter_diag)
         self.sensor_id = int(sensor_id)
+        self.skip_nan_rows = bool(skip_nan_rows)
 
 
 class SynthSpec:
@@ -364,6 +369,7 @@ class RBISBatch:
             m = len(st.idx)
             d = sarr[s]
             d.m, d.has_orientation, d.sensor_id = m, int(st.quat is not None), st.sensor_id
+            d.flags = capi.STREAM_SKIP_NAN_ROWS if st.skip_nan_rows else 0
             d.r_mode = capi.R_PER_FILTER_DIAG if st.per_filter_diag else capi.R_SHARED_FULL
             for a, i in enumerate(st.idx):
                 d.idx[a] = i
@@ -437,6 +443,7 @@ class RBISBatch:
             m = len(st.idx)
             d = sarr[s]
             d.m, d.has_orientation, d.sensor_id = m, int(st.quat is not None), st.sensor_id
+            d.flags = capi.STREAM_SKIP_NAN_ROWS if st.skip_nan_rows else 0   # rejected by the library: rows are drawn, not read
             d.r_mode = capi.R_PER_FILTER_DIAG if st.per_filter_diag else capi.R_SHARED_FULL
             for a, i in enumerate(st.idx):
                 d.idx[a] = i
@@ -483,7 +490,8 @@ class RBISBatch:
     @property
     def last_kernel_variant(self):
         """0 dense, 2 decoupled (rbis_batch_config_t::dense_only), +1 with correlated-row chunks, +4 input rows drawn in the
-        kernel, +8 a program with RBIS_OP_RECORD ops, +16 * lanes per filter for the warp-group kernels; -1 before any launch."""
+        kernel, +8 a program with RBIS_OP_RECORD ops, +16 * lanes per filter for the warp-group kernels, +512 a stream that skips
+        NaN rows (MeasStream skip_nan_rows); -1 before any launch."""
         return int(self.lib.rbis_batch_last_kernel_variant(self.h))
 
     @property

@@ -20,6 +20,7 @@ MEM_F32_ROWS = 4  # rbis_batch_run_fused: imu / z / quat are float32 arrays (wid
 OP_IMU, OP_MEAS, OP_SNAPSHOT, OP_RESTORE, OP_RECORD = 0, 1, 2, 3, 4
 REC_FIELDS = 47  # record fields: 0..20 vec, 21..24 quat w,x,y,z, 25 loglik, 26..46 covariance diagonal
 R_SHARED_FULL, R_PER_FILTER_DIAG, R_PER_ROW_FULL = 0, 1, 2
+STREAM_SKIP_NAN_ROWS = 1  # rbis_stream_t::flags: a filter whose row holds a NaN in a value the update reads skips that update
 
 c_double_p = C.POINTER(C.c_double)
 c_int32_p = C.POINTER(C.c_int32)
@@ -50,7 +51,7 @@ class Stream(C.Structure):
         ("r_mode", C.c_int32),
         ("sensor_id", C.c_int32),
         ("idx", C.c_int32 * MAX_MEAS),
-        ("reserved", C.c_int32),
+        ("flags", C.c_int32),
         ("z", C.c_void_p),
         ("quat", C.c_void_p),
         ("R", C.c_void_p),

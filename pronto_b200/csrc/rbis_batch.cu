@@ -241,9 +241,11 @@ LaunchGeom launch_geom(int variant, int mapping, int lane_tpb, long long N, int 
   return g;
 }
 
-// variant bit 3: the program records (REC instantiations)
+// variant bit 3: the program records (REC instantiations); bit 9 (+512): a stream skips NaN rows (MASK instantiations)
+constexpr int kVariantMask = 512;
 cudaError_t launch_variant(int variant, int syn, const LaunchGeom& g, unsigned blocks, cudaStream_t st, const rbisk::KParams& kp) {
-  return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, (variant & 8) ? 1 : 0, blocks, g.threads, g.smem, st, &kp);
+  return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, (variant & 8) ? 1 : 0, (variant & kVariantMask) ? 1 : 0, blocks, g.threads,
+                      g.smem, st, &kp);
 }
 
 // Automatic choice of the mapping (rbis_batch_config_t::mapping == 0) from the ensemble size: cycles per filter step of one
@@ -444,6 +446,7 @@ int validate_stream(int s, const rbis_stream_t& in) {
   if (in.has_orientation && in.rows > 0 && !in.quat) return fail(RBIS_ERR_INVALID, "stream %d: has_orientation but quat is NULL", s);
   if (in.r_mode != RBIS_R_SHARED_FULL && in.r_mode != RBIS_R_PER_FILTER_DIAG && in.r_mode != RBIS_R_PER_ROW_FULL)
     return fail(RBIS_ERR_INVALID, "stream %d: bad r_mode", s);
+  if (in.flags & ~RBIS_STREAM_SKIP_NAN_ROWS) return fail(RBIS_ERR_INVALID, "stream %d: unknown flags 0x%x", s, (unsigned)in.flags);
   return 0;
 }
 
@@ -571,6 +574,10 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     const rbis_stream_t& in = streams[s];
     rbisk::StreamDesc& d = kp.streams[s];
     if (int rc = validate_stream(s, in)) return rc;
+    if (in.flags & RBIS_STREAM_SKIP_NAN_ROWS) {
+      if (syn) return fail(RBIS_ERR_INVALID, "stream %d: RBIS_STREAM_SKIP_NAN_ROWS does not apply to synthesised inputs (z is drawn, not read)", s);
+      kp.skip_nan_streams |= 1u << s;
+    }
     d.m = in.m; d.has_orient = in.has_orientation ? 1 : 0; d.r_mode = in.r_mode;
     for (int a = 0; a < in.m; a++) d.idx[a] = in.idx[a];
     d.map = use_maps ? h->d_map[1 + s] : nullptr;
@@ -609,7 +616,8 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     }
   }
   // ---- kernel variant ----
-  int variant = needs_general ? 1 : 0;
+  // skipping a row changes no coupling, so decoupled eligibility does not depend on the MASK instantiations
+  int variant = (needs_general ? 1 : 0) | (kp.skip_nan_streams ? kVariantMask : 0);
   const bool dc_eligible = !h->cfg.dense_only && !passive_index && restores_ok;
   if (dc_eligible && h->decoupled < 0) {
     // one device pass over the couplings, then a host read: happens once after set_state / set_filter, not per launch

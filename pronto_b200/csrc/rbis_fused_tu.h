@@ -15,7 +15,8 @@ struct rbis_fused_tu_t {
   // decoupled: which kernels of a warp-group unit (it holds both); a lane-per-filter unit holds either kind and ignores it
   // syn: the SYN instantiation (input rows drawn inside the kernel, KParams::syn); decoupled kernels without blocks_variant only
   // rec: the REC instantiation (the program has RBIS_OP_RECORD ops, KParams::rec)
-  cudaError_t (*launch)(int blocks_variant, int decoupled, int syn, int rec, unsigned grid, int threads, int smem, cudaStream_t st,
+  // mask: the MASK instantiation (a stream of the program has RBIS_STREAM_SKIP_NAN_ROWS, KParams::skip_nan_streams); not with syn
+  cudaError_t (*launch)(int blocks_variant, int decoupled, int syn, int rec, int mask, unsigned grid, int threads, int smem, cudaStream_t st,
                         const void* kparams);
 };
 extern "C" {

@@ -300,10 +300,11 @@ __device__ __forceinline__ void g_cov_propagate(double* Pf, const int l, const L
 // triangle: the expression of rbisk::meas3 / rank1_sweep element for element.  NY = rows of Y (3 or 1).  wj[j][a] = the
 // lane's own Y[a][c_j] * r_a, formed BEFORE the barrier that precedes the sweep (a mirrored store of another lane may
 // overwrite the lower-triangle element it was read from).  Column slot j only visits rows k < G (j + 1): the rest lie
-// below the diagonal for every lane.
-template <int G, bool DC, int NY>
+// below the diagonal for every lane.  MASK, skip: the filter's row is missing, its lanes store back the values they loaded
+// (the matrix keeps its bits); the G lanes of a group read the same z, so they agree on skip.
+template <int G, bool DC, int NY, bool MASK = false>
 __device__ __forceinline__ void g_sweep(double* Pf, const Own<G, Geo<G, DC>::NA>& w, const double (&Y)[NY][Geo<G, DC>::NA],
-                                        const double (&wj)[Geo<G, DC>::NJ][NY]) {
+                                        const double (&wj)[Geo<G, DC>::NJ][NY], bool skip = false) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   static_for<NJ>([&](auto jc) {
@@ -320,6 +321,7 @@ __device__ __forceinline__ void g_sweep(double* Pf, const Own<G, Geo<G, DC>::NA>
       double acc = v[k];
 #pragma unroll
       for (int a = NY - 1; a >= 0; a--) acc = fma(-Y[a][k], wj[j][a], acc);
+      if constexpr (MASK) acc = skip ? v[k] : acc;
       if (w.own[j] && (k < G * j || k <= c)) { b[k * LD] = acc; m[k] = acc; }
     }
   });
@@ -327,9 +329,10 @@ __device__ __forceinline__ void g_sweep(double* Pf, const Own<G, Geo<G, DC>::NA>
 
 // Aligned index triple I0..I0+2 (leg-odometry velocity, pose position / orientation, ...): rbis.cpp:124-143 with
 // S = L D L^T, Y = L^-1 P[idx,:], P -= Y^T D^-1 Y, x += Y^T D^-1 L^-1 r.  Same arithmetic as rbisk::meas3.
-template <int G, bool DC, bool SYN>
+template <int G, bool DC, bool SYN, bool MASK = false>
 __device__ __forceinline__ void g_meas3(double* Pf, const int l, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int I0,
-                                        long long row, long long N, long long n, long long sn, const V3& dquat, const V3& chi0) {
+                                        long long row, long long N, long long n, long long sn, const V3& dquat, const V3& chi0,
+                                        bool skip = false) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   double z[3], Rdg[3];
@@ -377,7 +380,7 @@ __device__ __forceinline__ void g_meas3(double* Pf, const int l, FilterState& s,
     const double y2 = fma(-l21, y1, fma(-l20, yo[j][0], yo[j][2]));
     wj[j][0] = yo[j][0] * r0; wj[j][1] = y1 * r1; wj[j][2] = y2 * r2;
   }
-  g_sweep<G, DC, 3>(Pf, w, Y, wj);
+  g_sweep<G, DC, 3, MASK>(Pf, w, Y, wj, skip);
   __syncwarp();
   double r[3];
   if (I0 == 6 && st.has_orient) {
@@ -390,15 +393,18 @@ __device__ __forceinline__ void g_meas3(double* Pf, const int l, FilterState& s,
   static_for<NA>([&](auto cc) {
     constexpr int c = cc;
     constexpr int xc = idx_of<DC>(c);
-    s.x[xc] = fma(Y[0][c], u0, fma(Y[1][c], u1, fma(Y[2][c], u2, s.x[xc])));
+    if constexpr (MASK) s.x[xc] = skip ? s.x[xc] : fma(Y[0][c], u0, fma(Y[1][c], u1, fma(Y[2][c], u2, s.x[xc])));
+    else s.x[xc] = fma(Y[0][c], u0, fma(Y[1][c], u1, fma(Y[2][c], u2, s.x[xc])));
   });
-  s.ll += -logdet - fma(e2, u2, fma(e1, u1, e0 * u0));
+  if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-logdet - fma(e2, u2, fma(e1, u1, e0 * u0)));
+  else s.ll += -logdet - fma(e2, u2, fma(e1, u1, e0 * u0));
 }
 
 // One-row chunk on state index idx (rbisk::meas1).
-template <int G, bool DC, bool SYN>
+template <int G, bool DC, bool SYN, bool MASK = false>
 __device__ __forceinline__ void g_meas1(double* Pf, const int l, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int idx,
-                                        long long row, long long N, long long n, long long sn, const V3& dquat, const V3& chi0) {
+                                        long long row, long long N, long long n, long long sn, const V3& dquat, const V3& chi0,
+                                        bool skip = false) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   const double z = src.z(st, row, a0, sn);
@@ -417,7 +423,7 @@ __device__ __forceinline__ void g_meas1(double* Pf, const int l, FilterState& s,
   const double r = 1.0 / sv;
 #pragma unroll
   for (int j = 0; j < NJ; j++) wj[j][0] *= r;
-  g_sweep<G, DC, 1>(Pf, w, h, wj);
+  g_sweep<G, DC, 1, MASK>(Pf, w, h, wj, skip);
   __syncwarp();
   double rr;
   if (st.has_orient && idx >= 6 && idx <= 8) {
@@ -432,16 +438,18 @@ __device__ __forceinline__ void g_meas1(double* Pf, const int l, FilterState& s,
   static_for<NA>([&](auto cc) {
     constexpr int c = cc;
     constexpr int xc = idx_of<DC>(c);
-    s.x[xc] = fma(h[0][c], u, s.x[xc]);
+    if constexpr (MASK) s.x[xc] = skip ? s.x[xc] : fma(h[0][c], u, s.x[xc]);
+    else s.x[xc] = fma(h[0][c], u, s.x[xc]);
   });
-  s.ll += -log(sv) - rr * u;
+  if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rr * u);
+  else s.ll += -log(sv) - rr * u;
 }
 
 // A chunk of M correlated rows, decorrelated by the host (rbisk::meas_block): M scalar updates with rows
 // H'_a = sum_{b<=a} w_ab H_b and noise D_a.
-template <int G, bool DC, bool SYN>
+template <int G, bool DC, bool SYN, bool MASK = false>
 __device__ __forceinline__ void g_meas_block(double* Pf, const int l, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int M,
-                                             long long row, long long sn, const V3& dquat, const V3& chi0) {
+                                             long long row, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   const double* W = st.R + row * st.r_stride + RS_W;
@@ -487,15 +495,17 @@ __device__ __forceinline__ void g_meas_block(double* Pf, const int l, FilterStat
     const double r = 1.0 / sv;
 #pragma unroll
     for (int j = 0; j < NJ; j++) wj[j][0] *= r;
-    g_sweep<G, DC, 1>(Pf, w, g, wj);
+    g_sweep<G, DC, 1, MASK>(Pf, w, g, wj, skip);
     __syncwarp();
     const double u = rp_ * r;
     static_for<NA>([&](auto cc) {
       constexpr int c = cc;
       constexpr int xc = idx_of<DC>(c);
-      s.x[xc] = fma(g[0][c], u, s.x[xc]);
+      if constexpr (MASK) s.x[xc] = skip ? s.x[xc] : fma(g[0][c], u, s.x[xc]);
+      else s.x[xc] = fma(g[0][c], u, s.x[xc]);
     });
-    s.ll += -log(sv) - rp_ * u;
+    if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rp_ * u);
+    else s.ll += -log(sv) - rp_ * u;
   }
 }
 
@@ -585,8 +595,10 @@ __device__ __forceinline__ void g_record_fields(const KParams& p, const double* 
 // ------------------------------------------------------------------------------------------------
 // SYN = true: input rows drawn inside the kernel (KParams::syn), as in rbisk::rbis_fused_kernel.
 // REC = true: programs with RBIS_OP_RECORD ops (KParams::rec), as in rbisk::rbis_fused_kernel.
-template <int G, bool DC, int MAXW, bool SYN = false, bool REC = false>
+// MASK = true: programs with RBIS_STREAM_SKIP_NAN_ROWS streams (KParams::skip_nan_streams), as in rbisk::rbis_fused_kernel.
+template <int G, bool DC, int MAXW, bool SYN = false, bool REC = false, bool MASK = false>
 __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_constant__ KParams p) {
+  static_assert(!(MASK && SYN), "MASK instantiations read z from HBM");
   using GE = Geo<G, DC>;
   constexpr int FPW = GE::FPW, S = GE::S;
   extern __shared__ __align__(16) double smem[];
@@ -711,17 +723,22 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
         src.ss = &p.syn.st[op.stream];
         src.kfs = syn_kf ^ ((unsigned long long)__ldg(src.ss->step + op.row) * SYN_K2);
       }
+      // MASK: a filter whose row is missing passes the warp barriers like every lane and keeps its values
+      bool skip = false;
+      if constexpr (MASK) {
+        if ((p.skip_nan_streams >> op.stream) & 1u) skip = row_missing(st, op.row, sn);
+      }
       V3 dquat{0, 0, 0};
       if (st.has_orient) dquat = subtract_quats(src.quat(st, op.row, sn), {s.qw, s.qx, s.qy, s.qz});  // rbis.cpp:199
       const V3 chi0{s.x[6], s.x[7], s.x[8]};
       for (int ci = 0; ci < st.n_chunks; ci++) {
         const int a0 = st.chunk_start[ci];
         const int fast = st.chunk_fast[ci];
-        if (fast >= 0 && fast < 100) g_meas3<G, DC>(Pf, l, s, st, src, a0, fast, op.row, N, n, sn, dquat, chi0);
-        else if (fast >= 100) g_meas1<G, DC>(Pf, l, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0);
-        else g_meas_block<G, DC>(Pf, l, s, st, src, a0, st.chunk_len[ci], op.row, sn, dquat, chi0);
+        if (fast >= 0 && fast < 100) g_meas3<G, DC, SYN, MASK>(Pf, l, s, st, src, a0, fast, op.row, N, n, sn, dquat, chi0, skip);
+        else if (fast >= 100) g_meas1<G, DC, SYN, MASK>(Pf, l, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0, skip);
+        else g_meas_block<G, DC, SYN, MASK>(Pf, l, s, st, src, a0, st.chunk_len[ci], op.row, sn, dquat, chi0, skip);
       }
-      meas_finish(s, chi0, p.chi_tol, p.ctor_folds_chi, p.renorm);
+      if (!MASK || !skip) meas_finish(s, chi0, p.chi_tol, p.ctor_folds_chi, p.renorm);
     } else if (op.kind == OP_SNAPSHOT) {
       // ---- snapshot into ring slot ----
       double* d = p.snap + op.row * SNAP_ROWS * N + n;

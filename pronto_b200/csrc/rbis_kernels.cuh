@@ -310,6 +310,9 @@ struct KParams {
   StreamDesc streams[MAX_STREAMS];
   SynK syn;          // SYN kernel instantiations only
   RecK rec;          // REC kernel instantiations only (last: the parameter offsets of everything above stay as they were)
+  // MASK kernel instantiations only (appended for the same reason): bit s set = stream s has RBIS_STREAM_SKIP_NAN_ROWS, a
+  // filter whose row of that stream holds a NaN in a value the update reads skips the MEAS op (see row_missing)
+  unsigned skip_nan_streams;
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -895,6 +898,24 @@ constexpr uint32_t PARK_ALL = PARK_EVERYTHING & ~PARK_MEAS_KEEP;
 // step that follows; the linearisation point is already in Lin)
 constexpr uint32_t PARK_COV = PARK_EVERYTHING & ~(0x7u | (0x7u << 12)) & ~(uint32_t)(RBIS_PARK_COV_KEEP);
 
+// ---- rows missing per filter (MASK kernel instantiations, RBIS_STREAM_SKIP_NAN_ROWS) ----
+// Row `row` of stream st is missing for this lane's filter when any z value the update reads in its column sn is NaN; the
+// chi entries of an orientation stream are not read.  At most MAX_MEAS coalesced loads.
+__device__ __forceinline__ bool row_missing(const StreamDesc& st, long long row, long long sn) {
+  bool miss = false;
+  for (int a = 0; a < st.m; a++) {
+    const int i = st.idx[a];
+    if (st.has_orient && i >= 6 && i <= 8) continue;
+    miss = miss | (bool)isnan(__ldg(st.z + (row * st.m + a) * st.cols + sn));
+  }
+  return miss;
+}
+// A lane that skips runs the same instruction stream (the tensor-memory accesses and warp barriers of the updates are
+// warp-collective) and keeps its old values: every store of an update selects the old value, `skip ? old : new`.  A
+// select, not arithmetic on zeroed factors, which would turn a stored -0.0 into +0.0.  Without MASK the updates keep
+// their plain statements (`if constexpr (MASK) ... else <statement>`): even an inlined identity wrapper around them
+// changes the register allocation of the instantiations that exist without MASK.
+
 // x[idx] with a runtime (warp-uniform) index: select chain, registers cannot be indexed dynamically
 __device__ __forceinline__ double pick_state(const double (&x)[NS], int idx) {
   double v = x[0];
@@ -933,9 +954,10 @@ template <bool DC>
 __host__ __device__ constexpr int carried_pos(int c) { return DC ? act_pos(c) : c; }
 
 // DC: only the 15 active rows/columns exist (the couplings to omega / a are exactly zero, so are their gains).
-template <int I0, bool DC, bool SYN>
+// MASK: skip = the row is missing for this lane's filter, which then keeps covariance, state and log-likelihood (see row_missing).
+template <int I0, bool DC, bool SYN, bool MASK = false>
 __device__ __forceinline__ void meas3(Cov& P, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, long long row, long long N,
-                                      long long n, long long sn, const V3& dquat, const V3& chi0) {
+                                      long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
   static_assert(!DC || (is_act(I0) && I0 % 3 == 0), "a DC kernel cannot update on omega / a indices");
   constexpr int NC = DC ? N_ACT : NS;        // columns of HP that are carried
   constexpr int NB = NC / 3;                 // index triples
@@ -1031,7 +1053,8 @@ __device__ __forceinline__ void meas3(Cov& P, FilterState& s, const StreamDesc& 
         constexpr int i = Cur::row(k), j = Cur::col(k);
         constexpr int yi = pos(i), yj = pos(j);
         const double v = fma(-Y[0][yi], Y[0][yj] * r0, fma(-Y[1][yi], Y[1][yj] * r1, fma(-Y[2][yi], Y[2][yj] * r2, cur.d[k])));
-        P.template set<i, j>(v);
+        if constexpr (MASK) P.template set<i, j>(skip ? cur.d[k] : v);
+        else P.template set<i, j>(v);
       });
       RBIS_SCHED_FENCE();
     });
@@ -1058,9 +1081,11 @@ __device__ __forceinline__ void meas3(Cov& P, FilterState& s, const StreamDesc& 
   static_for<NC>([&](auto cc) {
     constexpr int c = cc;
     constexpr int xc = DC ? act_col(c) : c;
-    s.x[xc] = fma(Y[0][c], u0, fma(Y[1][c], u1, fma(Y[2][c], u2, s.x[xc])));
+    if constexpr (MASK) s.x[xc] = skip ? s.x[xc] : fma(Y[0][c], u0, fma(Y[1][c], u1, fma(Y[2][c], u2, s.x[xc])));
+    else s.x[xc] = fma(Y[0][c], u0, fma(Y[1][c], u1, fma(Y[2][c], u2, s.x[xc])));
   });
-  s.ll += -logdet - fma(e2, u2, fma(e1, u1, e0 * u0));
+  if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-logdet - fma(e2, u2, fma(e1, u1, e0 * u0)));
+  else s.ll += -logdet - fma(e2, u2, fma(e1, u1, e0 * u0));
 }
 
 // Row idx (run time, warp uniform) of the covariance over the carried columns: all loads issued, ONE tensor-memory wait.
@@ -1099,9 +1124,9 @@ __device__ __forceinline__ double pick_carried(const double (&g)[DC ? N_ACT : NS
   });
   return v;
 }
-// P -= g g^T r over the carried slots, pipelined tiles
-template <bool DC>
-__device__ __forceinline__ void rank1_sweep(Cov& P, const double (&g)[DC ? N_ACT : NS], double r) {
+// P -= g g^T r over the carried slots, pipelined tiles (MASK, skip: as in meas3)
+template <bool DC, bool MASK = false>
+__device__ __forceinline__ void rank1_sweep(Cov& P, const double (&g)[DC ? N_ACT : NS], double r, bool skip = false) {
   constexpr auto pos = &carried_pos<DC>;
   constexpr int TS = SWEEP_TILE;
   constexpr int NSW = kSweepLen<DC>;
@@ -1124,7 +1149,8 @@ __device__ __forceinline__ void rank1_sweep(Cov& P, const double (&g)[DC ? N_ACT
     static_for<len>([&](auto kc) {
       constexpr int k = kc;
       constexpr int i = Cur::row(k), j = Cur::col(k);
-      P.template set<i, j>(fma(-g[pos(i)], g[pos(j)] * r, cur.d[k]));
+      if constexpr (MASK) P.template set<i, j>(skip ? cur.d[k] : fma(-g[pos(i)], g[pos(j)] * r, cur.d[k]));
+      else P.template set<i, j>(fma(-g[pos(i)], g[pos(j)] * r, cur.d[k]));
     });
     RBIS_SCHED_FENCE();
   });
@@ -1135,9 +1161,9 @@ __device__ __forceinline__ void rank1_sweep(Cov& P, const double (&g)[DC ? N_ACT
 // that is not an aligned triple when its noise is uncorrelated with the other rows).  The index is a run-time, warp-uniform
 // value: the row P[idx, :] is fetched with run-time addressing (15 or 21 loads), everything after that -- the rank-1
 // sweep P -= h h^T / s and the state update -- runs over compile-time slots with h in registers.
-template <bool DC, bool SYN>
+template <bool DC, bool SYN, bool MASK = false>
 __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int idx, long long row, long long N,
-                                      long long n, long long sn, const V3& dquat, const V3& chi0) {
+                                      long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
   constexpr int NC = DC ? N_ACT : NS;
   constexpr auto pos = &carried_pos<DC>;
   const double z = src.z(st, row, a0, sn);
@@ -1147,7 +1173,7 @@ __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& 
   const double hii = pick_carried<DC>(h, idx);
   const double sv = Rv + hii;
   const double r = 1.0 / sv;
-  rank1_sweep<DC>(P, h, r);
+  rank1_sweep<DC, MASK>(P, h, r, skip);
   double rr;
   if (st.has_orient && idx >= 6 && idx <= 8) {
     const int k = idx - 6;
@@ -1161,9 +1187,11 @@ __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& 
   static_for<NC>([&](auto cc) {
     constexpr int c = cc;
     constexpr int xc = DC ? act_col(c) : c;
-    s.x[xc] = fma(h[c], u, s.x[xc]);
+    if constexpr (MASK) s.x[xc] = skip ? s.x[xc] : fma(h[c], u, s.x[xc]);
+    else s.x[xc] = fma(h[c], u, s.x[xc]);
   });
-  s.ll += -log(sv) - rr * u;
+  if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rr * u);
+  else s.ll += -log(sv) - rr * u;
 }
 
 // meas_block: a chunk of M (2..9) rows with CORRELATED noise on any indices.  The host factors R_block = L D L^T; with
@@ -1172,9 +1200,9 @@ __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& 
 // Row a of H' combines the covariance rows idx_b, b <= a, so everything lives in registers: g = P H'_a^T (15 / 21
 // doubles), a rank-1 sweep over compile-time slots, the state update.  No local-memory arrays, no separate kernel variant.
 // Only the BLOCKS = true kernel variants contain it.
-template <bool DC, bool SYN>
+template <bool DC, bool SYN, bool MASK = false>
 __device__ __forceinline__ void meas_block(Cov& P, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int M, long long row, long long N,
-                                           long long n, long long sn, const V3& dquat, const V3& chi0) {
+                                           long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
   constexpr int NC = DC ? N_ACT : NS;
   const double* W = st.R + row * st.r_stride + RS_W;
   const double* Dg = st.R + row * st.r_stride + RS_D;
@@ -1206,14 +1234,16 @@ __device__ __forceinline__ void meas_block(Cov& P, FilterState& s, const StreamD
       rp = fma(w, rb, rp);
     }
     const double r = 1.0 / sv;
-    rank1_sweep<DC>(P, g, r);
+    rank1_sweep<DC, MASK>(P, g, r, skip);
     const double u = rp * r;
     static_for<NC>([&](auto cc) {
       constexpr int c = cc;
       constexpr int xc = DC ? act_col(c) : c;
-      s.x[xc] = fma(g[c], u, s.x[xc]);
+      if constexpr (MASK) s.x[xc] = skip ? s.x[xc] : fma(g[c], u, s.x[xc]);
+      else s.x[xc] = fma(g[c], u, s.x[xc]);
     });
-    s.ll += -log(sv) - rp * u;
+    if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rp * u);
+    else s.ll += -log(sv) - rp * u;
   }
 }
 
@@ -1336,8 +1366,11 @@ __device__ __forceinline__ void record_fields(const KParams& p, const Cov& P, co
 // measurement of the program indexes omega or a (see "decoupled filters" above).
 // SYN = true: the input rows are drawn inside the kernel (KParams::syn, mode-1 generator) instead of being read from HBM.
 // REC = true: the program has RBIS_OP_RECORD ops (KParams::rec); launched only then, so that other programs keep their code.
-template <bool BLOCKS, bool DC = false, bool SYN = false, bool REC = false>
+// MASK = true: some stream of the program has RBIS_STREAM_SKIP_NAN_ROWS (KParams::skip_nan_streams); instantiated with BLOCKS
+// only (and without SYN), launched only for such programs.
+template <bool BLOCKS, bool DC = false, bool SYN = false, bool REC = false, bool MASK = false>
 __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constant__ KParams p) {
+  static_assert(!MASK || (BLOCKS && !SYN), "MASK instantiations have the one-row / correlated-block paths and read z from HBM");
   extern __shared__ __align__(16) double smem[];
   __shared__ uint32_t tm_base_s;
   const int tid = threadIdx.x;
@@ -1473,6 +1506,11 @@ __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constan
         src.ss = &p.syn.st[op.stream];
         src.kfs = syn_kf ^ ((unsigned long long)__ldg(src.ss->step + op.row) * SYN_K2);
       }
+      // MASK: a filter whose row is missing runs the sweeps like every lane and keeps its values (see row_missing)
+      bool skip = false;
+      if constexpr (MASK) {
+        if ((p.skip_nan_streams >> op.stream) & 1u) skip = row_missing(st, op.row, sn);
+      }
       V3 dquat{0, 0, 0};
       if (st.has_orient) dquat = subtract_quats(src.quat(st, op.row, sn), {s.qw, s.qx, s.qy, s.qz});  // rbis.cpp:199
       const V3 chi0{s.x[6], s.x[7], s.x[8]};
@@ -1480,25 +1518,25 @@ __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constan
         const int a0 = st.chunk_start[ci];
         const int fast = st.chunk_fast[ci];
         switch (fast) {
-          case 0: if constexpr (!DC) meas3<0, false>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0); break;
-          case 3: meas3<3, DC>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0); break;
-          case 6: meas3<6, DC>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0); break;
-          case 9: meas3<9, DC>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0); break;
-          case 12: if constexpr (!DC) meas3<12, false>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0); break;
-          case 15: meas3<15, DC>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0); break;
-          case 18: meas3<18, DC>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0); break;
+          case 0: if constexpr (!DC) meas3<0, false, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
+          case 3: meas3<3, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
+          case 6: meas3<6, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
+          case 9: meas3<9, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
+          case 12: if constexpr (!DC) meas3<12, false, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
+          case 15: meas3<15, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
+          case 18: meas3<18, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
           default:
             if constexpr (BLOCKS) {
               if (fast >= 100) {  // one-row chunk on state index fast - 100
-                meas1<DC>(P, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0);
+                meas1<DC, SYN, MASK>(P, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0, skip);
               } else {            // correlated rows: decorrelated scalar updates
-                meas_block<DC>(P, s, st, src, a0, st.chunk_len[ci], op.row, N, n, sn, dquat, chi0);
+                meas_block<DC, SYN, MASK>(P, s, st, src, a0, st.chunk_len[ci], op.row, N, n, sn, dquat, chi0, skip);
               }
             }
             break;
         }
       }
-      meas_finish(s, chi0, p.chi_tol, p.ctor_folds_chi, p.renorm);
+      if (!MASK || !skip) meas_finish(s, chi0, p.chi_tol, p.ctor_folds_chi, p.renorm);
     } else if (op.kind == OP_SNAPSHOT) {
       // ---- snapshot into ring slot ----
       double* d = p.snap + op.row * SNAP_ROWS * N + n;
