@@ -239,8 +239,14 @@ int rbis_batch_set_column_map(rbis_batch_t* h, int which, const int32_t* map, in
  * Record row r holds, bit for bit, what an RBIS_OP_SNAPSHOT at the same program position would hold in those fields.  Field f is
  * recorded when bit f of `fields` is set:
  *   0..20  vec[f]        21..24  quat w, x, y, z        25  log-likelihood        26..46  covariance diagonal P(f-26, f-26)
- * out is [rows][k][N], k = popcount(fields), the chosen fields in ascending bit order, filter index fastest; column maps do not
- * apply (records are always per filter).  Inactive filters of a launch write nothing; rows no RECORD op names stay untouched.
+ * After the fields a row can hold covariance BLOCKS: bit b of `cov_blocks` selects state block b, indices 3b..3b+2 (0 omega,
+ * 1 v, 2 chi, 3 p, 4 a, 5 gyro bias, 6 accel bias).  With I the ascending selected indices and nb = |I| = 3 popcount(cov_blocks),
+ * the packed upper triangle of P restricted to I follows the fields: P(I[ii], I[jj]), ii <= jj < nb, at field position
+ * popcount(fields) + jj (jj + 1) / 2 + ii.  With all seven blocks that is the covariance part of a snapshot slot
+ * (slot(i, j) = j (j + 1) / 2 + i, 231 entries); {v, chi, p} is the 9x9 block of the NEES, {p, chi} the pose covariance.
+ * out is [rows][k][N], k = popcount(fields) + nb (nb + 1) / 2, the chosen fields in ascending bit order, then the covariance
+ * entries, filter index fastest; column maps do not apply (records are always per filter).  Inactive filters of a launch write
+ * nothing; rows no RECORD op names stay untouched.
  *   RBIS_MEM_DEVICE: the kernels write `out` in place.  It is valid once a ticket recorded after the call has been waited for
  *                    (rbis_batch_record / rbis_batch_wait) or after rbis_batch_synchronize.
  *   RBIS_MEM_HOST:   `out` must be PINNED host memory (pageable memory is rejected: a copy into it would synchronise).  The kernels
@@ -254,12 +260,13 @@ typedef struct {
   double* out;       /* [rows][k][N] */
   int64_t rows;
   int32_t mem;       /* RBIS_MEM_DEVICE or RBIS_MEM_HOST (pinned) */
-  int32_t reserved;
+  int32_t cov_blocks; /* bit b < 7: record the covariance block of state block b (0 = none; was a reserved zero field) */
 } rbis_record_t;
 /* Sets the record set used by the rbis_batch_run_fused / rbis_batch_run_fused_synth calls enqueued after it (handle state, like
  * the column maps; a copy of *rec is kept); NULL clears it.  Does not synchronise, so switching buffers between calls keeps the
- * device busy.  A RECORD op without a record set fails with RBIS_ERR_STATE, a row outside [0, rows) with RBIS_ERR_INVALID, both
- * before anything is enqueued.  The single-update entry points do not record. */
+ * device busy.  fields and cov_blocks must not both be empty; a cov_blocks bit >= 7 is RBIS_ERR_INVALID.  A RECORD op without a
+ * record set fails with RBIS_ERR_STATE, a row outside [0, rows) with RBIS_ERR_INVALID, both before anything is enqueued.  The
+ * single-update entry points do not record. */
 int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec);
 
 /* ---- the fused hot path: run `n_ops` ops (host array, executed in order) for every filter in ONE
@@ -418,6 +425,22 @@ int rbis_batch_stats_enqueue(rbis_batch_t* h, const double* truth_vec, const dou
  * replay (append RBIS_OP_SNAPSHOT to the step's last program, alternate two slots) without draining the device. */
 int rbis_batch_stats_snapshot_enqueue(rbis_batch_t* h, int32_t slot, const double* truth_vec, const double* truth_quat, int chunk,
                                       double* out_chunks, int64_t* n_chunks, int32_t* ticket);
+/* The same statistics over RECORD ROWS first_row .. first_row + n_rows - 1 of the current record set, one chunk table per row:
+ * the table of row r is bit-identical to rbis_batch_stats_snapshot_enqueue over a SNAPSHOT taken where the RECORD op that wrote
+ * row r stands, with the same truth and chunk.  One pass over all rows, on the same side stream and with the same ordering as
+ * rbis_batch_stats_snapshot_enqueue (after the launches of the last fused call; the fused calls that follow do not wait for it).
+ * The record set must be in device memory, have every field 0..25 (vec, quat, loglik) and the covariance blocks 1, 2 and 3
+ * (v, chi, p: the NEES block), and the rows must lie in [0, rows); otherwise the call fails before anything is enqueued.
+ *   truth_vec [n_rows][21] / truth_quat [n_rows][4]: host; row r is the truth at record row first_row + r.
+ *   out_chunks: PINNED host [n_rows][n_chunks][RBIS_NUM_STATS].  out_totals: PINNED host [n_rows][RBIS_NUM_STATS] or NULL, each
+ *   row's table summed in ascending chunk order (= rbis_stats_reduce_chunks).  Both are valid once rbis_batch_wait(*ticket)
+ *   returns.
+ * A later fused call whose RECORD ops write into the buffer a pending pass reads waits for that pass on the device.  To keep
+ * calls overlapping, alternate two record buffers with rbis_batch_set_record (which does not synchronise), as a driver
+ * alternates two snapshot slots. */
+int rbis_batch_stats_records_enqueue(rbis_batch_t* h, int64_t first_row, int64_t n_rows, const double* truth_vec,
+                                     const double* truth_quat, int chunk, double* out_chunks, double* out_totals, int64_t* n_chunks,
+                                     int32_t* ticket);
 /* ---- statistics of a SHARDED ensemble (SURVEY.md 8e): one process per GPU, each handle holds the contiguous filter range
  * [first_chunk * chunk, first_chunk * chunk + N) of an ensemble of total_chunks chunks.  The shard's chunk partials are written
  * into its rows of a zero-initialised DEVICE table [total_chunks][RBIS_NUM_STATS], the table is summed over the ranks with
@@ -466,6 +489,13 @@ int rbis_batch_get_filter_states(rbis_batch_t* h, int64_t first, int64_t count, 
 /* Filters first..first+count-1 := the messages (state, quaternion, covariance; log-likelihood 0), as RBIS(msg) +
  * Map<const RBIM>(msg->cov) of the reference's log loader (state-estimator/src/noise_id/noise_id.cpp:83-86). */
 int rbis_batch_set_filter_states(rbis_batch_t* h, int64_t first, int64_t count, const rbis_filter_state_t* msgs);
+/* One filter_state_t message per filter first..first+count-1 of a record row that is already on the
+ * host: row is [k][n_filters] in the layout above, with every field 0..24 and all seven covariance blocks (fields bit 25 and
+ * bits 26.. may be set too).  The messages are what rbis_batch_get_filter_states writes for the same state: both triangles of the
+ * covariance, column-major (MSE/rbis.cpp:282), utime = `utime`.  Host only; it hides the packed layout from a caller that
+ * publishes the reference's message per recorded head (MSE/lcm_front_end.cpp:144-166). */
+int rbis_record_filter_states(uint64_t fields, int32_t cov_blocks, const double* row, int64_t n_filters, int64_t utime,
+                              int64_t first, int64_t count, rbis_filter_state_t* out);
 
 /* indexed_measurement_t (pronto-lcmtypes/lcmtypes/pronto_indexed_measurement_t.lcm), bounded to RBIS_MAX_MEAS rows. */
 typedef struct {

@@ -156,15 +156,31 @@ def record_fields(vec=(), quat=False, loglik=False, cov_diag=()):
     return mask
 
 
-def record_layout(mask):
-    """Names of the fields of a record row in output order: 'vec<i>', 'quat_w' .. 'quat_z', 'loglik', 'cov_diag<i>'."""
+def record_cov_blocks(blocks=()):
+    """rbis_record_t::cov_blocks of covariance block numbers 0..6 (state indices 3b..3b+2: omega, v, chi, p, a, gyro bias,
+    accel bias)."""
+    cb = 0
+    for b in blocks:
+        if not 0 <= int(b) < capi.REC_BLOCKS:
+            raise ValueError(f"covariance block {b} outside [0, {capi.REC_BLOCKS})")
+        cb |= 1 << int(b)
+    return cb
+
+
+def record_layout(mask, cov_blocks=()):
+    """Names of the fields of a record row in output order: 'vec<i>', 'quat_w' .. 'quat_z', 'loglik', 'cov_diag<i>', then
+    'cov<i>_<j>' for P(i, j), i <= j, of the covariance blocks `cov_blocks` (block numbers 0..6), packed column by column."""
     mask = int(mask)
-    if mask <= 0 or mask >> capi.REC_FIELDS:
-        raise ValueError(f"record fields {mask:#x}: need a non-empty set of bits 0..{capi.REC_FIELDS - 1}")
+    cb = record_cov_blocks(cov_blocks)
+    if mask < 0 or mask >> capi.REC_FIELDS or (mask == 0 and cb == 0):
+        raise ValueError(f"record fields {mask:#x}: need a non-empty set of bits 0..{capi.REC_FIELDS - 1} or covariance blocks")
     names = []
     for f in range(capi.REC_FIELDS):
         if mask >> f & 1:
             names.append(f"vec{f}" if f < 21 else _QUAT_NAMES[f - 21] if f < 25 else "loglik" if f == 25 else f"cov_diag{f - 26}")
+    idx = [3 * b + c for b in range(capi.REC_BLOCKS) if cb >> b & 1 for c in range(3)]
+    for jj, j in enumerate(idx):
+        names.extend(f"cov{i}_{j}" for i in idx[:jj + 1])
     return names
 
 
@@ -396,18 +412,20 @@ class RBISBatch:
         return (len(ops), ops.ctypes.data_as(C.POINTER(capi.Op)), p_imu, imu_rows, len(streams), sarr, mem, keep)
 
     # ---- records ----
-    def set_record(self, out, fields):
+    def set_record(self, out, fields, cov_blocks=()):
         """Record set of the RBIS_OP_RECORD ops of later fused calls (rbis_batch_set_record).  out: float64 [rows][k][N], k the number
-        of fields (record_fields / record_layout), a CUDA tensor (written in place) or a PINNED CPU tensor or array (filled by an
-        asynchronous copy); its rows are valid after wait(record()) or synchronize().  Does not synchronise."""
+        of entries of record_layout(fields, cov_blocks), a CUDA tensor (written in place) or a PINNED CPU tensor or array (filled by an
+        asynchronous copy); its rows are valid after wait(record()) or synchronize().  cov_blocks: covariance block numbers 0..6
+        recorded after the fields.  Does not synchronise."""
         fields = int(fields)
-        if 0 < fields < 1 << capi.REC_FIELDS:
-            k = bin(fields).count("1")
+        cb = record_cov_blocks(cov_blocks)
+        if 0 <= fields < 1 << capi.REC_FIELDS and (fields or cb):
+            k = len(record_layout(fields, cov_blocks))
             if out.ndim != 3 or tuple(out.shape[1:]) != (k, self.N):
                 raise ValueError(f"record output must be [rows][{k}][{self.N}], got {tuple(out.shape)}")
         p, mem = _ptr(out, None, "out")
         rec = capi.Record()
-        rec.fields, rec.out, rec.rows, rec.mem = fields, p, int(out.shape[0]), mem
+        rec.fields, rec.out, rec.rows, rec.mem, rec.cov_blocks = fields, p, int(out.shape[0]), mem, cb
         capi.check(self.lib.rbis_batch_set_record(self.h, C.byref(rec)))
         # the previous buffer may still be written by enqueued calls: held until the next synchronize()
         self._pending_keep = getattr(self, "_pending_keep", [])
@@ -554,6 +572,23 @@ class RBISBatch:
                                                               C.byref(t)))
         return t.value
 
+    def stats_records_enqueue(self, first_row, truth_vec, truth_quat, out_chunks, out_totals=None, chunk=1024):
+        """Statistics of record rows first_row .. first_row + n_rows - 1 of the current (device) record set on the statistics side
+        stream (rbis_batch_stats_records_enqueue): truth_vec [n_rows][21], truth_quat [n_rows][4]; out_chunks a PINNED host array
+        [n_rows][n_chunks][96], out_totals a PINNED host array [n_rows][96] or None.  Returns the ticket to wait() for."""
+        tv = np.ascontiguousarray(truth_vec, dtype=np.float64).reshape(-1, 21)
+        tq = np.ascontiguousarray(truth_quat, dtype=np.float64).reshape(-1, 4)
+        n_rows = tv.shape[0]
+        if tq.shape[0] != n_rows:
+            raise ValueError(f"truth_vec has {n_rows} rows, truth_quat {tq.shape[0]}")
+        n_chunks = (self.N + chunk - 1) // chunk
+        po, _ = _ptr(out_chunks, (n_rows, n_chunks, capi.NUM_STATS), "out_chunks")
+        pt, _ = _ptr(out_totals, (n_rows, capi.NUM_STATS), "out_totals")
+        nch, t = C.c_int64(0), C.c_int32(0)
+        capi.check(self.lib.rbis_batch_stats_records_enqueue(self.h, int(first_row), n_rows, tv.ctypes.data, tq.ctypes.data, int(chunk),
+                                                             po, pt, C.byref(nch), C.byref(t)))
+        return t.value
+
     def record(self):
         t = C.c_int32(0)
         capi.check(self.lib.rbis_batch_record(self.h, C.byref(t)))
@@ -561,6 +596,21 @@ class RBISBatch:
 
     def wait(self, ticket):
         capi.check(self.lib.rbis_batch_wait(self.h, int(ticket)))
+
+
+def filter_states_from_record(row, fields, cov_blocks=range(7), utime=0, first=0, count=None):
+    """filter_state_t messages (capi.FilterState array) of filters first .. first+count-1 of one record row already on the host
+    (rbis_record_filter_states): row [k][N] with fields 0..24 and all seven covariance blocks; the messages are those
+    rbis_batch_get_filter_states writes for the same state."""
+    row = np.ascontiguousarray(row, dtype=np.float64)
+    if row.ndim != 2:
+        raise ValueError(f"record row must be [k][N], got {row.shape}")
+    n = row.shape[1]
+    count = n - int(first) if count is None else int(count)
+    out = (capi.FilterState * max(1, count))()
+    capi.check(capi.load().rbis_record_filter_states(int(fields), record_cov_blocks(cov_blocks), row.ctypes.data, n, int(utime), int(first),
+                                                     count, out))
+    return out
 
 
 def reduce_chunks(chunks):

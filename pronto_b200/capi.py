@@ -19,6 +19,7 @@ MEM_HOST, MEM_DEVICE = 0, 1
 MEM_F32_ROWS = 4  # rbis_batch_run_fused: imu / z / quat are float32 arrays (widened exactly on the device)
 OP_IMU, OP_MEAS, OP_SNAPSHOT, OP_RESTORE, OP_RECORD = 0, 1, 2, 3, 4
 REC_FIELDS = 47  # record fields: 0..20 vec, 21..24 quat w,x,y,z, 25 loglik, 26..46 covariance diagonal
+REC_BLOCKS = 7   # record covariance blocks: state indices 3b..3b+2 (omega, v, chi, p, a, gyro bias, accel bias)
 R_SHARED_FULL, R_PER_FILTER_DIAG, R_PER_ROW_FULL = 0, 1, 2
 STREAM_SKIP_NAN_ROWS = 1  # rbis_stream_t::flags: a filter whose row holds a NaN in a value the update reads skips that update
 
@@ -117,7 +118,7 @@ class Record(C.Structure):
         ("out", C.c_void_p),
         ("rows", C.c_int64),
         ("mem", C.c_int32),
-        ("reserved", C.c_int32),
+        ("cov_blocks", C.c_int32),
     ]
 
 
@@ -163,6 +164,8 @@ PROTOTYPES = {
     "rbis_batch_run_fused_synth": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Op), C.c_int, C.POINTER(Stream), C.POINTER(Synth)]),
     "rbis_batch_get_filter_states": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(FilterState)]),
     "rbis_batch_set_filter_states": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.POINTER(FilterState)]),
+    "rbis_record_filter_states": (C.c_int, [C.c_uint64, C.c_int32, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
+                                            C.POINTER(FilterState)]),
     "rbis_stream_from_indexed_measurement": (C.c_int, [C.POINTER(IndexedMeasurement), C.POINTER(Stream), C.c_void_p]),
     "rbis_stream_from_indexed_measurements": (C.c_int, [C.POINTER(IndexedMeasurement), C.c_int64, C.POINTER(Stream), C.c_void_p]),
     "rbis_kvh_stream_create": (C.c_int, [C.POINTER(C.c_void_p)]),
@@ -179,6 +182,8 @@ PROTOTYPES = {
     "rbis_batch_stats_enqueue": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, c_int64_p]),
     "rbis_batch_stats_snapshot_enqueue": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, c_int64_p,
                                                      C.POINTER(C.c_int32)]),
+    "rbis_batch_stats_records_enqueue": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
+                                                    C.c_void_p, c_int64_p, C.POINTER(C.c_int32)]),
     "rbis_batch_stats_allreduce": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),
     "rbis_batch_window_neg_loglik": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
                                                C.c_void_p, C.c_void_p, C.c_int]),

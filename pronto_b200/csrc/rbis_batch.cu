@@ -163,7 +163,7 @@ struct rbis_batch {
   // rec_stream moves out after the call's last launches.  Nothing but the reuse of a staging buffer waits for that copy.
   bool rec_set = false;
   rbis_record_t rec{};
-  int rec_k = 0;                          // popcount(rec.fields)
+  int rec_k = 0;                          // doubles per filter and row: popcount(rec.fields) + the covariance entries
   cudaStream_t rec_stream = nullptr;
   cudaEvent_t rec_launched = nullptr;     // ungrouped launch done (rec_stream waits for it)
   DevBuf rec_stage[2];
@@ -179,6 +179,17 @@ struct rbis_batch {
   std::vector<cudaEvent_t> snap_read_evt;   // per slot, created on first use
   std::vector<char> snap_read_pending;
   std::vector<DevBuf> snap_stats_scratch;   // per slot: truth [25] + chunk partials
+  // ---- statistics over record rows (rbis_batch_stats_records_enqueue), on the same side stream: per device record buffer a
+  // pending pass reads, the event after that pass; a fused call whose RECORD ops write into the buffer waits for it
+  struct RecReader {
+    const double *lo, *hi;  // [lo, hi): the record buffer
+    cudaEvent_t done;
+    bool pending;
+  };
+  std::vector<RecReader> rec_readers;
+  DevBuf rec_stats_scratch;                 // truth [rows][25] + tables [rows][chunks][96] + totals [rows][96]
+  cudaEvent_t rec_stats_done = nullptr;     // the last pass (scratch reuse)
+  bool rec_stats_pending = false;
 };
 
 namespace {
@@ -698,6 +709,7 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     kp.rec.fields = h->rec.fields;
     kp.rec.k = h->rec_k;
     kp.rec.out = h->rec.out;
+    kp.rec_cov_blocks = (unsigned)h->rec.cov_blocks;
     if (rec_host) {
       rec_distinct = rec_rows;
       std::sort(rec_distinct.begin(), rec_distinct.end());
@@ -802,6 +814,16 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
       if (ops[i].kind == RBIS_OP_SNAPSHOT && h->snap_read_pending[(size_t)ops[i].row]) {
         slot_readers.push_back(h->snap_read_evt[(size_t)ops[i].row]);
         h->snap_read_pending[(size_t)ops[i].row] = 0;
+      }
+  }
+  // a device record buffer this program writes that a side-stream statistics pass may still be reading
+  if (any_record && !rec_host) {
+    const double* lo = h->rec.out;
+    const double* hi = lo + (size_t)h->rec.rows * (size_t)h->rec_k * N;
+    for (auto& r : h->rec_readers)
+      if (r.pending && r.lo < hi && lo < r.hi) {
+        slot_readers.push_back(r.done);
+        r.pending = false;
       }
   }
   if (!grouped) {
@@ -1120,6 +1142,9 @@ int rbis_batch_destroy(rbis_batch_t* h) {
   h->full_cov.release(); h->misc.release(); h->stats_async.release(); h->stats_table.release(); h->synth_small.release(); h->d_syn.release();
   for (auto& b : h->snap_stats_scratch) b.release();
   for (cudaEvent_t e : h->snap_read_evt) if (e) cudaEventDestroy(e);
+  for (auto& r : h->rec_readers) cudaEventDestroy(r.done);
+  if (h->rec_stats_done) cudaEventDestroy(h->rec_stats_done);
+  h->rec_stats_scratch.release();
   if (h->stats_stream) cudaStreamDestroy(h->stats_stream);
   for (auto& b : h->d_syn_ring) b.release();
   for (auto& s : h->slots) {
@@ -1148,6 +1173,8 @@ int rbis_batch_synchronize(rbis_batch_t* h) {
   if (h->stats_stream) {  // side-stream statistics (rbis_batch_stats_snapshot_enqueue): done too, their slots are free again
     CUDA_TRY(cudaStreamSynchronize(h->stats_stream));
     std::fill(h->snap_read_pending.begin(), h->snap_read_pending.end(), 0);
+    for (auto& r : h->rec_readers) r.pending = false;
+    h->rec_stats_pending = false;
   }
   return 0;
 }
@@ -1317,8 +1344,11 @@ int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec) {
     h->rec_set = false;
     return 0;
   }
-  if (rec->fields == 0 || (rec->fields >> rbisk::REC_FIELDS) != 0)
-    return fail(RBIS_ERR_INVALID, "record fields 0x%llx: need a non-empty set of bits 0..%d", (unsigned long long)rec->fields, rbisk::REC_FIELDS - 1);
+  if ((rec->fields >> rbisk::REC_FIELDS) != 0)
+    return fail(RBIS_ERR_INVALID, "record fields 0x%llx: bits 0..%d only", (unsigned long long)rec->fields, rbisk::REC_FIELDS - 1);
+  if ((unsigned)rec->cov_blocks >> rbisk::REC_BLOCKS)
+    return fail(RBIS_ERR_INVALID, "record cov_blocks 0x%x: bits 0..%d only", (unsigned)rec->cov_blocks, rbisk::REC_BLOCKS - 1);
+  if (rec->fields == 0 && rec->cov_blocks == 0) return fail(RBIS_ERR_INVALID, "record set is empty: no fields and no covariance blocks");
   if (!rec->out) return fail(RBIS_ERR_INVALID, "record output is NULL");
   if (rec->rows <= 0) return fail(RBIS_ERR_INVALID, "record rows must be positive");
   if (rec->mem != RBIS_MEM_HOST && rec->mem != RBIS_MEM_DEVICE) return fail(RBIS_ERR_INVALID, "record mem must be RBIS_MEM_HOST or RBIS_MEM_DEVICE");
@@ -1334,7 +1364,8 @@ int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec) {
   if (rec->mem == RBIS_MEM_DEVICE && ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != h->cfg.device))
     return fail(RBIS_ERR_INVALID, "record output is not memory of device %d", h->cfg.device);
   h->rec = *rec;
-  h->rec_k = __builtin_popcountll(rec->fields);
+  const int nb = 3 * __builtin_popcount((unsigned)rec->cov_blocks);
+  h->rec_k = __builtin_popcountll(rec->fields) + nb * (nb + 1) / 2;
   h->rec_set = true;
   return 0;
 }
@@ -1496,7 +1527,7 @@ int rbis_batch_stats(rbis_batch_t* h, const double* truth_vec, const double* tru
   double* pf = d_pf;
   if (out_per_filter && mem == RBIS_MEM_DEVICE) pf = out_per_filter;
   rbisk::stats_kernel<<<(unsigned)nch, chunk, chunk * sizeof(double), h->stream>>>(
-      h->vec, h->quat, h->P, h->loglik, tv, tq, per_filter, (long long)N, pf, d_chunks);
+      rbisk::StatsArrays{h->vec, h->quat, h->P, h->loglik}, tv, tq, per_filter, (long long)N, pf, d_chunks);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   CUDA_TRY(cudaMemcpyAsync(out_chunks, d_chunks, (size_t)nch * RBIS_NUM_STATS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
@@ -1525,7 +1556,7 @@ int rbis_batch_stats_enqueue(rbis_batch_t* h, const double* truth_vec, const dou
   std::memcpy(tbuf + 21, truth_quat, 4 * sizeof(double));
   if (int rc = upload_small(h, d_truth, tbuf, sizeof(tbuf), h->stream)) return rc;  // pinned ring: the host does not wait for the stream
   rbisk::stats_kernel<<<(unsigned)nch, chunk, chunk * sizeof(double), h->stream>>>(
-      h->vec, h->quat, h->P, h->loglik, d_truth, d_truth + 21, 0, (long long)N, nullptr, d_chunks);
+      rbisk::StatsArrays{h->vec, h->quat, h->P, h->loglik}, d_truth, d_truth + 21, 0, (long long)N, nullptr, d_chunks);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   CUDA_TRY(cudaMemcpyAsync(out_chunks, d_chunks, (size_t)nch * RBIS_NUM_STATS * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
@@ -1572,13 +1603,112 @@ int rbis_batch_stats_snapshot_enqueue(rbis_batch_t* h, int32_t slot, const doubl
   std::memcpy(tbuf + 21, truth_quat, 4 * sizeof(double));
   if (int rc = upload_small(h, d_truth, tbuf, sizeof(tbuf), ss)) return rc;
   const double* d = h->snap + (size_t)slot * rbisk::SNAP_ROWS * N;  // [257][N]: vec 0..20, quat 21..24, loglik 25, packed covariance 26..
-  rbisk::stats_kernel<<<(unsigned)nch, chunk, chunk * sizeof(double), ss>>>(d, d + 21 * N, d + 26 * N, d + 25 * N, d_truth, d_truth + 21, 0,
+  rbisk::stats_kernel<<<(unsigned)nch, chunk, chunk * sizeof(double), ss>>>(rbisk::StatsArrays{d, d + 21 * N, d + 26 * N, d + 25 * N}, d_truth, d_truth + 21, 0,
                                                                             (long long)N, nullptr, d_chunks);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   CUDA_TRY(cudaMemcpyAsync(out_chunks, d_chunks, (size_t)nch * RBIS_NUM_STATS * sizeof(double), cudaMemcpyDeviceToHost, ss));
   CUDA_TRY(cudaEventRecord(h->snap_read_evt[(size_t)slot], ss));
   h->snap_read_pending[(size_t)slot] = 1;
+  const int t = h->next_ticket;
+  h->next_ticket = (t + 1) % 8;
+  CUDA_TRY(cudaEventRecord(h->tickets[t], ss));
+  *ticket = t;
+  if (n_chunks) *n_chunks = nch;
+  return 0;
+}
+
+int rbis_batch_stats_records_enqueue(rbis_batch_t* h, int64_t first_row, int64_t n_rows, const double* truth_vec,
+                                     const double* truth_quat, int chunk, double* out_chunks, double* out_totals, int64_t* n_chunks,
+                                     int32_t* ticket) {
+  if (!h) return fail(RBIS_ERR_INVALID, "null handle");
+  if (!truth_vec || !truth_quat || !out_chunks || !ticket) return fail(RBIS_ERR_INVALID, "truth, out_chunks and ticket are required");
+  if (chunk < 32 || chunk > 1024 || (chunk & (chunk - 1))) return fail(RBIS_ERR_INVALID, "chunk must be a power of two in [32,1024]");
+  if (!h->rec_set) return fail(RBIS_ERR_STATE, "no record set (rbis_batch_set_record)");
+  const rbis_record_t& rec = h->rec;
+  if (rec.mem != RBIS_MEM_DEVICE) return fail(RBIS_ERR_INVALID, "statistics of record rows need a record set in device memory");
+  if ((rec.fields & 0x3FFFFFFull) != 0x3FFFFFFull) return fail(RBIS_ERR_INVALID, "statistics of record rows need record fields 0..25 (vec, quat, loglik)");
+  if ((rec.cov_blocks & 0xE) != 0xE) return fail(RBIS_ERR_INVALID, "statistics of record rows need covariance blocks 1, 2 and 3 (v, chi, p)");
+  if (n_rows < 1 || first_row < 0 || first_row + n_rows > rec.rows)
+    return fail(RBIS_ERR_INVALID, "record rows %lld..%lld outside [0, %lld)", (long long)first_row, (long long)(first_row + n_rows), (long long)rec.rows);
+  if (int rc = use_device(h)) return rc;
+  if (!h->stats_stream) {
+    CUDA_TRY(cudaStreamCreateWithFlags(&h->stats_stream, cudaStreamNonBlocking));
+    h->snap_read_evt.assign((size_t)h->cfg.snapshot_slots, nullptr);
+    h->snap_read_pending.assign((size_t)h->cfg.snapshot_slots, 0);
+    h->snap_stats_scratch.resize((size_t)h->cfg.snapshot_slots);
+  }
+  if (!h->rec_stats_done) CUDA_TRY(cudaEventCreateWithFlags(&h->rec_stats_done, cudaEventDisableTiming));
+  // the reader entry of this buffer (buffers no pass reads any more are dropped)
+  const size_t N = (size_t)h->N, k = (size_t)h->rec_k;
+  const double* lo = rec.out;
+  const double* hi = lo + (size_t)rec.rows * k * N;
+  rbis_batch::RecReader* rd = nullptr;
+  for (auto& r : h->rec_readers)
+    if (r.lo == lo && r.hi == hi) rd = &r;
+  if (!rd) {
+    for (size_t i = 0; i < h->rec_readers.size();)
+      if (!h->rec_readers[i].pending) {
+        cudaEventDestroy(h->rec_readers[i].done);
+        h->rec_readers.erase(h->rec_readers.begin() + (long)i);
+      } else {
+        i++;
+      }
+    cudaEvent_t e;
+    CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    h->rec_readers.push_back({lo, hi, e, false});
+    rd = &h->rec_readers.back();
+  }
+  const int64_t nch = (int64_t)((N + chunk - 1) / chunk);
+  const size_t n_table = (size_t)nch * RBIS_NUM_STATS;
+  const size_t need = (size_t)n_rows * (25 + n_table + RBIS_NUM_STATS);
+  DevBuf& scratch = h->rec_stats_scratch;
+  if (scratch.cap < need) {
+    if (h->rec_stats_pending) CUDA_TRY(cudaEventSynchronize(h->rec_stats_done));  // the last pass still reads the old scratch
+    if (scratch.ensure(need)) return fail(RBIS_ERR_ALLOC, "scratch allocation failed");
+  }
+  cudaStream_t ss = h->stats_stream;
+  // after the launches that wrote the rows: the group streams of the last fused call, or the main stream; the main stream is
+  // NOT made to join anything (as rbis_batch_stats_snapshot_enqueue)
+  if (h->groups_dirty) {
+    for (int g = 0; g < h->n_groups; g++) CUDA_TRY(cudaStreamWaitEvent(ss, h->gdone[h->last_ring][g], 0));
+  }
+  if (!h->syn_evt) CUDA_TRY(cudaEventCreateWithFlags(&h->syn_evt, cudaEventDisableTiming));
+  CUDA_TRY(cudaEventRecord(h->syn_evt, h->stream));
+  CUDA_TRY(cudaStreamWaitEvent(ss, h->syn_evt, 0));
+  // scratch: truth vec [n_rows][21] | truth quat [n_rows][4] | tables [n_rows][nch][96] | totals [n_rows][96]
+  double* d_tvec = scratch.p;
+  double* d_tquat = d_tvec + (size_t)n_rows * 21;
+  double* d_tables = d_tquat + (size_t)n_rows * 4;
+  double* d_totals = d_tables + (size_t)n_rows * n_table;
+  std::vector<double> tbuf((size_t)n_rows * 25);
+  std::memcpy(tbuf.data(), truth_vec, (size_t)n_rows * 21 * sizeof(double));
+  std::memcpy(tbuf.data() + (size_t)n_rows * 21, truth_quat, (size_t)n_rows * 4 * sizeof(double));
+  if (int rc = upload_small(h, d_tvec, tbuf.data(), tbuf.size() * sizeof(double), ss)) return rc;
+  rbisk::StatsRecords src{};
+  src.k = (long long)k;
+  src.kf = __builtin_popcountll(rec.fields);
+  src.base = (rec.cov_blocks & 1) ? 3 : 0;
+  constexpr int64_t kMaxY = 65535;  // gridDim.y limit
+  for (int64_t r0 = 0; r0 < n_rows; r0 += kMaxY) {
+    const int64_t ny = std::min<int64_t>(kMaxY, n_rows - r0);
+    src.rows = rec.out + (size_t)(first_row + r0) * k * N;
+    rbisk::stats_kernel<<<dim3((unsigned)nch, (unsigned)ny), chunk, chunk * sizeof(double), ss>>>(
+        src, d_tvec + r0 * 21, d_tquat + r0 * 4, 0, (long long)N, nullptr, d_tables + (size_t)r0 * n_table);
+    CUDA_TRY(cudaGetLastError());
+    h->launches++;
+  }
+  CUDA_TRY(cudaMemcpyAsync(out_chunks, d_tables, (size_t)n_rows * n_table * sizeof(double), cudaMemcpyDeviceToHost, ss));
+  if (out_totals) {
+    rbisk::reduce_chunk_table_kernel<<<(unsigned)n_rows, 128, 0, ss>>>(d_tables, (long long)nch, d_totals);
+    CUDA_TRY(cudaGetLastError());
+    h->launches++;
+    CUDA_TRY(cudaMemcpyAsync(out_totals, d_totals, (size_t)n_rows * RBIS_NUM_STATS * sizeof(double), cudaMemcpyDeviceToHost, ss));
+  }
+  CUDA_TRY(cudaEventRecord(rd->done, ss));
+  rd->pending = true;
+  CUDA_TRY(cudaEventRecord(h->rec_stats_done, ss));
+  h->rec_stats_pending = true;
   const int t = h->next_ticket;
   h->next_ticket = (t + 1) % 8;
   CUDA_TRY(cudaEventRecord(h->tickets[t], ss));
@@ -1634,7 +1764,7 @@ int rbis_batch_stats_allreduce(rbis_batch_t* h, void* nccl_comm, const double* t
   // exact in any order (x + 0 = x), SURVEY.md 8e
   CUDA_TRY(cudaMemsetAsync(d_table, 0, n_table * sizeof(double), h->stream));
   rbisk::stats_kernel<<<(unsigned)nch, chunk, chunk * sizeof(double), h->stream>>>(
-      h->vec, h->quat, h->P, h->loglik, d_truth, d_truth + 21, 0, (long long)N, nullptr, d_table + (size_t)first_chunk * RBIS_NUM_STATS);
+      rbisk::StatsArrays{h->vec, h->quat, h->P, h->loglik}, d_truth, d_truth + 21, 0, (long long)N, nullptr, d_table + (size_t)first_chunk * RBIS_NUM_STATS);
   CUDA_TRY(cudaGetLastError());
   h->launches++;
   if (allreduce) {

@@ -585,6 +585,28 @@ __device__ __forceinline__ void g_record_fields(const KParams& p, const double* 
     }
     if (active) d[(long long)pos * N] = v;
   });
+  // ---- covariance blocks (see RecK): position popcount(fields) + q, q = jj (jj + 1) / 2 + ii, belongs to lane l when it is l
+  // modulo G; the value is the element the SNAPSHOT branch stores for slot(i, j)
+  const unsigned cb = p.rec_cov_blocks;
+  if (!cb) return;
+  const int kf = __popcll(fields), nb = 3 * __popc(cb), nq = nb * (nb + 1) / 2;
+  double* const dc = d + (long long)kf * N;
+  int q = (l - kf) & (G - 1), jj = 0, ii = q;
+  while (ii > jj) { ii -= jj + 1; jj++; }
+  for (; q < nq; q += G) {
+    const int i = rec_cov_state(cb, ii), j = rec_cov_state(cb, jj);
+    double v;
+    if constexpr (DC) {
+      if (is_act(i) && is_act(j)) v = Pf[act_pos(i) * LD + act_pos(j)];
+      else if (j < 3 || (i >= 12 && j < 15)) v = imu_seen ? ((i != j) ? 0.0 : (j < 3 ? qn.q_gyro : qn.q_accel)) : p.P[(long long)slot(i, j) * N + n];
+      else v = 0.0;  // kAct.rest: exactly zero in a decoupled filter
+    } else {
+      v = Pf[i * LD + j];
+    }
+    if (active) dc[(long long)q * N] = v;
+    ii += G;
+    while (ii > jj) { ii -= jj + 1; jj++; }
+  }
 }
 
 // ------------------------------------------------------------------------------------------------

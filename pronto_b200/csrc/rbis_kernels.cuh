@@ -279,14 +279,35 @@ struct SynK {
 };
 // RBIS_OP_RECORD (REC kernel instantiations): bit f of `fields` records field f -- 0..20 state vector, 21..24 quaternion
 // w, x, y, z, 25 log-likelihood, 26..46 covariance diagonal P(f-26, f-26) -- at out[row * k + pos][n], pos =
-// popcount(fields & ((1 << f) - 1)).  For a host output `out` is the call's staging buffer and the host has renumbered the
-// RECORD rows into it (rbis_batch.cu).
+// popcount(fields & ((1 << f) - 1)).  After the fields, KParams::rec_cov_blocks selects covariance blocks: bit b is state
+// block b (indices 3b..3b+2); with I the ascending selected indices, P(I[ii], I[jj]), ii <= jj, goes to position
+// popcount(fields) + jj (jj + 1) / 2 + ii.  For a host output `out` is the call's staging buffer and the host has renumbered
+// the RECORD rows into it (rbis_batch.cu).
 constexpr int REC_FIELDS = 47;
+constexpr int REC_BLOCKS = 7;
 struct RecK {
   double* out;
   unsigned long long fields;
-  long long k;  // popcount(fields)
+  long long k;  // popcount(fields) + nb (nb + 1) / 2, nb = 3 popcount(rec_cov_blocks)
 };
+// packed position of state index i within the selected covariance blocks cb (i's block selected)
+__host__ __device__ __forceinline__ int rec_cov_index(unsigned cb, int i) {
+#ifdef __CUDA_ARCH__
+  return 3 * __popc(cb & ((1u << (i / 3)) - 1u)) + i % 3;
+#else
+  return 3 * __builtin_popcount(cb & ((1u << (i / 3)) - 1u)) + i % 3;
+#endif
+}
+// the inverse: state index of packed position c
+__host__ __device__ __forceinline__ int rec_cov_state(unsigned cb, int c) {
+  int t = c / 3;
+  for (int b = 0; b < REC_BLOCKS; b++)
+    if ((cb >> b) & 1u) {
+      if (t == 0) return 3 * b + c % 3;
+      t--;
+    }
+  return -1;
+}
 
 struct KParams {
   long long N;
@@ -313,6 +334,8 @@ struct KParams {
   // MASK kernel instantiations only (appended for the same reason): bit s set = stream s has RBIS_STREAM_SKIP_NAN_ROWS, a
   // filter whose row of that stream holds a NaN in a value the update reads skips the MEAS op (see row_missing)
   unsigned skip_nan_streams;
+  // REC kernel instantiations only (appended for the same reason): covariance blocks of the record set (see RecK)
+  unsigned rec_cov_blocks;
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -1354,6 +1377,58 @@ __device__ __forceinline__ void record_fields(const KParams& p, const Cov& P, co
     }
     if (active) d[(long long)__popcll(fields & ((1ull << f) - 1)) * N] = v;
   });
+  // ---- covariance blocks: the values of an RBIS_OP_SNAPSHOT's slot(i, j), loaded through the tiles SNAPSHOT uses.  cb is
+  // uniform, so a tile without a selected slot is skipped by the whole warp and the tensor-memory loads stay warp-aligned.
+  const unsigned cb = p.rec_cov_blocks;
+  if (!cb) return;
+  double* const dc = d + (long long)__popcll(fields) * N;
+  auto sel = [&](int i, int j) { return ((cb >> (i / 3)) & (cb >> (j / 3)) & 1u) != 0; };
+  auto put = [&](int i, int j, double v) {  // i <= j, both blocks selected
+    const int ii = rec_cov_index(cb, i), jj = rec_cov_index(cb, j);
+    if (active) dc[(long long)(jj * (jj + 1) / 2 + ii) * N] = v;
+  };
+  if constexpr (DC) {
+    constexpr int TILE = 12;  // the tiles of cov_store_active
+    static_for<NP_ACT / TILE>([&](auto tc) {
+      constexpr int k0 = tc * TILE;
+      bool any = false;
+      static_for<TILE>([&](auto kc) { any = any || sel(row_of_slot(kAct.s[k0 + kc]), col_of_slot(kAct.s[k0 + kc])); });
+      if (!any) return;
+      Buf<TILE> b;
+      issue<ActRun<k0, TILE>>(P, b);
+      commit<ActRun<k0, TILE>>(b);
+      static_for<TILE>([&](auto kc) {
+        constexpr int s_ = kAct.s[k0 + kc];
+        constexpr int i = row_of_slot(s_), j = col_of_slot(s_);
+        if (sel(i, j)) put(i, j, b.d[kc]);
+      });
+    });
+    static_for<N_REST>([&](auto kc) {
+      constexpr int s_ = kAct.rest[kc];
+      constexpr int i = row_of_slot(s_), j = col_of_slot(s_);
+      if (sel(i, j)) put(i, j, 0.0);
+    });
+    static_for<12>([&](auto kc) {
+      constexpr int s_ = kAct.blk[kc];
+      constexpr int i = row_of_slot(s_), j = col_of_slot(s_);
+      if (sel(i, j))
+        put(i, j, imu_seen ? ((i != j) ? 0.0 : __ldg((j < 3 ? p.q_gyro : p.q_accel) + n)) : p.P[(long long)s_ * N + n]);
+    });
+  } else {
+    static_for<NP / XFER_TILE>([&](auto tc) {  // the tiles of cov_store_all
+      constexpr int s0 = tc * XFER_TILE;
+      bool any = false;
+      static_for<XFER_TILE>([&](auto kc) { any = any || sel(row_of_slot(s0 + kc), col_of_slot(s0 + kc)); });
+      if (!any) return;
+      Buf<XFER_TILE> b;
+      issue<SlotRun<s0, XFER_TILE>>(P, b);
+      commit<SlotRun<s0, XFER_TILE>>(b);
+      static_for<XFER_TILE>([&](auto kc) {
+        constexpr int i = row_of_slot(s0 + kc), j = col_of_slot(s0 + kc);
+        if (sel(i, j)) put(i, j, b.d[kc]);
+      });
+    });
+  }
 }
 
 // ------------------------------------------------------------------------------------------------

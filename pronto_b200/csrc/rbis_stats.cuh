@@ -10,25 +10,55 @@ namespace rbisk {
 constexpr int NSTAT = 96;
 constexpr int NPF = 23;  // per-filter outputs: e[21], NEES, loglik
 
-// One CTA per chunk of blockDim.x filters.  Each statistic is reduced with the same fixed binary
-// tree (stride blockDim/2 ... 1) so the result depends on nothing but the per-filter values and
-// the chunk size: it is identical for any GPU count and reproducible on the host.
-__global__ void __launch_bounds__(1024) stats_kernel(const double* __restrict__ vec, const double* __restrict__ quat,
-                             const double* __restrict__ P, const double* __restrict__ loglik,
-                             const double* __restrict__ tvec, const double* __restrict__ tquat, int per_filter,
-                             long long N, double* __restrict__ out_pf, double* __restrict__ out_chunks) {
+// Where stats_kernel reads its filters: the live arrays or a snapshot slot ([21][N] vec, [4][N] quat, packed [231][N]
+// covariance, [N] loglik; one table, gridDim.y = 1) ...
+struct StatsArrays {
+  const double *vec, *quat, *P, *loglik;
+  __device__ __forceinline__ double x(int f, long long n, long long N) const {  // record field f < 26 (see RecK)
+    return f < 21 ? vec[(long long)f * N + n] : f < 25 ? quat[(long long)(f - 21) * N + n] : loglik[n];
+  }
+  __device__ __forceinline__ double cov(int i, int j, long long n, long long N) const {  // P(3 + i, 3 + j), i <= j < 9
+    return P[(long long)slot(3 + i, 3 + j) * N + n];
+  }
+};
+// ... or record rows ([rows][k][N], the layout of RecK): row blockIdx.y of `rows`, one table per row.  Fields 0..25 sit at
+// positions 0..25; the covariance blocks include v, chi and p, so P(3 + i, 3 + j) is at kf + jj (jj + 1) / 2 + ii with
+// ii = base + i, jj = base + j (base = 3 when the omega block is recorded too).
+struct StatsRecords {
+  const double* rows;
+  long long k;
+  int kf, base;  // popcount(fields); packed covariance index of state index 3
+  __device__ __forceinline__ double x(int f, long long n, long long N) const {
+    return rows[((long long)blockIdx.y * k + f) * N + n];
+  }
+  __device__ __forceinline__ double cov(int i, int j, long long n, long long N) const {
+    const int ii = base + i, jj = base + j;
+    return rows[((long long)blockIdx.y * k + kf + jj * (jj + 1) / 2 + ii) * N + n];
+  }
+};
+
+// One CTA per chunk of blockDim.x filters (and per table: blockIdx.y, with truth [21] / [4] and chunks [gridDim.x][96] per
+// table).  Each statistic is reduced with the same fixed binary tree (stride blockDim/2 ... 1) so the result depends on
+// nothing but the per-filter values and the chunk size: it is identical for any GPU count, for each source, and
+// reproducible on the host.
+template <class Src>
+__global__ void __launch_bounds__(1024) stats_kernel(const Src src, const double* __restrict__ tvec, const double* __restrict__ tquat,
+                                                     int per_filter, long long N, double* __restrict__ out_pf, double* __restrict__ out_chunks) {
   extern __shared__ double red[];
   const int t = threadIdx.x;
   const long long n = (long long)blockIdx.x * blockDim.x + t;
   const bool live = n < N;
+  tvec += (long long)blockIdx.y * 21;
+  tquat += (long long)blockIdx.y * 4;
+  out_chunks += (long long)blockIdx.y * gridDim.x * NSTAT;
   double val[48];
 #pragma unroll
   for (int k = 0; k < 48; k++) val[k] = 0.0;
   if (live) {
     double e[NS];
 #pragma unroll
-    for (int i = 0; i < NS; i++) e[i] = vec[(long long)i * N + n] - (per_filter ? tvec[(long long)i * N + n] : tvec[i]);
-    const Q4 q{quat[n], quat[N + n], quat[2 * N + n], quat[3 * N + n]};
+    for (int i = 0; i < NS; i++) e[i] = src.x(i, n, N) - (per_filter ? tvec[(long long)i * N + n] : tvec[i]);
+    const Q4 q{src.x(21, n, N), src.x(22, n, N), src.x(23, n, N), src.x(24, n, N)};
     const Q4 tq = per_filter ? Q4{tquat[n], tquat[N + n], tquat[2 * N + n], tquat[3 * N + n]}
                              : Q4{tquat[0], tquat[1], tquat[2], tquat[3]};
     const V3 dchi = subtract_quats(q, tq);  // Log(truth^-1 * est)
@@ -38,7 +68,7 @@ __global__ void __launch_bounds__(1024) stats_kernel(const double* __restrict__ 
 #pragma unroll
     for (int j = 0; j < 9; j++)
 #pragma unroll
-      for (int i = 0; i <= j; i++) L[j][i] = P[(long long)slot(3 + i, 3 + j) * N + n];  // lower: L[row][col]
+      for (int i = 0; i <= j; i++) L[j][i] = src.cov(i, j, n, N);  // lower: L[row][col]
     double y[9];
     double nees = 0;
 #pragma unroll
@@ -62,7 +92,7 @@ __global__ void __launch_bounds__(1024) stats_kernel(const double* __restrict__ 
       y[j] = v * rd;
       nees += y[j] * y[j];
     }
-    const double ll = loglik[n];
+    const double ll = src.x(25, n, N);
     bool finite = isfinite(nees) && isfinite(ll);
 #pragma unroll
     for (int i = 0; i < NS; i++) finite = finite && isfinite(e[i]);
@@ -97,14 +127,18 @@ __global__ void __launch_bounds__(1024) stats_kernel(const double* __restrict__ 
     if (t == 0) out_chunks[(long long)blockIdx.x * NSTAT + k] = red[0];
     __syncthreads();
   });
-  if (t >= 48 && t < NSTAT) out_chunks[(long long)blockIdx.x * NSTAT + t] = 0.0;
+  // the reserved statistics 48..95 are zero, also for chunks of fewer than 96 filters
+  for (int k = 48 + t; k < NSTAT; k += blockDim.x) out_chunks[(long long)blockIdx.x * NSTAT + k] = 0.0;
 }
 
 // Final reduction of a chunk table on the device: totals[k] = sum over chunks in ASCENDING chunk order (one thread per
-// statistic, a plain sequential sum: the same order as rbis_stats_reduce_chunks on the host).
+// statistic, a plain sequential sum: the same order as rbis_stats_reduce_chunks on the host).  One CTA per table:
+// table blockIdx.x is [n_chunks][96] at table + blockIdx.x * n_chunks * 96, its totals at totals + blockIdx.x * 96.
 __global__ void reduce_chunk_table_kernel(const double* __restrict__ table, long long n_chunks, double* __restrict__ totals) {
   const int k = threadIdx.x;
   if (k >= NSTAT) return;
+  table += (long long)blockIdx.x * n_chunks * NSTAT;
+  totals += (long long)blockIdx.x * NSTAT;
   double s = 0.0;
   for (long long c = 0; c < n_chunks; c++) s = __dadd_rn(s, table[c * NSTAT + k]);
   totals[k] = s;

@@ -47,6 +47,34 @@ int rbis_batch_get_filter_states(rbis_batch_t* h, int64_t first, int64_t count, 
   return 0;
 }
 
+int rbis_record_filter_states(uint64_t fields, int32_t cov_blocks, const double* row, int64_t n_filters, int64_t utime,
+                              int64_t first, int64_t count, rbis_filter_state_t* out) {
+  if (!row || !out) return rbis_set_error(RBIS_ERR_INVALID, "null argument");
+  if ((fields & 0x1FFFFFFull) != 0x1FFFFFFull || (fields >> 47) != 0)
+    return rbis_set_error(RBIS_ERR_INVALID, "record fields 0x%llx: need fields 0..24 (vec, quat) and nothing above 46", (unsigned long long)fields);
+  if (cov_blocks != 0x7F) return rbis_set_error(RBIS_ERR_INVALID, "record cov_blocks 0x%x: need all seven blocks (0x7f)", (unsigned)cov_blocks);
+  if (n_filters <= 0 || first < 0 || count < 0 || first + count > n_filters)
+    return rbis_set_error(RBIS_ERR_INVALID, "filter range out of bounds");
+  // all seven blocks: packed covariance index = state index, so P(i, j) sits at kf + slot(i, j)
+  const int64_t kf = __builtin_popcountll(fields);
+  for (int64_t k = 0; k < count; k++) {
+    const int64_t n = first + k;
+    rbis_filter_state_t& m = out[k];
+    m.utime = utime;
+    m.num_states = RBIS_NUM_STATES;
+    m.num_cov_elements = RBIS_NUM_STATES * RBIS_NUM_STATES;
+    m.reserved0 = m.reserved1 = 0;
+    for (int i = 0; i < 4; i++) m.quat[i] = row[(21 + i) * n_filters + n];
+    for (int i = 0; i < 21; i++) m.state[i] = row[i * n_filters + n];
+    for (int j = 0; j < 21; j++)
+      for (int i = 0; i < 21; i++) {
+        const int64_t s = i <= j ? j * (j + 1) / 2 + i : i * (i + 1) / 2 + j;
+        m.cov[i + 21 * j] = row[(kf + s) * n_filters + n];  // column-major, both triangles (rbis.cpp:282)
+      }
+  }
+  return 0;
+}
+
 int rbis_batch_set_filter_states(rbis_batch_t* h, int64_t first, int64_t count, const rbis_filter_state_t* msgs) {
   if (!h || !msgs) return rbis_set_error(RBIS_ERR_INVALID, "null argument");
   const int64_t N = rbis_batch_num_filters(h);
