@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """dev/all_kernels_check.py -- one small pass through every fused-kernel family with a bit-identity check (compute-sanitizer is closed on the GPU pool):
 lane-per-filter decoupled + dense, warp-group 4 / 8 lanes, SYN instantiations, snapshot / restore, snapshot statistics, the
-REC instantiations (RBIS_OP_RECORD) and the MASK instantiations (RBIS_STREAM_SKIP_NAN_ROWS, with and without records) over the
-same mappings and variants."""
+REC instantiations (RBIS_OP_RECORD), the MASK instantiations (RBIS_STREAM_SKIP_NAN_ROWS, with and without records) and the
+innovation sets (rbis_batch_set_innovations, REC instantiations: in-order, rewound, synthesised and masked programs) over the same
+mappings and variants."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -123,4 +124,52 @@ for cfg in (dict(mapping=1, lane_filters_per_cta=384), dict(mapping=1, lane_filt
         same = same and not np.isnan(got[0]).any()
         print("masked", cfg, "records" if with_rec else "", "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
         assert same and variant & 512
+# innovation sets: NIS, y and S(a,a) of every MEAS op of both streams; the rows of the rewound program equal those of the same
+# program's replay, the state equals the program without innovation sets
+INNOV = capi.INNOV_NIS | capi.INNOV_Y | capi.INNOV_S_DIAG
+
+
+def innov_bufs():
+    return [torch.full((st["legodo"].shape[0], 7, N), float("nan"), dtype=torch.float64, device="cuda"),
+            torch.full((st["pose_z"].shape[0], 13, N), float("nan"), dtype=torch.float64, device="cuda")]
+
+
+ref_innov = {}
+for cfg in (dict(mapping=1, lane_filters_per_cta=384), dict(mapping=1, lane_filters_per_cta=128), dict(mapping=1, dense_only=True),
+            dict(mapping=4), dict(mapping=8), dict(mapping=4, dense_only=True)):
+    for key, streams, want_state in (("plain", gpu_streams(st), ref_state), ("masked", masked(lego, pose_z), ref_mask)):
+        bufs = innov_bufs()
+        with RBISBatch(N, snapshot_slots=2, **cfg) as b:
+            b.set_process_noise(*nominal_q())
+            b.set_state(sc["vec"], sc["quat"], sc["cov"])
+            for s_, m_ in ((0, 3), (1, 6)):
+                b.set_innovations(s_, bufs[s_], m_, INNOV)
+            b.run_fused(prog, imu=st["imu"], streams=streams)
+            variant = b.last_kernel_variant
+            got = b.get_state()
+        rows_ = [x.cpu().numpy() for x in bufs]
+        ref_innov.setdefault(key, rows_)
+        same = all(np.array_equal(x, y, equal_nan=True) for x, y in zip(rows_, ref_innov[key]))
+        same = same and all(np.array_equal(x, y) for x, y in zip(got[:4], want_state[:4]))
+        same = same and (key == "masked" or not any(np.isnan(x).any() for x in rows_))
+        print("innovations", key, cfg, "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
+        assert same and variant & 8
+ref_innov = None
+for cfg in (dict(mapping=1), dict(mapping=4), dict(mapping=8), dict(mapping=1, synth_materialize=True)):
+    bufs = innov_bufs()
+    with RBISBatch(N, **cfg) as b:
+        b.set_process_noise(*nominal_q())
+        b.set_state(sc["vec"], sc["quat"], sc["cov"])
+        for s_, m_ in ((0, 3), (1, 6)):
+            b.set_innovations(s_, bufs[s_], m_, INNOV)
+        b.run_fused_synth(ev, [MeasStream(synth.LEGODO_IDX, None, st["R_legodo"]), MeasStream(synth.POSE_IDX, None, st["R_pose"], quat=True)],
+                          SynthSpec(synth.SEED, d["imu_mean"], d["imu_step"], d["streams"], mode=1))
+        variant = b.last_kernel_variant
+        b.synchronize()
+    rows_ = [x.cpu().numpy() for x in bufs]
+    if ref_innov is None:
+        ref_innov = rows_
+    same = all(np.array_equal(x, y) for x, y in zip(rows_, ref_innov)) and not any(np.isnan(x).any() for x in rows_)
+    print("innovations synth", cfg, "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
+    assert same and variant & 8
 print("ok")

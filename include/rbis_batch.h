@@ -186,8 +186,9 @@ int64_t rbis_batch_launch_count(const rbis_batch_t* h);
  * rbis_batch_config_t::dense_only), +1 when the program has measurement chunks other than uncorrelated aligned index
  * triples (the instantiations that also contain the one-row and the correlated-block updates), +4 when the kernel drew its
  * input rows itself (rbis_batch_run_fused_synth, SYN instantiations), + 16 * lanes per filter for the warp-group kernels
- * (rbis_batch_config_t::mapping > 1), +8 when the program records (RBIS_OP_RECORD: the REC instantiations, which programs without
- * records never run), +512 when a stream has RBIS_STREAM_SKIP_NAN_ROWS (the MASK instantiations, which contain the one-row and
+ * (rbis_batch_config_t::mapping > 1), +8 for the REC instantiations, which run when the program records (RBIS_OP_RECORD) or a MEAS op
+ * of it writes an innovation set (rbis_batch_set_innovations) and never otherwise, +1024 more when they carry the innovation path
+ * (the program writes an innovation set: programs that only record do not run that code), +512 when a stream has RBIS_STREAM_SKIP_NAN_ROWS (the MASK instantiations, which contain the one-row and
  * correlated-block updates whatever +1 says); -1 before the first launch. */
 int rbis_batch_last_kernel_variant(const rbis_batch_t* h);
 
@@ -268,6 +269,40 @@ typedef struct {
  * record set fails with RBIS_ERR_STATE, a row outside [0, rows) with RBIS_ERR_INVALID, both before anything is enqueued.  The
  * single-update entry points do not record. */
 int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec);
+
+/* ---- innovation sets: the innovation sequence of every measurement update, the consistency check that needs no truth (a log
+ * replay, a sweep of R or Q).  For a MEAS op on a stream with index set idx[0..m-1], from the PRIOR state of the op (x-, P-) as
+ * the reference's update forms them (MSE/rbis.cpp:124-143):
+ *   y_a    = z_a - x-[idx_a]; at the chi indices of an orientation stream, component idx_a - 6 of subtract_quats(meas_quat, quat)
+ *   S(a,a) = P-(idx_a, idx_a) + R(a,a), R's diagonal from the shared table, the row's table (RBIS_R_PER_ROW_FULL) or R[a][n]
+ *            (RBIS_R_PER_FILTER_DIAG)
+ *   NIS    = y^T S^-1 y with the full S: the sum of the quadratic forms of the update's chunks (the kernels apply an update as
+ *            chunks of uncorrelated rows, and decorrelated scalar rows inside a correlated block); by the chain rule of the Gaussian
+ *            likelihood that equals the single update's y^T S^-1 y up to rounding.  A consistent filter has NIS ~ chi2(m).
+ * out is DEVICE memory [rows][k][N], k = NIS + m Y + m S_DIAG: the chosen fields in the order NIS, y_0..y_m-1, S(0,0)..S(m-1,m-1),
+ * filter index fastest.  Every MEAS op on stream slot `stream` of a later rbis_batch_run_fused / rbis_batch_run_fused_synth call
+ * writes row op.row for every active filter:
+ *   - a filter that skips the row (RBIS_STREAM_SKIP_NAN_ROWS) writes NaN into all k entries;
+ *   - a row applied more than once holds the values of its last application (after a RESTORE and replay, the replayed one);
+ *   - rows no MEAS op writes keep their contents; column maps do not apply (the values are per filter).
+ * `out` is valid once a ticket recorded after the call has been waited for (rbis_batch_record / rbis_batch_wait) or after
+ * rbis_batch_synchronize.  The single-update entry points, and calls with fewer than stream + 1 streams, ignore the set. */
+#define RBIS_INNOV_NIS    1   /* y^T S^-1 y: 1 entry */
+#define RBIS_INNOV_Y      2   /* the innovation y: m entries */
+#define RBIS_INNOV_S_DIAG 4   /* S(a,a) = P-(idx_a, idx_a) + R(a,a): m entries */
+typedef struct {
+  uint32_t fields;   /* RBIS_INNOV_* bits, not 0 */
+  int32_t  m;        /* the stream's measurement dimension; a call whose stream `stream` has another m fails */
+  double*  out;      /* DEVICE [rows][k][N], k = NIS + m*Y + m*S_DIAG, in that order, filter index fastest */
+  int64_t  rows;
+} rbis_innovation_t;
+/* Sets the innovation set of stream slot `stream` (0..RBIS_MAX_STREAMS-1) used by the fused calls enqueued after it (handle state
+ * per slot, like the column maps and the record set; a copy of *spec is kept); NULL clears it.  Does not synchronise.  A bad slot,
+ * an unknown or empty `fields`, m outside 1..RBIS_MAX_MEAS and a NULL or non-device `out` are RBIS_ERR_INVALID.  A fused call
+ * whose stream `stream` has another m, or whose MEAS op on it names a row outside [0, rows), fails with RBIS_ERR_INVALID before
+ * anything is enqueued.  Programs that write an innovation set run the REC kernel instantiations with the innovation path
+ * (rbis_batch_last_kernel_variant +8 +1024). */
+int rbis_batch_set_innovations(rbis_batch_t* h, int32_t stream, const rbis_innovation_t* spec);
 
 /* ---- the fused hot path: run `n_ops` ops (host array, executed in order) for every filter in ONE
  * kernel launch, state and covariance resident on chip throughout.  This is the batch form of the
@@ -441,6 +476,18 @@ int rbis_batch_stats_snapshot_enqueue(rbis_batch_t* h, int32_t slot, const doubl
 int rbis_batch_stats_records_enqueue(rbis_batch_t* h, int64_t first_row, int64_t n_rows, const double* truth_vec,
                                      const double* truth_quat, int chunk, double* out_chunks, double* out_totals, int64_t* n_chunks,
                                      int32_t* ticket);
+/* Ensemble statistics of INNOVATION ROWS first_row .. first_row + n_rows - 1 of stream slot `stream`'s innovation set, which must
+ * include RBIS_INNOV_NIS; one chunk table per row, with the side stream, outputs, ticket and ordering of
+ * rbis_batch_stats_records_enqueue (a later fused call whose MEAS ops write into the buffer a pending pass reads waits for it on
+ * the device; alternate two innovation buffers to keep calls overlapping).  Table entries (all others zero):
+ *   [0] sum NIS   [1] sum NIS^2   [2] filters with a finite NIS   [3] of them, NIS inside the central 95 % of chi2(m)
+ *   [4] filters with a non-finite NIS (skipped rows, poisoned filters)   [5] filters
+ *   [6 + a] sum y_a, [15 + a] sum y_a^2 (with RBIS_INNOV_Y)   [24 + a] sum y_a^2 / S(a,a) (with RBIS_INNOV_Y and RBIS_INNOV_S_DIAG)
+ * Only filters with a finite NIS enter [0], [1], [3] and [6..32].  Each chunk is reduced with the fixed binary tree of the other
+ * statistics, so tables of chunk-aligned shards concatenate and reduce with rbis_stats_reduce_chunks.  ANIS = [0] / [2]; for a
+ * consistent filter ANIS is near m and [15 + a] / [2] near the mean S(a,a), i.e. [24 + a] / [2] near 1 for every axis a. */
+int rbis_batch_stats_innovations_enqueue(rbis_batch_t* h, int32_t stream, int64_t first_row, int64_t n_rows, int chunk,
+                                         double* out_chunks, double* out_totals, int64_t* n_chunks, int32_t* ticket);
 /* ---- statistics of a SHARDED ensemble (SURVEY.md 8e): one process per GPU, each handle holds the contiguous filter range
  * [first_chunk * chunk, first_chunk * chunk + N) of an ensemble of total_chunks chunks.  The shard's chunk partials are written
  * into its rows of a zero-initialised DEVICE table [total_chunks][RBIS_NUM_STATS], the table is summed over the ranks with

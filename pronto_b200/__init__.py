@@ -4,8 +4,8 @@ The product is librbis_b200.so (CUDA sm_100a, C ABI in include/rbis_batch.h); th
 Python host mirror used by tests, bench.py and the multi-GPU driver.  No CPU compute path exists.
 """
 from . import capi  # noqa: F401
-from .batch import (MeasStream, RBISBatch, SynthSpec, filter_states_from_record, make_ops, measure_fp64_peak,  # noqa: F401
-                    record_cov_blocks, record_fields, record_layout, reduce_chunks)
+from .batch import (MeasStream, RBISBatch, SynthSpec, filter_states_from_record, innovation_layout, make_ops,  # noqa: F401
+                    measure_fp64_peak, record_cov_blocks, record_fields, record_layout, reduce_chunks)
 
 __all__ = ["capi", "RBISBatch", "MeasStream", "make_ops", "record_fields", "record_layout", "record_cov_blocks",
-           "filter_states_from_record", "reduce_chunks", "measure_fp64_peak"]
+           "filter_states_from_record", "innovation_layout", "reduce_chunks", "measure_fp64_peak"]

@@ -184,6 +184,22 @@ def record_layout(mask, cov_blocks=()):
     return names
 
 
+def innovation_layout(m, fields):
+    """Names of the entries of an innovation row in output order: 'nis', then 'y<a>' and 's<a>' (S(a,a)) for a < m, as the
+    RBIS_INNOV_* bits of `fields` select them."""
+    m, fields = int(m), int(fields)
+    if not 1 <= m <= capi.MAX_MEAS:
+        raise ValueError(f"innovation m = {m} outside 1..{capi.MAX_MEAS}")
+    if fields <= 0 or fields & ~(capi.INNOV_NIS | capi.INNOV_Y | capi.INNOV_S_DIAG):
+        raise ValueError(f"innovation fields {fields:#x}: need a non-empty set of INNOV_NIS / INNOV_Y / INNOV_S_DIAG")
+    names = ["nis"] if fields & capi.INNOV_NIS else []
+    if fields & capi.INNOV_Y:
+        names += [f"y{a}" for a in range(m)]
+    if fields & capi.INNOV_S_DIAG:
+        names += [f"s{a}" for a in range(m)]
+    return names
+
+
 def make_ops(entries):
     """entries: iterable of (kind, stream, row, utime, dt) -> structured numpy op array."""
     entries = list(entries)
@@ -434,6 +450,42 @@ class RBISBatch:
 
     def clear_record(self):
         capi.check(self.lib.rbis_batch_set_record(self.h, None))
+
+    # ---- innovation sets ----
+    def set_innovations(self, stream, out, m, fields=capi.INNOV_NIS | capi.INNOV_Y | capi.INNOV_S_DIAG):
+        """Innovation set of stream slot `stream` (rbis_batch_set_innovations): every MEAS op on that stream of later fused calls
+        writes row op.row of out, a CUDA float64 tensor [rows][k][N] with the entries of innovation_layout(m, fields).  Valid after
+        wait(record()) or synchronize().  Does not synchronise."""
+        try:
+            k = len(innovation_layout(m, fields))
+        except ValueError:
+            k = None  # the library refuses it with its own message
+        if k is not None and (out.ndim != 3 or tuple(out.shape[1:]) != (k, self.N)):
+            raise ValueError(f"innovation output must be [rows][{k}][{self.N}], got {tuple(out.shape)}")
+        p, _ = _ptr(out, None, "out")
+        spec = capi.Innovation()
+        spec.fields, spec.m, spec.out, spec.rows = int(fields), int(m), p, int(out.shape[0])
+        capi.check(self.lib.rbis_batch_set_innovations(self.h, int(stream), C.byref(spec)))
+        self._pending_keep = getattr(self, "_pending_keep", [])
+        self._innov_out = getattr(self, "_innov_out", {})
+        self._pending_keep.append(self._innov_out.get(int(stream)))
+        self._innov_out[int(stream)] = out
+
+    def clear_innovations(self, stream):
+        capi.check(self.lib.rbis_batch_set_innovations(self.h, int(stream), None))
+
+    def stats_innovations_enqueue(self, stream, first_row, out_chunks, out_totals=None, chunk=1024):
+        """Statistics of innovation rows first_row .. first_row + n_rows - 1 of stream slot `stream`'s innovation set on the
+        statistics side stream (rbis_batch_stats_innovations_enqueue): out_chunks a PINNED host array [n_rows][n_chunks][96] (n_rows
+        is its first dimension), out_totals a PINNED host array [n_rows][96] or None.  Returns the ticket to wait() for."""
+        n_rows = int(out_chunks.shape[0])
+        n_chunks = (self.N + chunk - 1) // chunk
+        po, _ = _ptr(out_chunks, (n_rows, n_chunks, capi.NUM_STATS), "out_chunks")
+        pt, _ = _ptr(out_totals, (n_rows, capi.NUM_STATS), "out_totals")
+        nch, t = C.c_int64(0), C.c_int32(0)
+        capi.check(self.lib.rbis_batch_stats_innovations_enqueue(self.h, int(stream), int(first_row), n_rows, int(chunk), po, pt,
+                                                                 C.byref(nch), C.byref(t)))
+        return t.value
 
     def run_prepared(self, prep):
         capi.check(self.lib.rbis_batch_run_fused(self.h, *prep[:7]))

@@ -20,6 +20,7 @@ MEM_F32_ROWS = 4  # rbis_batch_run_fused: imu / z / quat are float32 arrays (wid
 OP_IMU, OP_MEAS, OP_SNAPSHOT, OP_RESTORE, OP_RECORD = 0, 1, 2, 3, 4
 REC_FIELDS = 47  # record fields: 0..20 vec, 21..24 quat w,x,y,z, 25 loglik, 26..46 covariance diagonal
 REC_BLOCKS = 7   # record covariance blocks: state indices 3b..3b+2 (omega, v, chi, p, a, gyro bias, accel bias)
+INNOV_NIS, INNOV_Y, INNOV_S_DIAG = 1, 2, 4  # rbis_innovation_t::fields: NIS (1 entry), y (m entries), S(a,a) (m entries)
 R_SHARED_FULL, R_PER_FILTER_DIAG, R_PER_ROW_FULL = 0, 1, 2
 STREAM_SKIP_NAN_ROWS = 1  # rbis_stream_t::flags: a filter whose row holds a NaN in a value the update reads skips that update
 
@@ -122,6 +123,15 @@ class Record(C.Structure):
     ]
 
 
+class Innovation(C.Structure):
+    _fields_ = [
+        ("fields", C.c_uint32),
+        ("m", C.c_int32),
+        ("out", C.c_void_p),
+        ("rows", C.c_int64),
+    ]
+
+
 class Op(C.Structure):
     _fields_ = [
         ("kind", C.c_int32),
@@ -159,6 +169,7 @@ PROTOTYPES = {
     "rbis_batch_indexed_orient_update": (C.c_int, [C.c_void_p, C.c_int, c_int32_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int]),
     "rbis_batch_set_column_map": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
     "rbis_batch_set_record": (C.c_int, [C.c_void_p, C.POINTER(Record)]),
+    "rbis_batch_set_innovations": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(Innovation)]),
     "rbis_batch_run_fused": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Op), C.c_void_p, C.c_int64, C.c_int, C.POINTER(Stream), C.c_int]),
     "rbis_batch_synthesize": (C.c_int, [C.c_void_p, C.POINTER(Synth), C.c_void_p, C.c_void_p, C.c_void_p]),
     "rbis_batch_run_fused_synth": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Op), C.c_int, C.POINTER(Stream), C.POINTER(Synth)]),
@@ -184,6 +195,8 @@ PROTOTYPES = {
                                                      C.POINTER(C.c_int32)]),
     "rbis_batch_stats_records_enqueue": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p,
                                                     C.c_void_p, c_int64_p, C.POINTER(C.c_int32)]),
+    "rbis_batch_stats_innovations_enqueue": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_int, C.c_void_p, C.c_void_p,
+                                                        c_int64_p, C.POINTER(C.c_int32)]),
     "rbis_batch_stats_allreduce": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p]),
     "rbis_batch_window_neg_loglik": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int,
                                                C.c_void_p, C.c_void_p, C.c_int]),

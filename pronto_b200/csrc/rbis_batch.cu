@@ -179,17 +179,22 @@ struct rbis_batch {
   std::vector<cudaEvent_t> snap_read_evt;   // per slot, created on first use
   std::vector<char> snap_read_pending;
   std::vector<DevBuf> snap_stats_scratch;   // per slot: truth [25] + chunk partials
-  // ---- statistics over record rows (rbis_batch_stats_records_enqueue), on the same side stream: per device record buffer a
-  // pending pass reads, the event after that pass; a fused call whose RECORD ops write into the buffer waits for it
-  struct RecReader {
-    const double *lo, *hi;  // [lo, hi): the record buffer
+  // ---- statistics over record or innovation rows (rbis_batch_stats_records_enqueue, rbis_batch_stats_innovations_enqueue),
+  // on the same side stream: per device buffer a pending pass reads, the event after that pass; a fused call whose RECORD or
+  // MEAS ops write into the buffer waits for it
+  struct RowReader {
+    const double *lo, *hi;  // [lo, hi): the record or innovation buffer
     cudaEvent_t done;
     bool pending;
   };
-  std::vector<RecReader> rec_readers;
-  DevBuf rec_stats_scratch;                 // truth [rows][25] + tables [rows][chunks][96] + totals [rows][96]
+  std::vector<RowReader> row_readers;
+  DevBuf rec_stats_scratch;                 // [truth [rows][25]] + tables [rows][chunks][96] + totals [rows][96]
   cudaEvent_t rec_stats_done = nullptr;     // the last pass (scratch reuse)
   bool rec_stats_pending = false;
+  // ---- innovation sets (rbis_batch_set_innovations), per stream slot: MEAS ops on the stream write rows of innov[s].out
+  bool innov_set[RBIS_MAX_STREAMS] = {};
+  rbis_innovation_t innov[RBIS_MAX_STREAMS] = {};
+  int innov_k[RBIS_MAX_STREAMS] = {};       // doubles per filter and row: NIS + m y + m S_DIAG
 };
 
 namespace {
@@ -200,6 +205,8 @@ constexpr int kRShared = rbisk::RS_STRIDE;
 
 static_assert(rbisk::OP_IMU == RBIS_OP_IMU && rbisk::OP_MEAS == RBIS_OP_MEAS && rbisk::OP_SNAPSHOT == RBIS_OP_SNAPSHOT &&
               rbisk::OP_RECORD == RBIS_OP_RECORD, "op kinds of the kernels and of the C ABI differ");
+static_assert(rbisk::INNOV_NIS == RBIS_INNOV_NIS && rbisk::INNOV_Y == RBIS_INNOV_Y && rbisk::INNOV_S_DIAG == RBIS_INNOV_S_DIAG,
+              "innovation fields of the kernels and of the C ABI differ");
 
 constexpr int kMaxSmemOptin = 232448;
 const rbis_fused_tu_t* const kTus[] = {&rbis_fused_tu_dense, &rbis_fused_tu_dc384, &rbis_fused_tu_dc256, &rbis_fused_tu_dc128,
@@ -252,11 +259,12 @@ LaunchGeom launch_geom(int variant, int mapping, int lane_tpb, long long N, int 
   return g;
 }
 
-// variant bit 3: the program records (REC instantiations); bit 9 (+512): a stream skips NaN rows (MASK instantiations)
-constexpr int kVariantMask = 512;
+// variant bit 3: the program records or writes innovation sets (REC instantiations); bit 9 (+512): a stream skips NaN rows (MASK
+// instantiations); bit 10 (+1024): the REC instantiations with the innovation path (INNOV)
+constexpr int kVariantMask = 512, kVariantInnov = 1024;
 cudaError_t launch_variant(int variant, int syn, const LaunchGeom& g, unsigned blocks, cudaStream_t st, const rbisk::KParams& kp) {
-  return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, (variant & 8) ? 1 : 0, (variant & kVariantMask) ? 1 : 0, blocks, g.threads,
-                      g.smem, st, &kp);
+  const int rec = (variant & kVariantInnov) ? 2 : (variant & 8) ? 1 : 0;
+  return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, rec, (variant & kVariantMask) ? 1 : 0, blocks, g.threads, g.smem, st, &kp);
 }
 
 // Automatic choice of the mapping (rbis_batch_config_t::mapping == 0) from the ensemble size: cycles per filter step of one
@@ -475,11 +483,103 @@ int r_table(const double* R, const rbisk::StreamDesc& d, double* out) {
 extern "C" int synthesize_into(rbis_batch_t* h, const rbis_synth_t* syn, double* imu_out, double* const* z_out, double* const* quat_out, cudaStream_t stream);
 namespace {
 
+// Pending side-stream passes that read [lo, hi): their events go to `waits` and they stop being pending.
+void take_readers(rbis_batch* h, const double* lo, const double* hi, std::vector<cudaEvent_t>& waits) {
+  for (auto& r : h->row_readers)
+    if (r.pending && r.lo < hi && lo < r.hi) {
+      waits.push_back(r.done);
+      r.pending = false;
+    }
+}
+
+// The side-stream pass of rbis_batch_stats_records_enqueue / rbis_batch_stats_innovations_enqueue over n_rows rows of the
+// device buffer [lo, hi): the reader entry of the buffer, the scratch ([pre] + tables [n_rows][nch][96] + totals
+// [n_rows][96]), ordering after the launches that wrote the rows, `pre` uploaded, launch(ss, d_pre, d_tables, r0, ny, nch)
+// for the tables of rows r0..r0+ny-1 (at most 65535 rows, the gridDim.y limit), the tables and optional totals copied out,
+// the reader event and a ticket.
+template <class Launch>
+int row_stats_pass(rbis_batch* h, const double* lo, const double* hi, int64_t n_rows, int chunk, const std::vector<double>& pre,
+                   double* out_chunks, double* out_totals, int64_t* n_chunks, int32_t* ticket, Launch&& launch) {
+  if (int rc = use_device(h)) return rc;
+  if (!h->stats_stream) {
+    CUDA_TRY(cudaStreamCreateWithFlags(&h->stats_stream, cudaStreamNonBlocking));
+    h->snap_read_evt.assign((size_t)h->cfg.snapshot_slots, nullptr);
+    h->snap_read_pending.assign((size_t)h->cfg.snapshot_slots, 0);
+    h->snap_stats_scratch.resize((size_t)h->cfg.snapshot_slots);
+  }
+  if (!h->rec_stats_done) CUDA_TRY(cudaEventCreateWithFlags(&h->rec_stats_done, cudaEventDisableTiming));
+  // the reader entry of this buffer (buffers no pass reads any more are dropped)
+  rbis_batch::RowReader* rd = nullptr;
+  for (auto& r : h->row_readers)
+    if (r.lo == lo && r.hi == hi) rd = &r;
+  if (!rd) {
+    for (size_t i = 0; i < h->row_readers.size();)
+      if (!h->row_readers[i].pending) {
+        cudaEventDestroy(h->row_readers[i].done);
+        h->row_readers.erase(h->row_readers.begin() + (long)i);
+      } else {
+        i++;
+      }
+    cudaEvent_t e;
+    CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    h->row_readers.push_back({lo, hi, e, false});
+    rd = &h->row_readers.back();
+  }
+  const size_t N = (size_t)h->N;
+  const int64_t nch = (int64_t)((N + chunk - 1) / chunk);
+  const size_t n_table = (size_t)nch * RBIS_NUM_STATS;
+  const size_t need = pre.size() + (size_t)n_rows * (n_table + RBIS_NUM_STATS);
+  DevBuf& scratch = h->rec_stats_scratch;
+  if (scratch.cap < need) {
+    if (h->rec_stats_pending) CUDA_TRY(cudaEventSynchronize(h->rec_stats_done));  // the last pass still reads the old scratch
+    if (scratch.ensure(need)) return fail(RBIS_ERR_ALLOC, "scratch allocation failed");
+  }
+  cudaStream_t ss = h->stats_stream;
+  // after the launches that wrote the rows: the group streams of the last fused call, or the main stream; the main stream is
+  // NOT made to join anything (as rbis_batch_stats_snapshot_enqueue)
+  if (h->groups_dirty) {
+    for (int g = 0; g < h->n_groups; g++) CUDA_TRY(cudaStreamWaitEvent(ss, h->gdone[h->last_ring][g], 0));
+  }
+  if (!h->syn_evt) CUDA_TRY(cudaEventCreateWithFlags(&h->syn_evt, cudaEventDisableTiming));
+  CUDA_TRY(cudaEventRecord(h->syn_evt, h->stream));
+  CUDA_TRY(cudaStreamWaitEvent(ss, h->syn_evt, 0));
+  double* d_pre = scratch.p;
+  double* d_tables = d_pre + pre.size();
+  double* d_totals = d_tables + (size_t)n_rows * n_table;
+  if (!pre.empty())
+    if (int rc = upload_small(h, d_pre, pre.data(), pre.size() * sizeof(double), ss)) return rc;
+  constexpr int64_t kMaxY = 65535;  // gridDim.y limit
+  for (int64_t r0 = 0; r0 < n_rows; r0 += kMaxY) {
+    const int64_t ny = std::min<int64_t>(kMaxY, n_rows - r0);
+    launch(ss, d_pre, d_tables + (size_t)r0 * n_table, r0, ny, nch);
+    CUDA_TRY(cudaGetLastError());
+    h->launches++;
+  }
+  CUDA_TRY(cudaMemcpyAsync(out_chunks, d_tables, (size_t)n_rows * n_table * sizeof(double), cudaMemcpyDeviceToHost, ss));
+  if (out_totals) {
+    rbisk::reduce_chunk_table_kernel<<<(unsigned)n_rows, 128, 0, ss>>>(d_tables, (long long)nch, d_totals);
+    CUDA_TRY(cudaGetLastError());
+    h->launches++;
+    CUDA_TRY(cudaMemcpyAsync(out_totals, d_totals, (size_t)n_rows * RBIS_NUM_STATS * sizeof(double), cudaMemcpyDeviceToHost, ss));
+  }
+  CUDA_TRY(cudaEventRecord(rd->done, ss));
+  rd->pending = true;
+  CUDA_TRY(cudaEventRecord(h->rec_stats_done, ss));
+  h->rec_stats_pending = true;
+  const int t = h->next_ticket;
+  h->next_ticket = (t + 1) % 8;
+  CUDA_TRY(cudaEventRecord(h->tickets[t], ss));
+  *ticket = t;
+  if (n_chunks) *n_chunks = nch;
+  return 0;
+}
+
 // syn != nullptr: the input rows are synthesised on the device into the staging slot (rbis_batch_run_fused_synth) instead of
 // being copied from the host; everything else -- double buffering, overlap with the previous launch -- is the host path's.
+// use_innov = false: the single-update entry points, which ignore innovation sets
 int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const double* imu, int64_t imu_rows,
                  int n_streams, const rbis_stream_t* streams_in, int mem, bool use_maps = true,
-                 const rbis_synth_t* syn = nullptr) {
+                 const rbis_synth_t* syn = nullptr, bool use_innov = true) {
   if (!h) return fail(RBIS_ERR_INVALID, "null handle");
   if (n_ops < 0 || (n_ops > 0 && !ops)) return fail(RBIS_ERR_INVALID, "bad op list");
   if (n_streams < 0 || n_streams > RBIS_MAX_STREAMS) return fail(RBIS_ERR_INVALID, "n_streams out of range");
@@ -519,6 +619,7 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
   bool restores_ok = true, any_snapshot = false;
   bool any_record = false;
   std::vector<int64_t> rec_rows;  // record rows of the call, in op order
+  bool innov_used[RBIS_MAX_STREAMS] = {};  // streams whose innovation set a MEAS op of the call writes
   int64_t last_utime = h->utime;
   for (int64_t i = 0; i < n_ops; i++) {
     const rbis_op_t& o = ops[i];
@@ -534,6 +635,12 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
       case RBIS_OP_MEAS:
         if (o.stream < 0 || o.stream >= n_streams) return fail(RBIS_ERR_INVALID, "op %lld: stream %d out of range", (long long)i, o.stream);
         if (o.row < 0 || o.row >= streams[o.stream].rows) return fail(RBIS_ERR_INVALID, "op %lld: row %lld out of range for stream %d", (long long)i, (long long)o.row, o.stream);
+        if (use_innov && h->innov_set[o.stream]) {
+          if (o.row >= h->innov[o.stream].rows)
+            return fail(RBIS_ERR_INVALID, "op %lld: row %lld out of range for the innovation set of stream %d (%lld rows)", (long long)i,
+                        (long long)o.row, o.stream, (long long)h->innov[o.stream].rows);
+          innov_used[o.stream] = true;
+        }
         last_utime = o.utime;
         break;
       case RBIS_OP_SNAPSHOT:
@@ -585,6 +692,8 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
     const rbis_stream_t& in = streams[s];
     rbisk::StreamDesc& d = kp.streams[s];
     if (int rc = validate_stream(s, in)) return rc;
+    if (use_innov && h->innov_set[s] && h->innov[s].m != in.m)
+      return fail(RBIS_ERR_INVALID, "stream %d has m = %d, its innovation set m = %d", s, in.m, h->innov[s].m);
     if (in.flags & RBIS_STREAM_SKIP_NAN_ROWS) {
       if (syn) return fail(RBIS_ERR_INVALID, "stream %d: RBIS_STREAM_SKIP_NAN_ROWS does not apply to synthesised inputs (z is drawn, not read)", s);
       kp.skip_nan_streams |= 1u << s;
@@ -726,6 +835,15 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
       kp.rec.out = sb.p;
     }
   }
+  // innovation sets: the REC instantiations with the innovation path
+  for (int s = 0; s < n_streams; s++)
+    if (innov_used[s]) {
+      variant |= 8 | kVariantInnov;
+      kp.innov[s].out = h->innov[s].out;
+      kp.innov[s].rows = h->innov[s].rows;
+      kp.innov[s].k = h->innov_k[s];
+      kp.innov[s].fields = (int)h->innov[s].fields;
+    }
   // ---- inputs: stage host arrays on the copy stream (double buffered), or use device arrays in place ----
   StagingSlot& slot = h->slots[h->slot_toggle];
   cudaStream_t cst = h->copy_stream;
@@ -816,16 +934,10 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
         h->snap_read_pending[(size_t)ops[i].row] = 0;
       }
   }
-  // a device record buffer this program writes that a side-stream statistics pass may still be reading
-  if (any_record && !rec_host) {
-    const double* lo = h->rec.out;
-    const double* hi = lo + (size_t)h->rec.rows * (size_t)h->rec_k * N;
-    for (auto& r : h->rec_readers)
-      if (r.pending && r.lo < hi && lo < r.hi) {
-        slot_readers.push_back(r.done);
-        r.pending = false;
-      }
-  }
+  // a device record or innovation buffer this program writes that a side-stream statistics pass may still be reading
+  if (any_record && !rec_host) take_readers(h, h->rec.out, h->rec.out + (size_t)h->rec.rows * (size_t)h->rec_k * N, slot_readers);
+  for (int s = 0; s < n_streams; s++)
+    if (innov_used[s]) take_readers(h, h->innov[s].out, h->innov[s].out + (size_t)h->innov[s].rows * (size_t)h->innov_k[s] * N, slot_readers);
   if (!grouped) {
     if (int rc = main_stream_work(h)) return rc;
     for (cudaEvent_t e : slot_readers) CUDA_TRY(cudaStreamWaitEvent(h->stream, e, 0));
@@ -1142,7 +1254,7 @@ int rbis_batch_destroy(rbis_batch_t* h) {
   h->full_cov.release(); h->misc.release(); h->stats_async.release(); h->stats_table.release(); h->synth_small.release(); h->d_syn.release();
   for (auto& b : h->snap_stats_scratch) b.release();
   for (cudaEvent_t e : h->snap_read_evt) if (e) cudaEventDestroy(e);
-  for (auto& r : h->rec_readers) cudaEventDestroy(r.done);
+  for (auto& r : h->row_readers) cudaEventDestroy(r.done);
   if (h->rec_stats_done) cudaEventDestroy(h->rec_stats_done);
   h->rec_stats_scratch.release();
   if (h->stats_stream) cudaStreamDestroy(h->stats_stream);
@@ -1173,7 +1285,7 @@ int rbis_batch_synchronize(rbis_batch_t* h) {
   if (h->stats_stream) {  // side-stream statistics (rbis_batch_stats_snapshot_enqueue): done too, their slots are free again
     CUDA_TRY(cudaStreamSynchronize(h->stats_stream));
     std::fill(h->snap_read_pending.begin(), h->snap_read_pending.end(), 0);
-    for (auto& r : h->rec_readers) r.pending = false;
+    for (auto& r : h->row_readers) r.pending = false;
     h->rec_stats_pending = false;
   }
   return 0;
@@ -1370,6 +1482,34 @@ int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec) {
   return 0;
 }
 
+int rbis_batch_set_innovations(rbis_batch_t* h, int32_t stream, const rbis_innovation_t* spec) {
+  if (!h) return fail(RBIS_ERR_INVALID, "null handle");
+  if (stream < 0 || stream >= RBIS_MAX_STREAMS) return fail(RBIS_ERR_INVALID, "stream slot %d outside 0..%d", stream, RBIS_MAX_STREAMS - 1);
+  if (!spec) {
+    h->innov_set[stream] = false;
+    return 0;
+  }
+  constexpr uint32_t all = RBIS_INNOV_NIS | RBIS_INNOV_Y | RBIS_INNOV_S_DIAG;
+  if (spec->fields == 0 || (spec->fields & ~all)) return fail(RBIS_ERR_INVALID, "innovation fields 0x%x: a non-empty set of RBIS_INNOV_* bits", spec->fields);
+  if (spec->m < 1 || spec->m > RBIS_MAX_MEAS) return fail(RBIS_ERR_INVALID, "innovation m = %d outside 1..%d", spec->m, RBIS_MAX_MEAS);
+  if (!spec->out) return fail(RBIS_ERR_INVALID, "innovation output is NULL");
+  if (spec->rows <= 0) return fail(RBIS_ERR_INVALID, "innovation rows must be positive");
+  if (int rc = use_device(h)) return rc;
+  cudaPointerAttributes a;
+  cudaError_t e = cudaPointerGetAttributes(&a, spec->out);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail(RBIS_ERR_INVALID, "innovation output: cudaPointerGetAttributes failed: %s", cudaGetErrorString(e));
+  }
+  if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != h->cfg.device)
+    return fail(RBIS_ERR_INVALID, "innovation output is not memory of device %d", h->cfg.device);
+  h->innov[stream] = *spec;
+  h->innov_k[stream] = ((spec->fields & RBIS_INNOV_NIS) ? 1 : 0) + ((spec->fields & RBIS_INNOV_Y) ? spec->m : 0) +
+                       ((spec->fields & RBIS_INNOV_S_DIAG) ? spec->m : 0);
+  h->innov_set[stream] = true;
+  return 0;
+}
+
 int rbis_batch_run_fused(rbis_batch_t* h, int64_t n_ops, const rbis_op_t* ops, const double* imu, int64_t imu_rows,
                          int n_streams, const rbis_stream_t* streams, int mem) {
   if (n_streams > 0 && !streams) return fail(RBIS_ERR_INVALID, "streams is NULL");
@@ -1487,7 +1627,7 @@ static int single_meas(rbis_batch_t* h, int m, const int32_t* idx, const double*
   st.z = z; st.quat = quat; st.R = R; st.rows = 1;
   rbis_op_t op;
   op.kind = RBIS_OP_MEAS; op.stream = 0; op.row = 0; op.utime = utime; op.dt = 0;
-  return launch_fused(h, 1, &op, nullptr, 0, 1, &st, mem, /*use_maps=*/false);
+  return launch_fused(h, 1, &op, nullptr, 0, 1, &st, mem, /*use_maps=*/false, nullptr, /*use_innov=*/false);
 }
 
 int rbis_batch_indexed_update(rbis_batch_t* h, int m, const int32_t* idx, const double* z, const double* R,
@@ -1631,90 +1771,42 @@ int rbis_batch_stats_records_enqueue(rbis_batch_t* h, int64_t first_row, int64_t
   if ((rec.cov_blocks & 0xE) != 0xE) return fail(RBIS_ERR_INVALID, "statistics of record rows need covariance blocks 1, 2 and 3 (v, chi, p)");
   if (n_rows < 1 || first_row < 0 || first_row + n_rows > rec.rows)
     return fail(RBIS_ERR_INVALID, "record rows %lld..%lld outside [0, %lld)", (long long)first_row, (long long)(first_row + n_rows), (long long)rec.rows);
-  if (int rc = use_device(h)) return rc;
-  if (!h->stats_stream) {
-    CUDA_TRY(cudaStreamCreateWithFlags(&h->stats_stream, cudaStreamNonBlocking));
-    h->snap_read_evt.assign((size_t)h->cfg.snapshot_slots, nullptr);
-    h->snap_read_pending.assign((size_t)h->cfg.snapshot_slots, 0);
-    h->snap_stats_scratch.resize((size_t)h->cfg.snapshot_slots);
-  }
-  if (!h->rec_stats_done) CUDA_TRY(cudaEventCreateWithFlags(&h->rec_stats_done, cudaEventDisableTiming));
-  // the reader entry of this buffer (buffers no pass reads any more are dropped)
   const size_t N = (size_t)h->N, k = (size_t)h->rec_k;
-  const double* lo = rec.out;
-  const double* hi = lo + (size_t)rec.rows * k * N;
-  rbis_batch::RecReader* rd = nullptr;
-  for (auto& r : h->rec_readers)
-    if (r.lo == lo && r.hi == hi) rd = &r;
-  if (!rd) {
-    for (size_t i = 0; i < h->rec_readers.size();)
-      if (!h->rec_readers[i].pending) {
-        cudaEventDestroy(h->rec_readers[i].done);
-        h->rec_readers.erase(h->rec_readers.begin() + (long)i);
-      } else {
-        i++;
-      }
-    cudaEvent_t e;
-    CUDA_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-    h->rec_readers.push_back({lo, hi, e, false});
-    rd = &h->rec_readers.back();
-  }
-  const int64_t nch = (int64_t)((N + chunk - 1) / chunk);
-  const size_t n_table = (size_t)nch * RBIS_NUM_STATS;
-  const size_t need = (size_t)n_rows * (25 + n_table + RBIS_NUM_STATS);
-  DevBuf& scratch = h->rec_stats_scratch;
-  if (scratch.cap < need) {
-    if (h->rec_stats_pending) CUDA_TRY(cudaEventSynchronize(h->rec_stats_done));  // the last pass still reads the old scratch
-    if (scratch.ensure(need)) return fail(RBIS_ERR_ALLOC, "scratch allocation failed");
-  }
-  cudaStream_t ss = h->stats_stream;
-  // after the launches that wrote the rows: the group streams of the last fused call, or the main stream; the main stream is
-  // NOT made to join anything (as rbis_batch_stats_snapshot_enqueue)
-  if (h->groups_dirty) {
-    for (int g = 0; g < h->n_groups; g++) CUDA_TRY(cudaStreamWaitEvent(ss, h->gdone[h->last_ring][g], 0));
-  }
-  if (!h->syn_evt) CUDA_TRY(cudaEventCreateWithFlags(&h->syn_evt, cudaEventDisableTiming));
-  CUDA_TRY(cudaEventRecord(h->syn_evt, h->stream));
-  CUDA_TRY(cudaStreamWaitEvent(ss, h->syn_evt, 0));
-  // scratch: truth vec [n_rows][21] | truth quat [n_rows][4] | tables [n_rows][nch][96] | totals [n_rows][96]
-  double* d_tvec = scratch.p;
-  double* d_tquat = d_tvec + (size_t)n_rows * 21;
-  double* d_tables = d_tquat + (size_t)n_rows * 4;
-  double* d_totals = d_tables + (size_t)n_rows * n_table;
+  // uploaded first: truth vec [n_rows][21] | truth quat [n_rows][4]
   std::vector<double> tbuf((size_t)n_rows * 25);
   std::memcpy(tbuf.data(), truth_vec, (size_t)n_rows * 21 * sizeof(double));
   std::memcpy(tbuf.data() + (size_t)n_rows * 21, truth_quat, (size_t)n_rows * 4 * sizeof(double));
-  if (int rc = upload_small(h, d_tvec, tbuf.data(), tbuf.size() * sizeof(double), ss)) return rc;
   rbisk::StatsRecords src{};
   src.k = (long long)k;
   src.kf = __builtin_popcountll(rec.fields);
   src.base = (rec.cov_blocks & 1) ? 3 : 0;
-  constexpr int64_t kMaxY = 65535;  // gridDim.y limit
-  for (int64_t r0 = 0; r0 < n_rows; r0 += kMaxY) {
-    const int64_t ny = std::min<int64_t>(kMaxY, n_rows - r0);
-    src.rows = rec.out + (size_t)(first_row + r0) * k * N;
-    rbisk::stats_kernel<<<dim3((unsigned)nch, (unsigned)ny), chunk, chunk * sizeof(double), ss>>>(
-        src, d_tvec + r0 * 21, d_tquat + r0 * 4, 0, (long long)N, nullptr, d_tables + (size_t)r0 * n_table);
-    CUDA_TRY(cudaGetLastError());
-    h->launches++;
-  }
-  CUDA_TRY(cudaMemcpyAsync(out_chunks, d_tables, (size_t)n_rows * n_table * sizeof(double), cudaMemcpyDeviceToHost, ss));
-  if (out_totals) {
-    rbisk::reduce_chunk_table_kernel<<<(unsigned)n_rows, 128, 0, ss>>>(d_tables, (long long)nch, d_totals);
-    CUDA_TRY(cudaGetLastError());
-    h->launches++;
-    CUDA_TRY(cudaMemcpyAsync(out_totals, d_totals, (size_t)n_rows * RBIS_NUM_STATS * sizeof(double), cudaMemcpyDeviceToHost, ss));
-  }
-  CUDA_TRY(cudaEventRecord(rd->done, ss));
-  rd->pending = true;
-  CUDA_TRY(cudaEventRecord(h->rec_stats_done, ss));
-  h->rec_stats_pending = true;
-  const int t = h->next_ticket;
-  h->next_ticket = (t + 1) % 8;
-  CUDA_TRY(cudaEventRecord(h->tickets[t], ss));
-  *ticket = t;
-  if (n_chunks) *n_chunks = nch;
-  return 0;
+  return row_stats_pass(h, rec.out, rec.out + (size_t)rec.rows * k * N, n_rows, chunk, tbuf, out_chunks, out_totals, n_chunks, ticket,
+                        [&](cudaStream_t ss, const double* d_pre, double* d_tables, int64_t r0, int64_t ny, int64_t nch) {
+                          const double* d_tvec = d_pre;
+                          const double* d_tquat = d_pre + (size_t)n_rows * 21;
+                          src.rows = rec.out + (size_t)(first_row + r0) * k * N;
+                          rbisk::stats_kernel<<<dim3((unsigned)nch, (unsigned)ny), chunk, chunk * sizeof(double), ss>>>(
+                              src, d_tvec + r0 * 21, d_tquat + r0 * 4, 0, (long long)N, nullptr, d_tables);
+                        });
+}
+
+int rbis_batch_stats_innovations_enqueue(rbis_batch_t* h, int32_t stream, int64_t first_row, int64_t n_rows, int chunk,
+                                         double* out_chunks, double* out_totals, int64_t* n_chunks, int32_t* ticket) {
+  if (!h) return fail(RBIS_ERR_INVALID, "null handle");
+  if (!out_chunks || !ticket) return fail(RBIS_ERR_INVALID, "out_chunks and ticket are required");
+  if (chunk < 32 || chunk > 1024 || (chunk & (chunk - 1))) return fail(RBIS_ERR_INVALID, "chunk must be a power of two in [32,1024]");
+  if (stream < 0 || stream >= RBIS_MAX_STREAMS) return fail(RBIS_ERR_INVALID, "stream slot %d outside 0..%d", stream, RBIS_MAX_STREAMS - 1);
+  if (!h->innov_set[stream]) return fail(RBIS_ERR_STATE, "no innovation set on stream slot %d (rbis_batch_set_innovations)", stream);
+  const rbis_innovation_t& iv = h->innov[stream];
+  if (!(iv.fields & RBIS_INNOV_NIS)) return fail(RBIS_ERR_INVALID, "statistics of innovation rows need the RBIS_INNOV_NIS field");
+  if (n_rows < 1 || first_row < 0 || first_row + n_rows > iv.rows)
+    return fail(RBIS_ERR_INVALID, "innovation rows %lld..%lld outside [0, %lld)", (long long)first_row, (long long)(first_row + n_rows), (long long)iv.rows);
+  const size_t N = (size_t)h->N, k = (size_t)h->innov_k[stream];
+  return row_stats_pass(h, iv.out, iv.out + (size_t)iv.rows * k * N, n_rows, chunk, std::vector<double>(), out_chunks, out_totals, n_chunks,
+                        ticket, [&](cudaStream_t ss, const double*, double* d_tables, int64_t r0, int64_t ny, int64_t nch) {
+                          rbisk::innov_stats_kernel<<<dim3((unsigned)nch, (unsigned)ny), chunk, chunk * sizeof(double), ss>>>(
+                              iv.out + (size_t)(first_row + r0) * k * N, (long long)k, iv.m, (int)iv.fields, (long long)N, d_tables);
+                        });
 }
 
 // NCCL is taken from the calling process at run time (dlsym): a host that passes an ncclComm_t has NCCL loaded already, and the

@@ -14,7 +14,8 @@ struct rbis_fused_tu_t {
   // blocks_variant: the program has one-row / correlated chunks (lane-per-filter kernels: instantiation with those paths)
   // decoupled: which kernels of a warp-group unit (it holds both); a lane-per-filter unit holds either kind and ignores it
   // syn: the SYN instantiation (input rows drawn inside the kernel, KParams::syn); decoupled kernels without blocks_variant only
-  // rec: the REC instantiation (the program has RBIS_OP_RECORD ops, KParams::rec)
+  // rec: 1 the REC instantiation (the program has RBIS_OP_RECORD ops, KParams::rec); 2 the REC instantiation with the
+  //      innovation path (INNOV: a MEAS op of the program writes an innovation set, KParams::innov)
   // mask: the MASK instantiation (a stream of the program has RBIS_STREAM_SKIP_NAN_ROWS, KParams::skip_nan_streams); not with syn
   cudaError_t (*launch)(int blocks_variant, int decoupled, int syn, int rec, int mask, unsigned grid, int threads, int smem, cudaStream_t st,
                         const void* kparams);

@@ -329,10 +329,11 @@ __device__ __forceinline__ void g_sweep(double* Pf, const Own<G, Geo<G, DC>::NA>
 
 // Aligned index triple I0..I0+2 (leg-odometry velocity, pose position / orientation, ...): rbis.cpp:124-143 with
 // S = L D L^T, Y = L^-1 P[idx,:], P -= Y^T D^-1 Y, x += Y^T D^-1 L^-1 r.  Same arithmetic as rbisk::meas3.
-template <int G, bool DC, bool SYN, bool MASK = false>
+// NISQ: *nisq += the chunk's quadratic form, as in rbisk::meas3 (the same for g_meas1 / g_meas_block).
+template <int G, bool DC, bool SYN, bool MASK = false, bool NISQ = false>
 __device__ __forceinline__ void g_meas3(double* Pf, const int l, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int I0,
                                         long long row, long long N, long long n, long long sn, const V3& dquat, const V3& chi0,
-                                        bool skip = false) {
+                                        bool skip = false, double* nisq = nullptr) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   double z[3], Rdg[3];
@@ -398,13 +399,14 @@ __device__ __forceinline__ void g_meas3(double* Pf, const int l, FilterState& s,
   });
   if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-logdet - fma(e2, u2, fma(e1, u1, e0 * u0)));
   else s.ll += -logdet - fma(e2, u2, fma(e1, u1, e0 * u0));
+  if constexpr (NISQ) *nisq += fma(e2, u2, fma(e1, u1, e0 * u0));
 }
 
 // One-row chunk on state index idx (rbisk::meas1).
-template <int G, bool DC, bool SYN, bool MASK = false>
+template <int G, bool DC, bool SYN, bool MASK = false, bool NISQ = false>
 __device__ __forceinline__ void g_meas1(double* Pf, const int l, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int idx,
                                         long long row, long long N, long long n, long long sn, const V3& dquat, const V3& chi0,
-                                        bool skip = false) {
+                                        bool skip = false, double* nisq = nullptr) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   const double z = src.z(st, row, a0, sn);
@@ -443,13 +445,15 @@ __device__ __forceinline__ void g_meas1(double* Pf, const int l, FilterState& s,
   });
   if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rr * u);
   else s.ll += -log(sv) - rr * u;
+  if constexpr (NISQ) *nisq += rr * u;
 }
 
 // A chunk of M correlated rows, decorrelated by the host (rbisk::meas_block): M scalar updates with rows
 // H'_a = sum_{b<=a} w_ab H_b and noise D_a.
-template <int G, bool DC, bool SYN, bool MASK = false>
+template <int G, bool DC, bool SYN, bool MASK = false, bool NISQ = false>
 __device__ __forceinline__ void g_meas_block(double* Pf, const int l, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int M,
-                                             long long row, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
+                                             long long row, long long sn, const V3& dquat, const V3& chi0, bool skip = false,
+                                             double* nisq = nullptr) {
   using GE = Geo<G, DC>;
   constexpr int NA = GE::NA, LD = GE::LD, NJ = GE::NJ;
   const double* W = st.R + row * st.r_stride + RS_W;
@@ -506,6 +510,7 @@ __device__ __forceinline__ void g_meas_block(double* Pf, const int l, FilterStat
     });
     if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rp_ * u);
     else s.ll += -log(sv) - rp_ * u;
+    if constexpr (NISQ) *nisq += rp_ * u;
   }
 }
 
@@ -609,6 +614,28 @@ __device__ __forceinline__ void g_record_fields(const KParams& p, const double* 
   }
 }
 
+// Innovation sets: the entries of rbisk::innov_begin with the same values; entry e of the row belongs to lane e modulo G.
+template <int G, bool DC, bool SYN>
+__device__ __forceinline__ void g_innov_begin(const InnovK& iv, const double* Pf, const int l, const FilterState& s, const StreamDesc& st,
+                                              const MeasSrc<SYN>& src, long long row, long long N, long long n, long long sn, const V3& dquat,
+                                              bool active, bool skip) {
+  constexpr int LD = Geo<G, DC>::LD;
+  double* const d = iv.out + row * iv.k * N + n;
+  const int m = st.m;
+  const int oy = iv.fields & INNOV_NIS, os = oy + ((iv.fields & INNOV_Y) ? m : 0);
+  for (int a = 0; a < m; a++) {
+    if ((iv.fields & INNOV_Y) && ((oy + a) & (G - 1)) == l) {
+      const double y = innov_y<SYN>(s, st, src, a, row, sn, dquat);
+      if (active) d[(long long)(oy + a) * N] = skip ? innov_nan() : y;
+    }
+    if ((iv.fields & INNOV_S_DIAG) && ((os + a) & (G - 1)) == l) {
+      const int pi = pos_of<DC>(st.idx[a]);
+      const double v = Pf[pi * LD + pi] + r_diag(st, a, row, N, n);
+      if (active) d[(long long)(os + a) * N] = skip ? innov_nan() : v;
+    }
+  }
+}
+
 // ------------------------------------------------------------------------------------------------
 // The fused kernel, warp-group mapping.  Same parameter block, op program and semantics as rbisk::rbis_fused_kernel;
 // all chunk kinds (aligned triples, one-row chunks, correlated blocks) are compiled in (the indices are run-time
@@ -618,9 +645,11 @@ __device__ __forceinline__ void g_record_fields(const KParams& p, const double* 
 // SYN = true: input rows drawn inside the kernel (KParams::syn), as in rbisk::rbis_fused_kernel.
 // REC = true: programs with RBIS_OP_RECORD ops (KParams::rec), as in rbisk::rbis_fused_kernel.
 // MASK = true: programs with RBIS_STREAM_SKIP_NAN_ROWS streams (KParams::skip_nan_streams), as in rbisk::rbis_fused_kernel.
-template <int G, bool DC, int MAXW, bool SYN = false, bool REC = false, bool MASK = false>
+// INNOV = true (with REC): programs that write innovation sets (KParams::innov), as in rbisk::rbis_fused_kernel.
+template <int G, bool DC, int MAXW, bool SYN = false, bool REC = false, bool MASK = false, bool INNOV = false>
 __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_constant__ KParams p) {
   static_assert(!(MASK && SYN), "MASK instantiations read z from HBM");
+  static_assert(!INNOV || REC, "INNOV instantiations are REC instantiations with the innovation path");
   using GE = Geo<G, DC>;
   constexpr int FPW = GE::FPW, S = GE::S;
   extern __shared__ __align__(16) double smem[];
@@ -752,13 +781,22 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
       }
       V3 dquat{0, 0, 0};
       if (st.has_orient) dquat = subtract_quats(src.quat(st, op.row, sn), {s.qw, s.qx, s.qy, s.qz});  // rbis.cpp:199
+      // INNOV: an innovation set on this stream (uniform branch), as in rbisk::rbis_fused_kernel
+      double nisq = 0.0;
+      if constexpr (INNOV) {
+        if (p.innov[op.stream].out) g_innov_begin<G, DC, SYN>(p.innov[op.stream], Pf, l, s, st, src, op.row, N, n, sn, dquat, active, skip);
+      }
       const V3 chi0{s.x[6], s.x[7], s.x[8]};
       for (int ci = 0; ci < st.n_chunks; ci++) {
         const int a0 = st.chunk_start[ci];
         const int fast = st.chunk_fast[ci];
-        if (fast >= 0 && fast < 100) g_meas3<G, DC, SYN, MASK>(Pf, l, s, st, src, a0, fast, op.row, N, n, sn, dquat, chi0, skip);
-        else if (fast >= 100) g_meas1<G, DC, SYN, MASK>(Pf, l, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0, skip);
-        else g_meas_block<G, DC, SYN, MASK>(Pf, l, s, st, src, a0, st.chunk_len[ci], op.row, sn, dquat, chi0, skip);
+        if (fast >= 0 && fast < 100) g_meas3<G, DC, SYN, MASK, INNOV>(Pf, l, s, st, src, a0, fast, op.row, N, n, sn, dquat, chi0, skip, &nisq);
+        else if (fast >= 100) g_meas1<G, DC, SYN, MASK, INNOV>(Pf, l, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0, skip, &nisq);
+        else g_meas_block<G, DC, SYN, MASK, INNOV>(Pf, l, s, st, src, a0, st.chunk_len[ci], op.row, sn, dquat, chi0, skip, &nisq);
+      }
+      if constexpr (INNOV) {
+        const InnovK& iv = p.innov[op.stream];
+        if (iv.out && (iv.fields & INNOV_NIS) && l == 0 && active) iv.out[op.row * iv.k * N + n] = skip ? innov_nan() : nisq;
       }
       if (!MASK || !skip) meas_finish(s, chi0, p.chi_tol, p.ctor_folds_chi, p.renorm);
     } else if (op.kind == OP_SNAPSHOT) {

@@ -308,6 +308,15 @@ __host__ __device__ __forceinline__ int rec_cov_state(unsigned cb, int c) {
     }
   return -1;
 }
+// Innovation sets (INNOV kernel instantiations, which are REC instantiations too): every MEAS op on stream s with
+// innov[s].out non-null writes row op.row of innov[s].out, [rows][k][N]: NIS = y^T S^-1 y (INNOV_NIS), then y_a = z_a - x-[idx_a] (INNOV_Y), then S(a,a) =
+// P-(idx_a, idx_a) + R(a,a) (INNOV_S_DIAG), all from the prior state of the op; a filter that skips the row writes NaN.
+constexpr int INNOV_NIS = 1, INNOV_Y = 2, INNOV_S_DIAG = 4;
+struct InnovK {
+  double* out;     // nullptr: no innovation set on this stream
+  long long rows;
+  int k, fields;   // k = NIS + m Y + m S_DIAG
+};
 
 struct KParams {
   long long N;
@@ -336,6 +345,8 @@ struct KParams {
   unsigned skip_nan_streams;
   // REC kernel instantiations only (appended for the same reason): covariance blocks of the record set (see RecK)
   unsigned rec_cov_blocks;
+  // INNOV kernel instantiations only (appended for the same reason): innovation sets per stream (see InnovK)
+  InnovK innov[MAX_STREAMS];
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -978,9 +989,12 @@ __host__ __device__ constexpr int carried_pos(int c) { return DC ? act_pos(c) : 
 
 // DC: only the 15 active rows/columns exist (the couplings to omega / a are exactly zero, so are their gains).
 // MASK: skip = the row is missing for this lane's filter, which then keeps covariance, state and log-likelihood (see row_missing).
-template <int I0, bool DC, bool SYN, bool MASK = false>
+// NISQ: *nisq += the chunk's quadratic form r^T S^-1 r (the same for meas1 / meas_block); their sum over the chunks of an
+// update is its NIS (innovation sets, see InnovK).
+template <int I0, bool DC, bool SYN, bool MASK = false, bool NISQ = false>
 __device__ __forceinline__ void meas3(Cov& P, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, long long row, long long N,
-                                      long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
+                                      long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false,
+                                      double* nisq = nullptr) {
   static_assert(!DC || (is_act(I0) && I0 % 3 == 0), "a DC kernel cannot update on omega / a indices");
   constexpr int NC = DC ? N_ACT : NS;        // columns of HP that are carried
   constexpr int NB = NC / 3;                 // index triples
@@ -1109,6 +1123,7 @@ __device__ __forceinline__ void meas3(Cov& P, FilterState& s, const StreamDesc& 
   });
   if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-logdet - fma(e2, u2, fma(e1, u1, e0 * u0)));
   else s.ll += -logdet - fma(e2, u2, fma(e1, u1, e0 * u0));
+  if constexpr (NISQ) *nisq += fma(e2, u2, fma(e1, u1, e0 * u0));
 }
 
 // Row idx (run time, warp uniform) of the covariance over the carried columns: all loads issued, ONE tensor-memory wait.
@@ -1184,9 +1199,10 @@ __device__ __forceinline__ void rank1_sweep(Cov& P, const double (&g)[DC ? N_ACT
 // that is not an aligned triple when its noise is uncorrelated with the other rows).  The index is a run-time, warp-uniform
 // value: the row P[idx, :] is fetched with run-time addressing (15 or 21 loads), everything after that -- the rank-1
 // sweep P -= h h^T / s and the state update -- runs over compile-time slots with h in registers.
-template <bool DC, bool SYN, bool MASK = false>
+template <bool DC, bool SYN, bool MASK = false, bool NISQ = false>
 __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int idx, long long row, long long N,
-                                      long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
+                                      long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false,
+                                      double* nisq = nullptr) {
   constexpr int NC = DC ? N_ACT : NS;
   constexpr auto pos = &carried_pos<DC>;
   const double z = src.z(st, row, a0, sn);
@@ -1215,6 +1231,7 @@ __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& 
   });
   if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rr * u);
   else s.ll += -log(sv) - rr * u;
+  if constexpr (NISQ) *nisq += rr * u;
 }
 
 // meas_block: a chunk of M (2..9) rows with CORRELATED noise on any indices.  The host factors R_block = L D L^T; with
@@ -1223,9 +1240,10 @@ __device__ __forceinline__ void meas1(Cov& P, FilterState& s, const StreamDesc& 
 // Row a of H' combines the covariance rows idx_b, b <= a, so everything lives in registers: g = P H'_a^T (15 / 21
 // doubles), a rank-1 sweep over compile-time slots, the state update.  No local-memory arrays, no separate kernel variant.
 // Only the BLOCKS = true kernel variants contain it.
-template <bool DC, bool SYN, bool MASK = false>
+template <bool DC, bool SYN, bool MASK = false, bool NISQ = false>
 __device__ __forceinline__ void meas_block(Cov& P, FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a0, int M, long long row, long long N,
-                                           long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false) {
+                                           long long n, long long sn, const V3& dquat, const V3& chi0, bool skip = false,
+                                           double* nisq = nullptr) {
   constexpr int NC = DC ? N_ACT : NS;
   const double* W = st.R + row * st.r_stride + RS_W;
   const double* Dg = st.R + row * st.r_stride + RS_D;
@@ -1267,6 +1285,7 @@ __device__ __forceinline__ void meas_block(Cov& P, FilterState& s, const StreamD
     });
     if constexpr (MASK) s.ll = skip ? s.ll : s.ll + (-log(sv) - rp * u);
     else s.ll += -log(sv) - rp * u;
+    if constexpr (NISQ) *nisq += rp * u;
   }
 }
 
@@ -1335,6 +1354,55 @@ __device__ __forceinline__ void store_overwritten_blocks(double* __restrict__ ds
     constexpr int i = row_of_slot(s_), j = col_of_slot(s_);
     dst[(long long)s_ * stride] = (i != j) ? 0.0 : (j < 3 ? q_gyro : q_accel);
   });
+}
+
+// ---- innovation sets (see InnovK) ----
+// P(idx, idx) for a run-time, warp-uniform index: the addressing of fetch_row
+__device__ __forceinline__ double cov_diag(const Cov& P, int idx) {
+  const int s_ = slot(idx, idx);
+  const int k = c_place.idx[s_];
+  const bool tm = c_place.tm[s_];
+  uint32_t lo = 0, hi = 0;
+  double v = 0.0;
+  if (tm) tm_ld2(P.tm + 2 * k, lo, hi);
+  else v = P.Ps[sm_off(k)];
+  tm_wait_ld();
+  const double t = tm_settle(lo, hi);
+  return tm ? t : v;
+}
+__device__ __forceinline__ double innov_nan() { return __longlong_as_double(0x7ff8000000000000ll); }
+// R(a, a) of a stream row: the shared table, the row's table (r_stride) or the per-filter diagonal [m][N]
+__device__ __forceinline__ double r_diag(const StreamDesc& st, int a, long long row, long long N, long long n) {
+  return st.r_mode == 1 ? __ldg(st.R + (long long)a * N + n) : __ldg(st.R + row * st.r_stride + a + (long long)st.m * a);
+}
+// y_a = z_a - x-[idx_a] (the component of dquat at the chi indices of an orientation stream), as the chunks form their
+// residuals before any chunk has run
+template <bool SYN>
+__device__ __forceinline__ double innov_y(const FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src, int a, long long row,
+                                          long long sn, const V3& dquat) {
+  const int i = st.idx[a];
+  if (st.has_orient && i >= 6 && i <= 8) return i == 6 ? dquat.x : i == 7 ? dquat.y : dquat.z;
+  return src.template z<false>(st, row, a, sn) - pick_state(s.x, i);
+}
+// y and S(a,a) of this lane's filter at the start of a MEAS op, one coalesced store each, straight to the output (nothing
+// is held across the chunks); NaN for a filter that skips the row.  m, idx and the fields are warp uniform, so the
+// tensor-memory loads stay warp-aligned.
+template <bool SYN>
+__device__ __forceinline__ void innov_begin(const InnovK& iv, const Cov& P, const FilterState& s, const StreamDesc& st, const MeasSrc<SYN>& src,
+                                            long long row, long long N, long long n, long long sn, const V3& dquat, bool active, bool skip) {
+  double* const d = iv.out + row * iv.k * N + n;
+  const int m = st.m;
+  const int oy = iv.fields & INNOV_NIS, os = oy + ((iv.fields & INNOV_Y) ? m : 0);
+  for (int a = 0; a < m; a++) {
+    if (iv.fields & INNOV_Y) {
+      const double y = innov_y<SYN>(s, st, src, a, row, sn, dquat);
+      if (active) d[(long long)(oy + a) * N] = skip ? innov_nan() : y;
+    }
+    if (iv.fields & INNOV_S_DIAG) {
+      const double v = cov_diag(P, st.idx[a]) + r_diag(st, a, row, N, n);
+      if (active) d[(long long)(os + a) * N] = skip ? innov_nan() : v;
+    }
+  }
 }
 
 // ---- RBIS_OP_RECORD (see RecK) ----
@@ -1443,9 +1511,12 @@ __device__ __forceinline__ void record_fields(const KParams& p, const Cov& P, co
 // REC = true: the program has RBIS_OP_RECORD ops (KParams::rec); launched only then, so that other programs keep their code.
 // MASK = true: some stream of the program has RBIS_STREAM_SKIP_NAN_ROWS (KParams::skip_nan_streams); instantiated with BLOCKS
 // only (and without SYN), launched only for such programs.
-template <bool BLOCKS, bool DC = false, bool SYN = false, bool REC = false, bool MASK = false>
+// INNOV = true (with REC): a MEAS op of the program writes an innovation set (KParams::innov); launched only then, so that
+// programs that only record keep the code of the REC instantiations.
+template <bool BLOCKS, bool DC = false, bool SYN = false, bool REC = false, bool MASK = false, bool INNOV = false>
 __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constant__ KParams p) {
   static_assert(!MASK || (BLOCKS && !SYN), "MASK instantiations have the one-row / correlated-block paths and read z from HBM");
+  static_assert(!INNOV || REC, "INNOV instantiations are REC instantiations with the innovation path");
   extern __shared__ __align__(16) double smem[];
   __shared__ uint32_t tm_base_s;
   const int tid = threadIdx.x;
@@ -1588,28 +1659,37 @@ __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constan
       }
       V3 dquat{0, 0, 0};
       if (st.has_orient) dquat = subtract_quats(src.quat(st, op.row, sn), {s.qw, s.qx, s.qy, s.qz});  // rbis.cpp:199
+      // INNOV: an innovation set on this stream (uniform branch) gets y and S(a,a) now and the NIS after the chunks
+      double nisq = 0.0;
+      if constexpr (INNOV) {
+        if (p.innov[op.stream].out) innov_begin<SYN>(p.innov[op.stream], P, s, st, src, op.row, N, n, sn, dquat, active, skip);
+      }
       const V3 chi0{s.x[6], s.x[7], s.x[8]};
       for (int ci = 0; ci < st.n_chunks; ci++) {
         const int a0 = st.chunk_start[ci];
         const int fast = st.chunk_fast[ci];
         switch (fast) {
-          case 0: if constexpr (!DC) meas3<0, false, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
-          case 3: meas3<3, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
-          case 6: meas3<6, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
-          case 9: meas3<9, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
-          case 12: if constexpr (!DC) meas3<12, false, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
-          case 15: meas3<15, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
-          case 18: meas3<18, DC, SYN, MASK>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip); break;
+          case 0: if constexpr (!DC) meas3<0, false, SYN, MASK, INNOV>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip, &nisq); break;
+          case 3: meas3<3, DC, SYN, MASK, INNOV>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip, &nisq); break;
+          case 6: meas3<6, DC, SYN, MASK, INNOV>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip, &nisq); break;
+          case 9: meas3<9, DC, SYN, MASK, INNOV>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip, &nisq); break;
+          case 12: if constexpr (!DC) meas3<12, false, SYN, MASK, INNOV>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip, &nisq); break;
+          case 15: meas3<15, DC, SYN, MASK, INNOV>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip, &nisq); break;
+          case 18: meas3<18, DC, SYN, MASK, INNOV>(P, s, st, src, a0, op.row, N, n, sn, dquat, chi0, skip, &nisq); break;
           default:
             if constexpr (BLOCKS) {
               if (fast >= 100) {  // one-row chunk on state index fast - 100
-                meas1<DC, SYN, MASK>(P, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0, skip);
+                meas1<DC, SYN, MASK, INNOV>(P, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0, skip, &nisq);
               } else {            // correlated rows: decorrelated scalar updates
-                meas_block<DC, SYN, MASK>(P, s, st, src, a0, st.chunk_len[ci], op.row, N, n, sn, dquat, chi0, skip);
+                meas_block<DC, SYN, MASK, INNOV>(P, s, st, src, a0, st.chunk_len[ci], op.row, N, n, sn, dquat, chi0, skip, &nisq);
               }
             }
             break;
         }
+      }
+      if constexpr (INNOV) {
+        const InnovK& iv = p.innov[op.stream];
+        if (iv.out && (iv.fields & INNOV_NIS) && active) iv.out[op.row * iv.k * N + n] = skip ? innov_nan() : nisq;
       }
       if (!MASK || !skip) meas_finish(s, chi0, p.chi_tol, p.ctor_folds_chi, p.renorm);
     } else if (op.kind == OP_SNAPSHOT) {

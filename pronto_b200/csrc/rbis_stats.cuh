@@ -131,6 +131,65 @@ __global__ void __launch_bounds__(1024) stats_kernel(const Src src, const double
   for (int k = 48 + t; k < NSTAT; k += blockDim.x) out_chunks[(long long)blockIdx.x * NSTAT + k] = 0.0;
 }
 
+// chi2(m) 2.5 % / 97.5 % quantiles for m = 1..9 (scipy.stats.chi2.ppf; m = 9 is the pair of stats_kernel)
+__constant__ double c_chi2_lo[9] = {0.000982069117, 0.050635616, 0.215795283, 0.484418557, 0.831211613,
+                                    1.23734425,     1.68986918,  2.17973075,  2.7003895};
+__constant__ double c_chi2_hi[9] = {5.02388619, 7.37775891, 9.3484036, 11.1432868, 12.832502,
+                                    14.4493753, 16.0127643, 17.5345461, 19.0227678};
+constexpr int NINNOV = 33;  // statistics of an innovation table; the rest of the 96 are zero
+// Ensemble statistics of innovation rows ([rows][k][N], the layout of InnovK with INNOV_NIS at position 0): row blockIdx.y of
+// `rows`, one CTA per chunk of blockDim.x filters, one table [gridDim.x][96] per row.  [0] sum NIS, [1] sum NIS^2, [2] finite
+// NIS, [3] NIS inside the central 95 % of chi2(m), [4] non-finite NIS, [5] filters, [6 + a] sum y_a, [15 + a] sum y_a^2,
+// [24 + a] sum y_a^2 / S(a,a); only filters with a finite NIS enter [0], [1], [3] and [6..32].  The fixed binary tree of
+// stats_kernel, so a numpy restatement reproduces every table bit for bit.
+__global__ void __launch_bounds__(1024) innov_stats_kernel(const double* __restrict__ rows, long long k, int m, int fields, long long N,
+                                                           double* __restrict__ out_chunks) {
+  extern __shared__ double red[];
+  const int t = threadIdx.x;
+  const long long n = (long long)blockIdx.x * blockDim.x + t;
+  rows += (long long)blockIdx.y * k * N;
+  out_chunks += (long long)blockIdx.y * gridDim.x * NSTAT;
+  double val[NINNOV];
+#pragma unroll
+  for (int i = 0; i < NINNOV; i++) val[i] = 0.0;
+  if (n < N) {
+    const double nis = rows[n];
+    if (isfinite(nis)) {
+      val[0] = nis;
+      val[1] = __dmul_rn(nis, nis);
+      val[2] = 1.0;
+      val[3] = (nis >= c_chi2_lo[m - 1] && nis <= c_chi2_hi[m - 1]) ? 1.0 : 0.0;
+      if (fields & INNOV_Y) {
+        const int os = 1 + m;  // S(a,a) follows y
+#pragma unroll
+        for (int a = 0; a < MAX_MEAS; a++) {
+          if (a < m) {
+            const double y = rows[(long long)(1 + a) * N + n];
+            const double y2 = __dmul_rn(y, y);
+            val[6 + a] = y;
+            val[15 + a] = y2;
+            if (fields & INNOV_S_DIAG) val[24 + a] = __ddiv_rn(y2, rows[(long long)(os + a) * N + n]);
+          }
+        }
+      }
+    } else {
+      val[4] = 1.0;
+    }
+    val[5] = 1.0;
+  }
+  static_for<NINNOV>([&](auto i) {
+    red[t] = val[i];
+    __syncthreads();
+    for (int s = blockDim.x >> 1; s > 0; s >>= 1) {
+      if (t < s) red[t] = __dadd_rn(red[t], red[t + s]);
+      __syncthreads();
+    }
+    if (t == 0) out_chunks[(long long)blockIdx.x * NSTAT + i] = red[0];
+    __syncthreads();
+  });
+  for (int i = NINNOV + t; i < NSTAT; i += blockDim.x) out_chunks[(long long)blockIdx.x * NSTAT + i] = 0.0;
+}
+
 // Final reduction of a chunk table on the device: totals[k] = sum over chunks in ASCENDING chunk order (one thread per
 // statistic, a plain sequential sum: the same order as rbis_stats_reduce_chunks on the host).  One CTA per table:
 // table blockIdx.x is [n_chunks][96] at table + blockIdx.x * n_chunks * 96, its totals at totals + blockIdx.x * 96.
