@@ -1,9 +1,10 @@
 #!/usr/bin/env python
 """dev/all_kernels_check.py -- one small pass through every fused-kernel family with a bit-identity check (compute-sanitizer is closed on the GPU pool):
 lane-per-filter decoupled + dense, warp-group 4 / 8 lanes, SYN instantiations, snapshot / restore, snapshot statistics, the
-REC instantiations (RBIS_OP_RECORD), the MASK instantiations (RBIS_STREAM_SKIP_NAN_ROWS, with and without records) and the
-innovation sets (rbis_batch_set_innovations, REC instantiations: in-order, rewound, synthesised and masked programs) over the same
-mappings and variants."""
+REC instantiations (RBIS_OP_RECORD), the MASK instantiations (RBIS_STREAM_SKIP_NAN_ROWS, with and without records), the
+innovation sets (rbis_batch_set_innovations, REC instantiations: in-order, rewound, synthesised and masked programs) and the NIS
+gates (rbis_batch_set_nis_gate, GATE instantiations: alone, with records, with innovation sets) over the same mappings and
+variants."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -172,4 +173,40 @@ for cfg in (dict(mapping=1), dict(mapping=4), dict(mapping=8), dict(mapping=1, s
     same = all(np.array_equal(x, y) for x, y in zip(rows_, ref_innov)) and not any(np.isnan(x).any() for x in rows_)
     print("innovations synth", cfg, "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
     assert same and variant & 8
+# NIS gates over the masked, rewound program: an open gate gives the masked bits; a tight gate (chi2_m(0.9)) gives the same
+# decisions and values in every mapping and variant, alone, with records, and with NIS + APPLIED innovation sets
+ref_gate = None
+for cfg in (dict(mapping=1, lane_filters_per_cta=384), dict(mapping=1, lane_filters_per_cta=128), dict(mapping=1, dense_only=True),
+            dict(mapping=4), dict(mapping=8), dict(mapping=4, dense_only=True)):
+    for extra in ("", "records", "innovations"):
+        out = torch.full((rows, capi.REC_FIELDS, N), float("nan"), dtype=torch.float64, device="cuda")
+        bufs = [torch.full((st["legodo"].shape[0], 2, N), float("nan"), dtype=torch.float64, device="cuda"),
+                torch.full((st["pose_z"].shape[0], 2, N), float("nan"), dtype=torch.float64, device="cuda")]
+        with RBISBatch(N, snapshot_slots=2, **cfg) as b:
+            b.set_process_noise(*nominal_q())
+            b.set_state(sc["vec"], sc["quat"], sc["cov"])
+            for s_ in (0, 1):
+                b.set_nis_gate(s_, float("inf"))
+            b.run_fused(prog, imu=st["imu"], streams=masked(lego, pose_z))
+            open_ = b.get_state()
+            b.set_state(sc["vec"], sc["quat"], sc["cov"])
+            for s_, thr in ((0, 0.5844), (1, 2.2041)):   # chi2_m(0.1): a tight gate that rejects many rows
+                b.set_nis_gate(s_, thr)
+            if extra == "records":
+                b.set_record(out, ALL)
+            if extra == "innovations":
+                for s_, m_ in ((0, 3), (1, 6)):
+                    b.set_innovations(s_, bufs[s_], m_, capi.INNOV_NIS | capi.INNOV_APPLIED)
+            b.run_fused(rec_prog if extra == "records" else prog, imu=st["imu"], streams=masked(lego, pose_z))
+            variant = b.last_kernel_variant
+            got = b.get_state()
+        applied = [x.cpu().numpy()[:, 1] for x in bufs]
+        if ref_gate is None:
+            ref_gate = got
+        same = all(np.array_equal(x, y) for x, y in zip(got[:4], ref_gate[:4])) and all(np.array_equal(x, y) for x, y in zip(open_[:4], ref_mask[:4]))
+        same = same and not np.isnan(got[0]).any() and not all(np.array_equal(x, y) for x, y in zip(got[:4], ref_mask[:4]))
+        if extra == "innovations":
+            same = same and all((a == 0.0).any() and (a == 1.0).any() for a in applied)
+        print("gated", cfg, extra, "variant", variant, "same bits" if same else "DIFFERENT", flush=True)
+        assert same and variant & 2048
 print("ok")

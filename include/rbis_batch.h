@@ -189,7 +189,8 @@ int64_t rbis_batch_launch_count(const rbis_batch_t* h);
  * (rbis_batch_config_t::mapping > 1), +8 for the REC instantiations, which run when the program records (RBIS_OP_RECORD) or a MEAS op
  * of it writes an innovation set (rbis_batch_set_innovations) and never otherwise, +1024 more when they carry the innovation path
  * (the program writes an innovation set: programs that only record do not run that code), +512 when a stream has RBIS_STREAM_SKIP_NAN_ROWS (the MASK instantiations, which contain the one-row and
- * correlated-block updates whatever +1 says); -1 before the first launch. */
+ * correlated-block updates whatever +1 says), +2048 +512 when a stream the program updates on has a NIS gate or an innovation set
+ * it writes has RBIS_INNOV_APPLIED (the GATE instantiations, MASK instantiations with the gate); -1 before the first launch. */
 int rbis_batch_last_kernel_variant(const rbis_batch_t* h);
 
 /* ---- RBISResetUpdate::updateFilter (MSE/rbis_update_interface.cpp:23-28): posterior := given,
@@ -279,10 +280,14 @@ int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec);
  *   NIS    = y^T S^-1 y with the full S: the sum of the quadratic forms of the update's chunks (the kernels apply an update as
  *            chunks of uncorrelated rows, and decorrelated scalar rows inside a correlated block); by the chain rule of the Gaussian
  *            likelihood that equals the single update's y^T S^-1 y up to rounding.  A consistent filter has NIS ~ chi2(m).
- * out is DEVICE memory [rows][k][N], k = NIS + m Y + m S_DIAG: the chosen fields in the order NIS, y_0..y_m-1, S(0,0)..S(m-1,m-1),
- * filter index fastest.  Every MEAS op on stream slot `stream` of a later rbis_batch_run_fused / rbis_batch_run_fused_synth call
+ * out is DEVICE memory [rows][k][N], k = NIS + m Y + m S_DIAG + APPLIED: the chosen fields in the order NIS, y_0..y_m-1,
+ * S(0,0)..S(m-1,m-1), applied, filter index fastest.  Every MEAS op on stream slot `stream` of a later rbis_batch_run_fused / rbis_batch_run_fused_synth call
  * writes row op.row for every active filter:
  *   - a filter that skips the row (RBIS_STREAM_SKIP_NAN_ROWS) writes NaN into all k entries;
+ *   - RBIS_INNOV_APPLIED adds one entry after S(a,a): 1.0 the update was applied, 0.0 the stream's NIS gate rejected it, NaN the
+ *     row was missing.  On a stream with a NIS gate (rbis_batch_set_nis_gate) the NIS entry is the gate's NIS (the full-S form)
+ *     for every filter that received the row, accepted or rejected, and y and S(a,a) are written for rejected filters as usual;
+ *     streams without a gate keep the values above;
  *   - a row applied more than once holds the values of its last application (after a RESTORE and replay, the replayed one);
  *   - rows no MEAS op writes keep their contents; column maps do not apply (the values are per filter).
  * `out` is valid once a ticket recorded after the call has been waited for (rbis_batch_record / rbis_batch_wait) or after
@@ -290,10 +295,11 @@ int rbis_batch_set_record(rbis_batch_t* h, const rbis_record_t* rec);
 #define RBIS_INNOV_NIS    1   /* y^T S^-1 y: 1 entry */
 #define RBIS_INNOV_Y      2   /* the innovation y: m entries */
 #define RBIS_INNOV_S_DIAG 4   /* S(a,a) = P-(idx_a, idx_a) + R(a,a): m entries */
+#define RBIS_INNOV_APPLIED 8  /* 1.0 applied, 0.0 rejected by the NIS gate, NaN missing: 1 entry */
 typedef struct {
-  uint32_t fields;   /* RBIS_INNOV_* bits, not 0 */
+  uint32_t fields;   /* RBIS_INNOV_* bits: at least one of NIS, Y, S_DIAG; APPLIED only beside them */
   int32_t  m;        /* the stream's measurement dimension; a call whose stream `stream` has another m fails */
-  double*  out;      /* DEVICE [rows][k][N], k = NIS + m*Y + m*S_DIAG, in that order, filter index fastest */
+  double*  out;      /* DEVICE [rows][k][N], k = NIS + m*Y + m*S_DIAG + APPLIED, in that order, filter index fastest */
   int64_t  rows;
 } rbis_innovation_t;
 /* Sets the innovation set of stream slot `stream` (0..RBIS_MAX_STREAMS-1) used by the fused calls enqueued after it (handle state
@@ -301,8 +307,37 @@ typedef struct {
  * an unknown or empty `fields`, m outside 1..RBIS_MAX_MEAS and a NULL or non-device `out` are RBIS_ERR_INVALID.  A fused call
  * whose stream `stream` has another m, or whose MEAS op on it names a row outside [0, rows), fails with RBIS_ERR_INVALID before
  * anything is enqueued.  Programs that write an innovation set run the REC kernel instantiations with the innovation path
- * (rbis_batch_last_kernel_variant +8 +1024). */
+ * (rbis_batch_last_kernel_variant +8 +1024); with RBIS_INNOV_APPLIED the GATE instantiations (+512 +2048). */
 int rbis_batch_set_innovations(rbis_batch_t* h, int32_t stream, const rbis_innovation_t* spec);
+
+/* ---- NIS gates: the EKF validation gate.  Each filter rejects a measurement row whose innovation is implausible under its own
+ * S (a foot-slip leg-odometry row, a failed scan-match pose fix), inside the same fused launch.  For every MEAS op on stream
+ * slot `stream` of a later rbis_batch_run_fused / rbis_batch_run_fused_synth call, every filter evaluates, from the op's PRIOR
+ * state (x-, P-) and before any part of the update is applied:
+ *   y   = the innovation of the innovation sets above (z_a - x-[idx_a]; the subtract_quats component at the chi indices of an
+ *         orientation stream)
+ *   S   = P-(I, I) + R, I the stream's index set, R the row's FULL m x m noise: the shared table, the row's table
+ *         (RBIS_R_PER_ROW_FULL) or the diagonal R[a][n] (RBIS_R_PER_FILTER_DIAG)
+ *   NIS = y^T S^-1 y from an unpivoted L D L^T of S in a fixed order (the same bits in every mapping and kernel variant)
+ * and REJECTS the row when !(NIS <= threshold).  A rejected filter behaves exactly like a missing row
+ * (RBIS_STREAM_SKIP_NAN_ROWS): state, quaternion, covariance and log-likelihood keep their bits and no addState runs.  Every
+ * other filter, the ensemble's utime, SNAPSHOT, RESTORE and RECORD proceed as usual.
+ *   - A NaN NIS is rejected.  So on a gated stream a NaN z is rejected even without RBIS_STREAM_SKIP_NAN_ROWS, instead of
+ *     poisoning the filter.  With RBIS_STREAM_SKIP_NAN_ROWS "missing" is decided first, and a missing row is not gated.
+ *   - After a RESTORE a replayed row is gated again against its replayed prior, as the reference calls updateFilter again.
+ *   - The single-update entry points, and calls with fewer than stream + 1 streams, ignore the gate.
+ *   - Programs that update on a gated stream run the GATE kernel instantiations (rbis_batch_last_kernel_variant +512 +2048); a
+ *     gated synthesised call generates its rows into device memory first (no in-kernel drawing).
+ * An innovation set with RBIS_INNOV_APPLIED reports each filter's decision. */
+typedef struct {
+  double nis_max;                    /* reject when !(NIS <= nis_max); > 0, +inf allowed */
+  const double* nis_max_per_filter;  /* DEVICE [N] or NULL; when set it replaces nis_max for filter n (column maps do not apply) */
+} rbis_nis_gate_t;
+/* Sets the NIS gate of stream slot `stream` (0..RBIS_MAX_STREAMS-1) used by the fused calls enqueued after it (handle state per
+ * slot, like the innovation sets; a copy of *gate is kept, the per-filter array is read by the kernels and must stay valid while
+ * they run); NULL clears it.  Does not synchronise.  A bad slot, nis_max NaN or <= 0 without a per-filter array, and a
+ * per-filter array that is not memory of the handle's device are RBIS_ERR_INVALID, refused before anything is enqueued. */
+int rbis_batch_set_nis_gate(rbis_batch_t* h, int32_t stream, const rbis_nis_gate_t* gate);
 
 /* ---- the fused hot path: run `n_ops` ops (host array, executed in order) for every filter in ONE
  * kernel launch, state and covariance resident on chip throughout.  This is the batch form of the
@@ -483,6 +518,7 @@ int rbis_batch_stats_records_enqueue(rbis_batch_t* h, int64_t first_row, int64_t
  *   [0] sum NIS   [1] sum NIS^2   [2] filters with a finite NIS   [3] of them, NIS inside the central 95 % of chi2(m)
  *   [4] filters with a non-finite NIS (skipped rows, poisoned filters)   [5] filters
  *   [6 + a] sum y_a, [15 + a] sum y_a^2 (with RBIS_INNOV_Y)   [24 + a] sum y_a^2 / S(a,a) (with RBIS_INNOV_Y and RBIS_INNOV_S_DIAG)
+ *   [33] filters whose update the NIS gate rejected, APPLIED == 0 (with RBIS_INNOV_APPLIED)
  * Only filters with a finite NIS enter [0], [1], [3] and [6..32].  Each chunk is reduced with the fixed binary tree of the other
  * statistics, so tables of chunk-aligned shards concatenate and reduce with rbis_stats_reduce_chunks.  ANIS = [0] / [2]; for a
  * consistent filter ANIS is near m and [15 + a] / [2] near the mean S(a,a), i.e. [24 + a] / [2] near 1 for every axis a. */

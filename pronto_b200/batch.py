@@ -185,18 +185,22 @@ def record_layout(mask, cov_blocks=()):
 
 
 def innovation_layout(m, fields):
-    """Names of the entries of an innovation row in output order: 'nis', then 'y<a>' and 's<a>' (S(a,a)) for a < m, as the
-    RBIS_INNOV_* bits of `fields` select them."""
+    """Names of the entries of an innovation row in output order: 'nis', then 'y<a>' and 's<a>' (S(a,a)) for a < m, then
+    'applied', as the RBIS_INNOV_* bits of `fields` select them (INNOV_APPLIED only beside one of the others)."""
     m, fields = int(m), int(fields)
     if not 1 <= m <= capi.MAX_MEAS:
         raise ValueError(f"innovation m = {m} outside 1..{capi.MAX_MEAS}")
-    if fields <= 0 or fields & ~(capi.INNOV_NIS | capi.INNOV_Y | capi.INNOV_S_DIAG):
-        raise ValueError(f"innovation fields {fields:#x}: need a non-empty set of INNOV_NIS / INNOV_Y / INNOV_S_DIAG")
+    values = capi.INNOV_NIS | capi.INNOV_Y | capi.INNOV_S_DIAG
+    if fields <= 0 or not fields & values or fields & ~(values | capi.INNOV_APPLIED):
+        raise ValueError(f"innovation fields {fields:#x}: need a non-empty set of INNOV_NIS / INNOV_Y / INNOV_S_DIAG, optionally "
+                         "with INNOV_APPLIED")
     names = ["nis"] if fields & capi.INNOV_NIS else []
     if fields & capi.INNOV_Y:
         names += [f"y{a}" for a in range(m)]
     if fields & capi.INNOV_S_DIAG:
         names += [f"s{a}" for a in range(m)]
+    if fields & capi.INNOV_APPLIED:
+        names.append("applied")
     return names
 
 
@@ -474,6 +478,28 @@ class RBISBatch:
     def clear_innovations(self, stream):
         capi.check(self.lib.rbis_batch_set_innovations(self.h, int(stream), None))
 
+    # ---- NIS gates ----
+    def set_nis_gate(self, stream, nis_max=float("inf"), per_filter=None):
+        """NIS gate of stream slot `stream` (rbis_batch_set_nis_gate): in later fused calls every filter rejects a row of that
+        stream whose prior NIS exceeds its threshold, and then keeps its values as for a missing row.  per_filter: a CUDA float64
+        tensor [N] of thresholds (filter n uses per_filter[n]) or None for nis_max everywhere.  Does not synchronise."""
+        gate = capi.NisGate()
+        gate.nis_max = float(nis_max)
+        gate.nis_max_per_filter = None
+        if per_filter is not None:
+            if tuple(per_filter.shape) != (self.N,):
+                raise ValueError(f"per-filter NIS thresholds must be [{self.N}], got {tuple(per_filter.shape)}")
+            gate.nis_max_per_filter, _ = _ptr(per_filter, None, "per_filter")
+        capi.check(self.lib.rbis_batch_set_nis_gate(self.h, int(stream), C.byref(gate)))
+        # the previous array may still be read by enqueued calls: held until the next synchronize()
+        self._pending_keep = getattr(self, "_pending_keep", [])
+        self._gate_thr = getattr(self, "_gate_thr", {})
+        self._pending_keep.append(self._gate_thr.get(int(stream)))
+        self._gate_thr[int(stream)] = per_filter
+
+    def clear_nis_gate(self, stream):
+        capi.check(self.lib.rbis_batch_set_nis_gate(self.h, int(stream), None))
+
     def stats_innovations_enqueue(self, stream, first_row, out_chunks, out_totals=None, chunk=1024):
         """Statistics of innovation rows first_row .. first_row + n_rows - 1 of stream slot `stream`'s innovation set on the
         statistics side stream (rbis_batch_stats_innovations_enqueue): out_chunks a PINNED host array [n_rows][n_chunks][96] (n_rows
@@ -561,7 +587,7 @@ class RBISBatch:
     def last_kernel_variant(self):
         """0 dense, 2 decoupled (rbis_batch_config_t::dense_only), +1 with correlated-row chunks, +4 input rows drawn in the
         kernel, +8 a program with RBIS_OP_RECORD ops, +16 * lanes per filter for the warp-group kernels, +512 a stream that skips
-        NaN rows (MeasStream skip_nan_rows); -1 before any launch."""
+        NaN rows (MeasStream skip_nan_rows), +2048 (with +512) a NIS gate or INNOV_APPLIED (set_nis_gate); -1 before any launch."""
         return int(self.lib.rbis_batch_last_kernel_variant(self.h))
 
     @property

@@ -21,6 +21,7 @@ OP_IMU, OP_MEAS, OP_SNAPSHOT, OP_RESTORE, OP_RECORD = 0, 1, 2, 3, 4
 REC_FIELDS = 47  # record fields: 0..20 vec, 21..24 quat w,x,y,z, 25 loglik, 26..46 covariance diagonal
 REC_BLOCKS = 7   # record covariance blocks: state indices 3b..3b+2 (omega, v, chi, p, a, gyro bias, accel bias)
 INNOV_NIS, INNOV_Y, INNOV_S_DIAG = 1, 2, 4  # rbis_innovation_t::fields: NIS (1 entry), y (m entries), S(a,a) (m entries)
+INNOV_APPLIED = 8  # one entry after S(a,a): 1.0 applied, 0.0 rejected by the stream's NIS gate, NaN missing
 R_SHARED_FULL, R_PER_FILTER_DIAG, R_PER_ROW_FULL = 0, 1, 2
 STREAM_SKIP_NAN_ROWS = 1  # rbis_stream_t::flags: a filter whose row holds a NaN in a value the update reads skips that update
 
@@ -132,6 +133,13 @@ class Innovation(C.Structure):
     ]
 
 
+class NisGate(C.Structure):
+    _fields_ = [
+        ("nis_max", C.c_double),
+        ("nis_max_per_filter", C.c_void_p),
+    ]
+
+
 class Op(C.Structure):
     _fields_ = [
         ("kind", C.c_int32),
@@ -170,6 +178,7 @@ PROTOTYPES = {
     "rbis_batch_set_column_map": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_int64]),
     "rbis_batch_set_record": (C.c_int, [C.c_void_p, C.POINTER(Record)]),
     "rbis_batch_set_innovations": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(Innovation)]),
+    "rbis_batch_set_nis_gate": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(NisGate)]),
     "rbis_batch_run_fused": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Op), C.c_void_p, C.c_int64, C.c_int, C.POINTER(Stream), C.c_int]),
     "rbis_batch_synthesize": (C.c_int, [C.c_void_p, C.POINTER(Synth), C.c_void_p, C.c_void_p, C.c_void_p]),
     "rbis_batch_run_fused_synth": (C.c_int, [C.c_void_p, C.c_int64, C.POINTER(Op), C.c_int, C.POINTER(Stream), C.POINTER(Synth)]),

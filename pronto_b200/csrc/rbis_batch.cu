@@ -194,7 +194,10 @@ struct rbis_batch {
   // ---- innovation sets (rbis_batch_set_innovations), per stream slot: MEAS ops on the stream write rows of innov[s].out
   bool innov_set[RBIS_MAX_STREAMS] = {};
   rbis_innovation_t innov[RBIS_MAX_STREAMS] = {};
-  int innov_k[RBIS_MAX_STREAMS] = {};       // doubles per filter and row: NIS + m y + m S_DIAG
+  int innov_k[RBIS_MAX_STREAMS] = {};       // doubles per filter and row: NIS + m y + m S_DIAG + APPLIED
+  // ---- NIS gates (rbis_batch_set_nis_gate), per stream slot: MEAS ops on the stream reject rows whose prior NIS exceeds the gate
+  bool gate_set[RBIS_MAX_STREAMS] = {};
+  rbis_nis_gate_t gate[RBIS_MAX_STREAMS] = {};
 };
 
 namespace {
@@ -205,7 +208,8 @@ constexpr int kRShared = rbisk::RS_STRIDE;
 
 static_assert(rbisk::OP_IMU == RBIS_OP_IMU && rbisk::OP_MEAS == RBIS_OP_MEAS && rbisk::OP_SNAPSHOT == RBIS_OP_SNAPSHOT &&
               rbisk::OP_RECORD == RBIS_OP_RECORD, "op kinds of the kernels and of the C ABI differ");
-static_assert(rbisk::INNOV_NIS == RBIS_INNOV_NIS && rbisk::INNOV_Y == RBIS_INNOV_Y && rbisk::INNOV_S_DIAG == RBIS_INNOV_S_DIAG,
+static_assert(rbisk::INNOV_NIS == RBIS_INNOV_NIS && rbisk::INNOV_Y == RBIS_INNOV_Y && rbisk::INNOV_S_DIAG == RBIS_INNOV_S_DIAG &&
+                  rbisk::INNOV_APPLIED == RBIS_INNOV_APPLIED,
               "innovation fields of the kernels and of the C ABI differ");
 
 constexpr int kMaxSmemOptin = 232448;
@@ -260,11 +264,13 @@ LaunchGeom launch_geom(int variant, int mapping, int lane_tpb, long long N, int 
 }
 
 // variant bit 3: the program records or writes innovation sets (REC instantiations); bit 9 (+512): a stream skips NaN rows (MASK
-// instantiations); bit 10 (+1024): the REC instantiations with the innovation path (INNOV)
-constexpr int kVariantMask = 512, kVariantInnov = 1024;
+// instantiations); bit 10 (+1024): the REC instantiations with the innovation path (INNOV); bit 11 (+2048, always with +512):
+// the MASK instantiations with the NIS gates (GATE)
+constexpr int kVariantMask = 512, kVariantInnov = 1024, kVariantGate = 2048;
 cudaError_t launch_variant(int variant, int syn, const LaunchGeom& g, unsigned blocks, cudaStream_t st, const rbisk::KParams& kp) {
   const int rec = (variant & kVariantInnov) ? 2 : (variant & 8) ? 1 : 0;
-  return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, rec, (variant & kVariantMask) ? 1 : 0, blocks, g.threads, g.smem, st, &kp);
+  const int mask = (variant & kVariantGate) ? 2 : (variant & kVariantMask) ? 1 : 0;
+  return g.tu->launch(variant & 1, (variant & 2) ? 1 : 0, syn, rec, mask, blocks, g.threads, g.smem, st, &kp);
 }
 
 // Automatic choice of the mapping (rbis_batch_config_t::mapping == 0) from the ensemble size: cycles per filter step of one
@@ -576,7 +582,7 @@ int row_stats_pass(rbis_batch* h, const double* lo, const double* hi, int64_t n_
 
 // syn != nullptr: the input rows are synthesised on the device into the staging slot (rbis_batch_run_fused_synth) instead of
 // being copied from the host; everything else -- double buffering, overlap with the previous launch -- is the host path's.
-// use_innov = false: the single-update entry points, which ignore innovation sets
+// use_innov = false: the single-update entry points, which ignore innovation sets and NIS gates
 int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const double* imu, int64_t imu_rows,
                  int n_streams, const rbis_stream_t* streams_in, int mem, bool use_maps = true,
                  const rbis_synth_t* syn = nullptr, bool use_innov = true) {
@@ -620,6 +626,7 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
   bool any_record = false;
   std::vector<int64_t> rec_rows;  // record rows of the call, in op order
   bool innov_used[RBIS_MAX_STREAMS] = {};  // streams whose innovation set a MEAS op of the call writes
+  bool meas_on[RBIS_MAX_STREAMS] = {};     // streams a MEAS op of the call updates on
   int64_t last_utime = h->utime;
   for (int64_t i = 0; i < n_ops; i++) {
     const rbis_op_t& o = ops[i];
@@ -641,6 +648,7 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
                         (long long)o.row, o.stream, (long long)h->innov[o.stream].rows);
           innov_used[o.stream] = true;
         }
+        meas_on[o.stream] = true;
         last_utime = o.utime;
         break;
       case RBIS_OP_SNAPSHOT:
@@ -735,9 +743,21 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
         }
     }
   }
+  // NIS gates of the streams the program updates on; an innovation set that asks for INNOV_APPLIED needs the GATE
+  // instantiations too (gated or not, they are the ones that write the entry)
+  bool gate_kernels = false;
+  for (int s = 0; s < n_streams; s++) {
+    if (use_innov && h->gate_set[s] && meas_on[s]) {
+      kp.gate_streams |= 1u << s;
+      kp.gate_nis[s] = h->gate[s].nis_max;
+      kp.gate_nis_filter[s] = h->gate[s].nis_max_per_filter;
+      gate_kernels = true;
+    }
+    if (innov_used[s] && (h->innov[s].fields & RBIS_INNOV_APPLIED)) gate_kernels = true;
+  }
   // ---- kernel variant ----
-  // skipping a row changes no coupling, so decoupled eligibility does not depend on the MASK instantiations
-  int variant = (needs_general ? 1 : 0) | (kp.skip_nan_streams ? kVariantMask : 0);
+  // skipping or rejecting a row changes no coupling, so decoupled eligibility does not depend on the MASK / GATE instantiations
+  int variant = (needs_general ? 1 : 0) | (kp.skip_nan_streams ? kVariantMask : 0) | (gate_kernels ? kVariantMask | kVariantGate : 0);
   const bool dc_eligible = !h->cfg.dense_only && !passive_index && restores_ok;
   if (dc_eligible && h->decoupled < 0) {
     // one device pass over the couplings, then a host read: happens once after set_state / set_filter, not per launch
@@ -753,9 +773,10 @@ int launch_fused(rbis_batch* h, int64_t n_ops, const rbis_op_t* ops, const doubl
   }
   if (dc_eligible && h->decoupled == 1) variant |= 2;
   // Synthesised inputs: the decoupled kernels have SYN instantiations that draw the rows themselves (mode 1), so nothing is
-  // materialised and the launch reads no per-filter input; otherwise the rows are generated into the staging slot first.
+  // materialised and the launch reads no per-filter input; otherwise the rows are generated into the staging slot first.  The
+  // GATE instantiations read their rows from HBM: a gated program materialises them.
   const bool fuse_syn = syn != nullptr && syn->mode == 1 && !h->cfg.synth_materialize && (variant & 2) != 0 &&
-                        (h->mapping > 1 || !(variant & 1));
+                        (h->mapping > 1 || !(variant & 1)) && !gate_kernels;
   if (syn) {
     if (kp.imu_map) return fail(RBIS_ERR_STATE, "synthesised inputs draw one column per filter: clear the column maps first");
     for (int s = 0; s < n_streams; s++)
@@ -1489,8 +1510,10 @@ int rbis_batch_set_innovations(rbis_batch_t* h, int32_t stream, const rbis_innov
     h->innov_set[stream] = false;
     return 0;
   }
-  constexpr uint32_t all = RBIS_INNOV_NIS | RBIS_INNOV_Y | RBIS_INNOV_S_DIAG;
-  if (spec->fields == 0 || (spec->fields & ~all)) return fail(RBIS_ERR_INVALID, "innovation fields 0x%x: a non-empty set of RBIS_INNOV_* bits", spec->fields);
+  constexpr uint32_t values = RBIS_INNOV_NIS | RBIS_INNOV_Y | RBIS_INNOV_S_DIAG;
+  if (!(spec->fields & values) || (spec->fields & ~(values | RBIS_INNOV_APPLIED)))
+    return fail(RBIS_ERR_INVALID, "innovation fields 0x%x: a non-empty set of RBIS_INNOV_NIS / _Y / _S_DIAG, optionally with RBIS_INNOV_APPLIED",
+                spec->fields);
   if (spec->m < 1 || spec->m > RBIS_MAX_MEAS) return fail(RBIS_ERR_INVALID, "innovation m = %d outside 1..%d", spec->m, RBIS_MAX_MEAS);
   if (!spec->out) return fail(RBIS_ERR_INVALID, "innovation output is NULL");
   if (spec->rows <= 0) return fail(RBIS_ERR_INVALID, "innovation rows must be positive");
@@ -1505,8 +1528,33 @@ int rbis_batch_set_innovations(rbis_batch_t* h, int32_t stream, const rbis_innov
     return fail(RBIS_ERR_INVALID, "innovation output is not memory of device %d", h->cfg.device);
   h->innov[stream] = *spec;
   h->innov_k[stream] = ((spec->fields & RBIS_INNOV_NIS) ? 1 : 0) + ((spec->fields & RBIS_INNOV_Y) ? spec->m : 0) +
-                       ((spec->fields & RBIS_INNOV_S_DIAG) ? spec->m : 0);
+                       ((spec->fields & RBIS_INNOV_S_DIAG) ? spec->m : 0) + ((spec->fields & RBIS_INNOV_APPLIED) ? 1 : 0);
   h->innov_set[stream] = true;
+  return 0;
+}
+
+int rbis_batch_set_nis_gate(rbis_batch_t* h, int32_t stream, const rbis_nis_gate_t* gate) {
+  if (!h) return fail(RBIS_ERR_INVALID, "null handle");
+  if (stream < 0 || stream >= RBIS_MAX_STREAMS) return fail(RBIS_ERR_INVALID, "stream slot %d outside 0..%d", stream, RBIS_MAX_STREAMS - 1);
+  if (!gate) {
+    h->gate_set[stream] = false;
+    return 0;
+  }
+  if (!gate->nis_max_per_filter) {
+    if (!(gate->nis_max > 0)) return fail(RBIS_ERR_INVALID, "NIS gate threshold %g: must be > 0 (+inf allowed)", gate->nis_max);
+  } else {
+    if (int rc = use_device(h)) return rc;
+    cudaPointerAttributes a;
+    cudaError_t e = cudaPointerGetAttributes(&a, gate->nis_max_per_filter);
+    if (e != cudaSuccess) {
+      cudaGetLastError();
+      return fail(RBIS_ERR_INVALID, "per-filter NIS thresholds: cudaPointerGetAttributes failed: %s", cudaGetErrorString(e));
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != h->cfg.device)
+      return fail(RBIS_ERR_INVALID, "per-filter NIS thresholds are not memory of device %d", h->cfg.device);
+  }
+  h->gate[stream] = *gate;
+  h->gate_set[stream] = true;
   return 0;
 }
 

@@ -16,7 +16,9 @@ struct rbis_fused_tu_t {
   // syn: the SYN instantiation (input rows drawn inside the kernel, KParams::syn); decoupled kernels without blocks_variant only
   // rec: 1 the REC instantiation (the program has RBIS_OP_RECORD ops, KParams::rec); 2 the REC instantiation with the
   //      innovation path (INNOV: a MEAS op of the program writes an innovation set, KParams::innov)
-  // mask: the MASK instantiation (a stream of the program has RBIS_STREAM_SKIP_NAN_ROWS, KParams::skip_nan_streams); not with syn
+  // mask: 1 the MASK instantiation (a stream of the program has RBIS_STREAM_SKIP_NAN_ROWS, KParams::skip_nan_streams); 2 the MASK
+  //       instantiation with the NIS gates (GATE: a stream has a gate or an innovation set asks for INNOV_APPLIED,
+  //       KParams::gate_streams); not with syn
   cudaError_t (*launch)(int blocks_variant, int decoupled, int syn, int rec, int mask, unsigned grid, int threads, int smem, cudaStream_t st,
                         const void* kparams);
 };

@@ -646,10 +646,12 @@ __device__ __forceinline__ void g_innov_begin(const InnovK& iv, const double* Pf
 // REC = true: programs with RBIS_OP_RECORD ops (KParams::rec), as in rbisk::rbis_fused_kernel.
 // MASK = true: programs with RBIS_STREAM_SKIP_NAN_ROWS streams (KParams::skip_nan_streams), as in rbisk::rbis_fused_kernel.
 // INNOV = true (with REC): programs that write innovation sets (KParams::innov), as in rbisk::rbis_fused_kernel.
-template <int G, bool DC, int MAXW, bool SYN = false, bool REC = false, bool MASK = false, bool INNOV = false>
+// GATE = true (with MASK): programs with NIS gates or INNOV_APPLIED (KParams::gate_streams), as in rbisk::rbis_fused_kernel.
+template <int G, bool DC, int MAXW, bool SYN = false, bool REC = false, bool MASK = false, bool INNOV = false, bool GATE = false>
 __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_constant__ KParams p) {
   static_assert(!(MASK && SYN), "MASK instantiations read z from HBM");
   static_assert(!INNOV || REC, "INNOV instantiations are REC instantiations with the innovation path");
+  static_assert(!GATE || MASK, "GATE instantiations are MASK instantiations with the gate");
   using GE = Geo<G, DC>;
   constexpr int FPW = GE::FPW, S = GE::S;
   extern __shared__ __align__(16) double smem[];
@@ -781,10 +783,24 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
       }
       V3 dquat{0, 0, 0};
       if (st.has_orient) dquat = subtract_quats(src.quat(st, op.row, sn), {s.qw, s.qx, s.qy, s.qz});  // rbis.cpp:199
+      // GATE: as in rbisk::rbis_fused_kernel; the G lanes of a group compute the same NIS from the same Pf entries and inputs,
+      // so they take the same decision
+      const bool missing = skip;
+      double gnis = 0.0;
+      if constexpr (GATE) {
+        if ((p.gate_streams >> op.stream) & 1u) {
+          constexpr int LD = GE::LD;
+          gnis = gate_nis<SYN>(st, src, s, op.row, N, n, sn, dquat, [&](int a, int b) {
+            const int i = min(st.idx[a], st.idx[b]), j = max(st.idx[a], st.idx[b]);  // the upper triangle, as g_record_fields reads it
+            return Pf[pos_of<DC>(i) * LD + pos_of<DC>(j)];
+          });
+          skip = missing || gate_rejects(p, op.stream, n, gnis);
+        }
+      }
       // INNOV: an innovation set on this stream (uniform branch), as in rbisk::rbis_fused_kernel
       double nisq = 0.0;
       if constexpr (INNOV) {
-        if (p.innov[op.stream].out) g_innov_begin<G, DC, SYN>(p.innov[op.stream], Pf, l, s, st, src, op.row, N, n, sn, dquat, active, skip);
+        if (p.innov[op.stream].out) g_innov_begin<G, DC, SYN>(p.innov[op.stream], Pf, l, s, st, src, op.row, N, n, sn, dquat, active, missing);
       }
       const V3 chi0{s.x[6], s.x[7], s.x[8]};
       for (int ci = 0; ci < st.n_chunks; ci++) {
@@ -794,7 +810,9 @@ __global__ void __launch_bounds__(32 * MAXW, 1) rbis_group_kernel(const __grid_c
         else if (fast >= 100) g_meas1<G, DC, SYN, MASK, INNOV>(Pf, l, s, st, src, a0, fast - 100, op.row, N, n, sn, dquat, chi0, skip, &nisq);
         else g_meas_block<G, DC, SYN, MASK, INNOV>(Pf, l, s, st, src, a0, st.chunk_len[ci], op.row, sn, dquat, chi0, skip, &nisq);
       }
-      if constexpr (INNOV) {
+      if constexpr (INNOV && GATE) {
+        innov_end(p, op, N, n, writer, missing, skip, gnis, nisq);
+      } else if constexpr (INNOV) {
         const InnovK& iv = p.innov[op.stream];
         if (iv.out && (iv.fields & INNOV_NIS) && l == 0 && active) iv.out[op.row * iv.k * N + n] = skip ? innov_nan() : nisq;
       }

@@ -311,11 +311,13 @@ __host__ __device__ __forceinline__ int rec_cov_state(unsigned cb, int c) {
 // Innovation sets (INNOV kernel instantiations, which are REC instantiations too): every MEAS op on stream s with
 // innov[s].out non-null writes row op.row of innov[s].out, [rows][k][N]: NIS = y^T S^-1 y (INNOV_NIS), then y_a = z_a - x-[idx_a] (INNOV_Y), then S(a,a) =
 // P-(idx_a, idx_a) + R(a,a) (INNOV_S_DIAG), all from the prior state of the op; a filter that skips the row writes NaN.
-constexpr int INNOV_NIS = 1, INNOV_Y = 2, INNOV_S_DIAG = 4;
+// INNOV_APPLIED (GATE instantiations only): one entry after S(a,a), 1.0 applied, 0.0 rejected by the stream's NIS gate, NaN
+// missing (see gate_nis).
+constexpr int INNOV_NIS = 1, INNOV_Y = 2, INNOV_S_DIAG = 4, INNOV_APPLIED = 8;
 struct InnovK {
   double* out;     // nullptr: no innovation set on this stream
   long long rows;
-  int k, fields;   // k = NIS + m Y + m S_DIAG
+  int k, fields;   // k = NIS + m Y + m S_DIAG + APPLIED
 };
 
 struct KParams {
@@ -347,6 +349,11 @@ struct KParams {
   unsigned rec_cov_blocks;
   // INNOV kernel instantiations only (appended for the same reason): innovation sets per stream (see InnovK)
   InnovK innov[MAX_STREAMS];
+  // GATE kernel instantiations only (appended for the same reason): bit s set = stream s has a NIS gate; a filter rejects the
+  // row when !(NIS <= threshold), threshold gate_nis_filter[s][n] when that pointer is set, gate_nis[s] otherwise (see gate_nis)
+  unsigned gate_streams;
+  double gate_nis[MAX_STREAMS];
+  const double* gate_nis_filter[MAX_STREAMS];
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -1357,9 +1364,9 @@ __device__ __forceinline__ void store_overwritten_blocks(double* __restrict__ ds
 }
 
 // ---- innovation sets (see InnovK) ----
-// P(idx, idx) for a run-time, warp-uniform index: the addressing of fetch_row
-__device__ __forceinline__ double cov_diag(const Cov& P, int idx) {
-  const int s_ = slot(idx, idx);
+// P(i, j) for run-time, warp-uniform indices: the addressing of fetch_row
+__device__ __forceinline__ double cov_at(const Cov& P, int i, int j) {
+  const int s_ = slot(i, j);
   const int k = c_place.idx[s_];
   const bool tm = c_place.tm[s_];
   uint32_t lo = 0, hi = 0;
@@ -1370,6 +1377,7 @@ __device__ __forceinline__ double cov_diag(const Cov& P, int idx) {
   const double t = tm_settle(lo, hi);
   return tm ? t : v;
 }
+__device__ __forceinline__ double cov_diag(const Cov& P, int idx) { return cov_at(P, idx, idx); }
 __device__ __forceinline__ double innov_nan() { return __longlong_as_double(0x7ff8000000000000ll); }
 // R(a, a) of a stream row: the shared table, the row's table (r_stride) or the per-filter diagonal [m][N]
 __device__ __forceinline__ double r_diag(const StreamDesc& st, int a, long long row, long long N, long long n) {
@@ -1403,6 +1411,70 @@ __device__ __forceinline__ void innov_begin(const InnovK& iv, const Cov& P, cons
       if (active) d[(long long)(os + a) * N] = skip ? innov_nan() : v;
     }
   }
+}
+
+// ---- NIS gates (GATE kernel instantiations, KParams::gate_streams) ----
+// The gate's NIS of a MEAS op from its prior state: y as innov_y forms it, S = P-(I, I) + R with R the row's FULL m x m noise
+// (the shared table, the row's table, or the per-filter diagonal), NIS = y^T S^-1 y from an unpivoted L D L^T of S, row by row,
+// with every multiply-add explicit -- the full-S form, not the chunks' chain-rule sum.  pij(a, b), a <= b, returns
+// P-(idx_a, idx_b); the lane kernels read it from shared / tensor memory, the warp-group kernels from Pf, and both families
+// call this one function, so the NIS and the decision are bit-identical across mappings and dense / decoupled kernels.  S (up
+// to 45 doubles) lives in a small local array and the loops are not unrolled: nothing of it is live across the sweeps.
+template <bool SYN, class PIJ>
+__device__ __forceinline__ double gate_nis(const StreamDesc& st, const MeasSrc<SYN>& src, const FilterState& s, long long row, long long N,
+                                           long long n, long long sn, const V3& dquat, PIJ&& pij) {
+  const int m = st.m;
+  double A[MAX_MEAS * (MAX_MEAS + 1) / 2];  // lower triangle row by row: S(a, b), b <= a, overwritten by L below the diagonal
+  double d[MAX_MEAS], w[MAX_MEAS];          // D; y, overwritten by L^-1 y
+  const double* Rt = st.R + row * st.r_stride;
+#pragma unroll 1
+  for (int a = 0; a < m; a++) {
+    w[a] = innov_y<SYN>(s, st, src, a, row, sn, dquat);
+#pragma unroll 1
+    for (int b = 0; b <= a; b++) {
+      const double r = st.r_mode == 1 ? (a == b ? __ldg(st.R + (long long)a * N + n) : 0.0) : __ldg(Rt + a + (long long)m * b);
+      A[a * (a + 1) / 2 + b] = pij(b, a) + r;
+    }
+  }
+  double nis = 0.0;
+#pragma unroll 1
+  for (int i = 0; i < m; i++) {
+    double* const Li = A + i * (i + 1) / 2;
+#pragma unroll 1
+    for (int j = 0; j < i; j++) {
+      const double* const Lj = A + j * (j + 1) / 2;
+      double t = Li[j];
+#pragma unroll 1
+      for (int k = 0; k < j; k++) t = fma(-(Li[k] * d[k]), Lj[k], t);
+      Li[j] = t / d[j];
+    }
+    double t = Li[i], v = w[i];
+#pragma unroll 1
+    for (int k = 0; k < i; k++) {
+      t = fma(-(Li[k] * d[k]), Li[k], t);
+      v = fma(-Li[k], w[k], v);
+    }
+    d[i] = t;
+    w[i] = v;
+    nis = fma(v / t, v, nis);
+  }
+  return nis;
+}
+// The row's threshold for filter n (column maps do not apply) and the decision: reject when !(NIS <= threshold), so a NaN NIS
+// is rejected too.
+__device__ __forceinline__ bool gate_rejects(const KParams& p, int stream, long long n, double nis) {
+  const double* const tf = p.gate_nis_filter[stream];
+  return !(nis <= (tf ? __ldg(tf + n) : p.gate_nis[stream]));
+}
+// The entries an innovation set gets after the chunks in the GATE instantiations: the NIS -- the gate's on a gated stream,
+// for accepted and rejected filters alike -- and INNOV_APPLIED (the last entry of the row); NaN for a missing row.
+__device__ __forceinline__ void innov_end(const KParams& p, const Op& op, long long N, long long n, bool store, bool missing, bool skip,
+                                          double gnis, double nisq) {
+  const InnovK& iv = p.innov[op.stream];
+  if (!iv.out || !store) return;
+  double* const d = iv.out + op.row * iv.k * N + n;
+  if (iv.fields & INNOV_NIS) d[0] = missing ? innov_nan() : ((p.gate_streams >> op.stream) & 1u) ? gnis : nisq;
+  if (iv.fields & INNOV_APPLIED) d[(long long)(iv.k - 1) * N] = missing ? innov_nan() : skip ? 0.0 : 1.0;
 }
 
 // ---- RBIS_OP_RECORD (see RecK) ----
@@ -1513,10 +1585,13 @@ __device__ __forceinline__ void record_fields(const KParams& p, const Cov& P, co
 // only (and without SYN), launched only for such programs.
 // INNOV = true (with REC): a MEAS op of the program writes an innovation set (KParams::innov); launched only then, so that
 // programs that only record keep the code of the REC instantiations.
-template <bool BLOCKS, bool DC = false, bool SYN = false, bool REC = false, bool MASK = false, bool INNOV = false>
+// GATE = true (with MASK): a stream of the program has a NIS gate, or an innovation set of it asks for INNOV_APPLIED
+// (KParams::gate_streams); launched only then, so that the MASK instantiations keep their code.
+template <bool BLOCKS, bool DC = false, bool SYN = false, bool REC = false, bool MASK = false, bool INNOV = false, bool GATE = false>
 __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constant__ KParams p) {
   static_assert(!MASK || (BLOCKS && !SYN), "MASK instantiations have the one-row / correlated-block paths and read z from HBM");
   static_assert(!INNOV || REC, "INNOV instantiations are REC instantiations with the innovation path");
+  static_assert(!GATE || MASK, "GATE instantiations are MASK instantiations with the gate");
   extern __shared__ __align__(16) double smem[];
   __shared__ uint32_t tm_base_s;
   const int tid = threadIdx.x;
@@ -1659,10 +1734,20 @@ __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constan
       }
       V3 dquat{0, 0, 0};
       if (st.has_orient) dquat = subtract_quats(src.quat(st, op.row, sn), {s.qw, s.qx, s.qy, s.qz});  // rbis.cpp:199
+      // GATE: a gated stream (uniform branch) rejects the row for a filter whose prior NIS exceeds its threshold; that filter
+      // then skips it like a missing row.  Every lane evaluates the gate (warp-collective loads); a missing row is not gated.
+      const bool missing = skip;
+      double gnis = 0.0;
+      if constexpr (GATE) {
+        if ((p.gate_streams >> op.stream) & 1u) {
+          gnis = gate_nis<SYN>(st, src, s, op.row, N, n, sn, dquat, [&](int a, int b) { return cov_at(P, st.idx[a], st.idx[b]); });
+          skip = missing || gate_rejects(p, op.stream, n, gnis);
+        }
+      }
       // INNOV: an innovation set on this stream (uniform branch) gets y and S(a,a) now and the NIS after the chunks
       double nisq = 0.0;
       if constexpr (INNOV) {
-        if (p.innov[op.stream].out) innov_begin<SYN>(p.innov[op.stream], P, s, st, src, op.row, N, n, sn, dquat, active, skip);
+        if (p.innov[op.stream].out) innov_begin<SYN>(p.innov[op.stream], P, s, st, src, op.row, N, n, sn, dquat, active, missing);
       }
       const V3 chi0{s.x[6], s.x[7], s.x[8]};
       for (int ci = 0; ci < st.n_chunks; ci++) {
@@ -1687,7 +1772,9 @@ __global__ void __launch_bounds__(TPB, 1) rbis_fused_kernel(const __grid_constan
             break;
         }
       }
-      if constexpr (INNOV) {
+      if constexpr (INNOV && GATE) {
+        innov_end(p, op, N, n, active, missing, skip, gnis, nisq);
+      } else if constexpr (INNOV) {
         const InnovK& iv = p.innov[op.stream];
         if (iv.out && (iv.fields & INNOV_NIS) && active) iv.out[op.row * iv.k * N + n] = skip ? innov_nan() : nisq;
       }

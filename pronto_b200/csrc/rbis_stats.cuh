@@ -136,11 +136,12 @@ __constant__ double c_chi2_lo[9] = {0.000982069117, 0.050635616, 0.215795283, 0.
                                     1.23734425,     1.68986918,  2.17973075,  2.7003895};
 __constant__ double c_chi2_hi[9] = {5.02388619, 7.37775891, 9.3484036, 11.1432868, 12.832502,
                                     14.4493753, 16.0127643, 17.5345461, 19.0227678};
-constexpr int NINNOV = 33;  // statistics of an innovation table; the rest of the 96 are zero
+constexpr int NINNOV = 34;  // statistics of an innovation table; the rest of the 96 are zero
 // Ensemble statistics of innovation rows ([rows][k][N], the layout of InnovK with INNOV_NIS at position 0): row blockIdx.y of
 // `rows`, one CTA per chunk of blockDim.x filters, one table [gridDim.x][96] per row.  [0] sum NIS, [1] sum NIS^2, [2] finite
 // NIS, [3] NIS inside the central 95 % of chi2(m), [4] non-finite NIS, [5] filters, [6 + a] sum y_a, [15 + a] sum y_a^2,
-// [24 + a] sum y_a^2 / S(a,a); only filters with a finite NIS enter [0], [1], [3] and [6..32].  The fixed binary tree of
+// [24 + a] sum y_a^2 / S(a,a); only filters with a finite NIS enter [0], [1], [3] and [6..32].  [33] filters whose INNOV_APPLIED
+// entry (the last of the row, k - 1) is 0.0, i.e. rejected by a NIS gate; zero without that field.  The fixed binary tree of
 // stats_kernel, so a numpy restatement reproduces every table bit for bit.
 __global__ void __launch_bounds__(1024) innov_stats_kernel(const double* __restrict__ rows, long long k, int m, int fields, long long N,
                                                            double* __restrict__ out_chunks) {
@@ -176,6 +177,7 @@ __global__ void __launch_bounds__(1024) innov_stats_kernel(const double* __restr
       val[4] = 1.0;
     }
     val[5] = 1.0;
+    if ((fields & INNOV_APPLIED) && rows[(k - 1) * N + n] == 0.0) val[33] = 1.0;
   }
   static_for<NINNOV>([&](auto i) {
     red[t] = val[i];
